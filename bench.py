@@ -4,6 +4,8 @@
 Contract (one JSON line on stdout, rank 0):
   python bench.py --gpus N --steps K --warmup W            our arm (CUDA)
   python bench.py --impl reference --gpus N --steps K ...   CPU arm (oracle port)
+  python bench.py ... --dump-outputs DIR                    also writes the last timed launch's
+                                                            outputs to DIR/*.npy (dump_outputs)
 
 Workload (config.workload): swimming salamander (28 links, nv=33) with
 hydrodynamic drag + buoyancy and full sensor logging (links/joints/contacts/
@@ -77,6 +79,10 @@ def parse_args():
     ap.add_argument('--team-constraints', action='store_true',
                     help='hand-overs (limits / contacts) go to the team kernel instead of the per-thread '
                          'constrained kernel (comparison runs)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last timed launch computed as DIR/<name>.npy '
+                         '(float32): qpos, qvel and the log rows the launch wrote (links, joints, contacts, '
+                         'xfrc) of a fixed seeded sample of the environments (rank 0), at most 60 MiB in all')
     return ap.parse_args()
 
 
@@ -412,6 +418,29 @@ def short_device_run(name, n_envs, inner, ring, steps, warmup, device, peaks, am
     return out
 
 
+DUMP_BYTES = 60 << 20
+
+
+def dump_outputs(physics, inner, out_dir):
+    """``--dump-outputs``: the state ``qpos`` [S, nq], ``qvel`` [S, nv] and the log rows the last
+    launch wrote, ``<kind>`` [S, rows, n_items, n_cols], float32 as the engine holds them, so that
+    two builds can be compared output for output on the same inputs.  The S environments are
+    ``np.random.default_rng(0).choice(n_envs, S, replace=False)`` in ascending order, S as large
+    as DUMP_BYTES allows."""
+    rows = min(inner, physics.buffer_size)
+    first = physics.iteration - rows + 1          # step j writes ring row (j + 1) % ring
+    per_env = 4*(physics.model.nq + physics.model.nv) + rows*physics.log_bytes_per_env_step
+    n_sample = min(physics.n_envs, DUMP_BYTES//per_env)
+    envs = np.sort(np.random.default_rng(0).choice(physics.n_envs, n_sample, replace=False))
+    out = {'qpos': physics.qpos[envs], 'qvel': physics.qvel[envs]}
+    for kind in ('links', 'joints', 'contacts', 'xfrc'):
+        out[kind] = np.stack([physics.log_row(kind, (first + r) % physics.buffer_size)[envs]
+                              for r in range(rows)], axis=1)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in out.items():
+        np.save(os.path.join(out_dir, f'{name}.npy'), arr)
+
+
 # ---------------------------------------------------------------- GPU arm
 def run_b200(args, rank, world, local_rank):
     import torch
@@ -484,6 +513,8 @@ def run_b200(args, rank, world, local_rank):
     total_ms = timed(one, args.steps)
     clocks = sampler.summary()
     launches = physics.launch_count() - launches0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(physics, args.inner, args.dump_outputs)
     # per-launch kernel time from the engine's own CUDA events (recorded on the engine's stream
     # around the launch pair): mean over a few more launches, each read back before the next
     for _ in range(5):
@@ -676,7 +707,8 @@ def run_b200(args, rank, world, local_rank):
                 if name == args.model and n_envs == n_local and amplitude == 0.3:
                     continue
                 try:
-                    extra.append(short_device_run(name, n_envs, args.inner, 64, 10, 3, local_rank, peaks, amplitude))
+                    extra.append(short_device_run(name, n_envs, args.inner, 64, args.steps, args.warmup, local_rank,
+                                                  peaks, amplitude))
                 except Exception as exc:  # pylint: disable=broad-except
                     extra.append({'workload': f'{name}: {n_envs} envs', 'error': str(exc)})
             out['extra'] = {'other_configs': extra}
@@ -698,6 +730,8 @@ def main():
     world = int(os.environ.get('WORLD_SIZE', 1))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))
     if args.impl == 'reference':
+        if args.dump_outputs:
+            raise SystemExit('--dump-outputs writes the outputs of the CUDA arm (--impl b200)')
         run_reference(args, rank, world)
         return
     if world == 1 and args.gpus > 1:

@@ -85,13 +85,11 @@ def test_h5py_reads_the_file(tmp_path):
 
 
 def test_structures_match_a_file_written_by_libhdf5():
-    """The one HDF5 file in this image written by libhdf5 itself (MATLAB 7.4, HDF5 1.6; scipy's test
-    data; 512-byte user block): its superblock, root symbol-table entry, B-tree node, symbol-table
+    """A file written by libhdf5 itself (MATLAB 7.4, HDF5 1.6; tests/golden/testhdf5_7.4_GLNX86.mat,
+    a copy of SciPy's test file scipy/io/matlab/tests/data/testhdf5_7.4_GLNX86.mat, BSD licence;
+    512-byte user block): its superblock, root symbol-table entry, B-tree node, symbol-table
     node, local heap and IEEE float64 datatype message are laid out as hdf5_min writes them."""
-    scipy_io = pytest.importorskip('scipy.io')
-    sample = os.path.join(os.path.dirname(scipy_io.__file__), 'matlab', 'tests', 'data', 'testhdf5_7.4_GLNX86.mat')
-    if not os.path.exists(sample):
-        pytest.skip('scipy test data not installed')
+    sample = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'testhdf5_7.4_GLNX86.mat')
     from farms_mujoco_b200.hdf5_min import _datatype, _read_messages
     raw = open(sample, 'rb').read()
     base = raw.find(SIGNATURE)

@@ -6,8 +6,9 @@ Walks every layout / kernel selection (regular and SLIM blocks, per-thread and t
 paths, box contacts, fixed base, host row gathers) so that an out-of-bounds index into the
 per-environment blocks and scratch regions shows up on the GPU-less box (compute-sanitizer is
 closed on the GPU pool)."""
-import sys, numpy as np
-sys.path.insert(0,'/root/repo'); sys.path.insert(0,'/root/repo/tests')
+import os, sys, numpy as np
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT); sys.path.insert(0, os.path.join(ROOT, 'tests'))
 from conftest import make_case
 import variant_models
 from farms_mujoco_b200 import mjcf_subset
@@ -30,7 +31,6 @@ spec=variant_models.salamander_box_feet(); model=mjcf_subset.parse_mjcf(spec.mjc
 ph=BatchedPhysics.from_spec(spec,2,buffer_size=6,library=lib); ph.step(5); print('box ok')
 spec=variant_models.swimmer8_fixed_base(); ph=BatchedPhysics.from_spec(spec,2,buffer_size=6,library=lib); ph.step(5); print('fixed ok')
 # explicit <pair> self-collisions: the dense Newton Hessian behind the contact Jacobians
-sys.path.insert(0, '/root/repo/tests')
 from test_emu_parity import _pair_case
 spec, model, qpos0, qvel0, ctrl = _pair_case(3)
 ph = BatchedPhysics.from_spec(spec, 3, buffer_size=6, library=lib)

@@ -1,5 +1,5 @@
-import sys, numpy as np, time
-sys.path.insert(0,'/root/repo')
+import os, sys, numpy as np, time
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from farms_mujoco_b200 import models, mjcf_subset
 from farms_mujoco_b200.engine import BatchedPhysics
 from farms_mujoco_b200.sharding import synthetic_inputs
