@@ -285,11 +285,12 @@ template <int TEAM> struct FbStep {
   float comx, comy, comz;
   int ncon, nlim;
   int npair_act;   /* active contacts of explicit pairs (two-body rows) */
+  int nhard_act;   /* ... of them frictionless: hard normal rows (kind 10) */
 
   FB_MEM FbStep(const DevModel &m_, float *s_, int *si_, const EnvPtrs &g_, int lane_, int base_,
                 unsigned mask_)
       : m(m_), s(s_), si(si_), g(g_), lane(lane_), base(base_), mask(mask_),
-        comx(0.f), comy(0.f), comz(0.f), ncon(0), nlim(0) {}
+        comx(0.f), comy(0.f), comz(0.f), ncon(0), nlim(0), npair_act(0), nhard_act(0) {}
 
   FB_MEM void sync() { T::sync(mask); }
 
@@ -771,7 +772,7 @@ FB_UNROLL
     }
     nlim = (int)(T::sum(mask, cnt) + 0.5f);
     /* plane vs sphere / capsule end; compact in candidate order */
-    int n = 0, npair = 0;
+    int n = 0, npair = 0, nhard = 0;
     for (int c0 = 0; c0 < m.ncand; c0 += TEAM) {
       int c = c0 + lane;
       int hit = 0;
@@ -788,7 +789,7 @@ FB_UNROLL
         radius = MF(cand_radius, c);
         float cdist = centre[0]*nrm[0] + centre[1]*nrm[1] + centre[2]*nrm[2] - MF(cand_pd, c);
         dist = cdist - radius;
-        if (MI(cand_iscapsule, c) == 9) {
+        if (MI(cand_iscapsule, c) == 9 || MI(cand_iscapsule, c) == 10) {
           /* explicit <pair>, sphere-sphere (mjc_SphereSphere): the other sphere (geom1) sits on body
            * cand_body1 at cand_pn, radius cand_pd; the normal runs from it to this one */
           const int b1 = MI(cand_body1, c);
@@ -839,6 +840,7 @@ FB_UNROLL
       }
       unsigned bits = T::ballot(mask, base, hit);
       npair += FB_POPC(T::ballot(mask, base, hit && MI(cand_iscapsule, c) == 9));
+      if (m.n_hard > 0) nhard += FB_POPC(T::ballot(mask, base, hit && MI(cand_iscapsule, c) == 10));
       if (hit) {
         int i = n + FB_POPC(bits & ((1u << lane) - 1u));
         con_cand[i] = c;
@@ -871,6 +873,7 @@ FB_UNROLL
     }
     ncon = n;
     npair_act = npair;
+    nhard_act = nhard;
     if (lane == 0) *g.d_ncon = n;
     sync();
   }
@@ -920,6 +923,16 @@ FB_UNROLL
       float cmu2 = mu*mu*(R1/R);
       float Rpy = fmaxf(FB_MINVAL, 2.f*cmu2*R1);
       float vn = g.prod3[3*i], vt1 = g.prod3[3*i+1], vt2 = g.prod3[3*i+2];
+      if (MI(cand_iscapsule, c) == 10) {
+        /* frictionless pair: one hard row Jn a >= aref_n with a multiplier (solve_constraints).  Its
+         * four slots carry D = 0 -- the soft rows' sums skip them -- and aref_n, the mean of the four
+         * pyramidal aref (the +-mu vt terms cancel) */
+        for (int sub = 0; sub < 4; sub++) {
+          D[2*nj + 4*i + sub] = 0.f;
+          aref[2*nj + 4*i + sub] = -B*vn - K*imp*(dist - includemargin);
+        }
+        continue;
+      }
       for (int sub = 0; sub < 4; sub++) {
         float sg = (sub & 1) ? -1.f : 1.f;
         float vel = vn + sg*mu*((sub < 2) ? vt1 : vt2);
@@ -927,6 +940,10 @@ FB_UNROLL
         D[r] = 1.0f/Rpy;
         aref[r] = -B*vel - K*imp*(dist - includemargin);
       }
+    }
+    if (nhard_act > 0 && lane == 0) {
+      int h = 0;
+      for (int i = 0; i < ncon; i++) if (MI(cand_iscapsule, con_cand[i]) == 10) si[m.L.hcon + h++] = i;
     }
     sync();
   }
@@ -1000,6 +1017,212 @@ FB_UNROLL
     sync();
   }
 
+  /* x <- H^-1 x with the dense Cholesky factor held in L.H (lower triangle): L y = x, L' x = y */
+  FB_MEM void dense_solve(float *x) {
+    const int nv = m.nv;
+    const float *H = s + m.L.H;
+    for (int k = 0; k < nv; k++) {
+      const float yk = x[k]/H[k*nv + k];
+      sync();
+      if (lane == 0) x[k] = yk;
+      for (int i = k + 1 + lane; i < nv; i += TEAM) x[i] -= H[i*nv + k]*yk;
+      sync();
+    }
+    for (int k = nv - 1; k >= 0; k--) {
+      const float xk = x[k]/H[k*nv + k];
+      sync();
+      if (lane == 0) x[k] = xk;
+      for (int i = lane; i < k; i += TEAM) x[i] -= H[k*nv + i]*xk;
+      sync();
+    }
+  }
+
+  /* ---------- hard normal rows of frictionless pairs (kind 10): equality-constrained Newton ----------
+   * Each active hard contact h (contact hcon[h]) has one row Jn_h = J3[3 i] with Jn_h a >= aref_h and a
+   * multiplier lambda_h >= 0, its normal force.  On the working set W (hon[h] = 1; -1: a row that
+   * depends on the others of W, out for the rest of the solve, force 0) the Newton step is
+   * taken in direct-multiplier form: u = H^-1 g, V = H^-1 Jn_W', S = Jn_W V, S lambda = Jn_W u - x_W,
+   * p = -u + V lambda, so that Jn_W (a + p) = aref_W.  A row counts as satisfied while
+   * |Jn a - aref| <= FB_HARD_TOL (sum_v |Jn_v a_v| + |aref| + S_hh |lambda_h|) + FB_HARD_ATOL: relative to
+   * the terms the residual is the difference of and to the normal acceleration its own force makes --
+   * one ulp of lambda moves Jn a by S_hh ulp(lambda), the floor a Newton step cannot go below. */
+#define FB_HARD_TOL 1e-4f
+#define FB_HARD_ATOL 1e-6f
+#define FB_HARD_PIVOT 1e-5f    /* a pivot of S below this share of its diagonal: the row depends on the others */
+/* On a settled W the Lagrangian gradient can stay above the soft solver's 2e-5 floor: the stiff soft
+ * rows (joint limits) put rounding noise of D eps |J a| into it, and the Newton steps it drives are
+ * ~1e-5 of |qacc| (SALAMANDER, both foot pairs and a joint limit active).  A step below 1e-4 of |qacc|
+ * on a settled W therefore counts as converged too. */
+#define FB_HARD_STALL 1e-8f
+
+  /* hx = Jn a - aref and its tolerance for every active hard row; prod3 holds J3 a */
+  FB_MEM void hard_residuals(const float *a) {
+    const int nv = m.nv, nj = m.njnt, NH = m.n_hard;
+    const int *hcon = si + m.L.hcon;
+    float *hx = s + m.L.hx, *htol = s + m.L.htol;
+    const float *S = s + m.L.hS, *hlam = s + m.L.hlam;
+    for (int h = 0; h < nhard_act; h++) {
+      const int i = hcon[h];
+      float mag = 0.f;
+      for (int v = lane; v < nv; v += TEAM) mag += fabsf(g.J3[(3*i)*nv + v]*a[v]);
+      mag = T::sum(mask, mag);
+      if (lane == 0) {
+        const float ar = g.efc[2*nj + 4*i];
+        /* (a non-zero multiplier was computed together with its S_hh) */
+        const float own = hlam[h] != 0.f ? S[h*NH + h]*fabsf(hlam[h]) : 0.f;
+        hx[h] = g.prod3[3*i] - ar;
+        htol[h] = FB_HARD_TOL*(mag + fabsf(ar) + own) + FB_HARD_ATOL;
+      }
+    }
+    sync();
+  }
+
+  /* violated rows outside W join it; returns whether any did (the same on every lane) */
+  FB_MEM int hard_add_violated() {
+    int *hon = si + m.L.hon;
+    const float *hx = s + m.L.hx, *htol = s + m.L.htol;
+    int add = 0;
+    for (int h = 0; h < nhard_act; h++) add |= hon[h] == 0 && hx[h] < -htol[h];
+    sync();
+    if (lane == 0) for (int h = 0; h < nhard_act; h++) if (hon[h] == 0 && hx[h] < -htol[h]) hon[h] = 1;
+    sync();
+    return add;
+  }
+
+  FB_MEM int hard_feasible() {
+    const int *hon = si + m.L.hon;
+    const float *hx = s + m.L.hx, *htol = s + m.L.htol;
+    for (int h = 0; h < nhard_act; h++) if (hon[h] == 1 && fabsf(hx[h]) > htol[h]) return 0;
+    return 1;
+  }
+
+  /* the row of W with the most negative multiplier leaves W; returns whether there was one */
+  FB_MEM int hard_release() {
+    int *hon = si + m.L.hon;
+    float *hlam = s + m.L.hlam;
+    int worst = -1;
+    for (int h = 0; h < nhard_act; h++)
+      if (hon[h] == 1 && hlam[h] < 0.f && (worst < 0 || hlam[h] < hlam[worst])) worst = h;
+    sync();
+    if (lane == 0 && worst >= 0) { hon[worst] = 0; hlam[worst] = 0.f; }
+    sync();
+    return worst >= 0;
+  }
+
+  /* |g - Jn_W' lambda|^2, the gradient of the Lagrangian with the multipliers of the last step;
+   * |Jn_W' lambda|^2 is added to *gref, the terms the gradient is the difference of */
+  FB_MEM float hard_lagrangian_norm2(const float *grad, float *gref) {
+    const int nv = m.nv;
+    const int *hcon = si + m.L.hcon, *hon = si + m.L.hon;
+    const float *hlam = s + m.L.hlam;
+    float gn = 0.f, fn = 0.f;
+    for (int v = lane; v < nv; v += TEAM) {
+      float f = 0.f;
+      for (int h = 0; h < nhard_act; h++) if (hon[h] == 1) f += hlam[h]*g.J3[(3*hcon[h])*nv + v];
+      const float gl = grad[v] - f;
+      gn += gl*gl; fn += f*f;
+    }
+    *gref += T::sum(mask, fn);
+    return T::sum(mask, gn);
+  }
+
+  /* sum over W of lambda_h Jn_h p (prod3 holds J3 p): the hard rows' term of the Lagrangian's slope */
+  FB_MEM float hard_lambda_jp() {
+    const int *hcon = si + m.L.hcon, *hon = si + m.L.hon;
+    const float *hlam = s + m.L.hlam;
+    float acc = 0.f;
+    for (int h = 0; h < nhard_act; h++) if (hon[h] == 1) acc += hlam[h]*g.prod3[3*hcon[h]];
+    return acc;
+  }
+
+  /* p = -H^-1 g on entry (H factored: dense while a kind-9 pair is active, else tree-sparse in qLD);
+   * on return p = -u + V lambda with the multipliers of W in hlam.  y: nv floats of scratch. */
+  FB_MEM void hard_step(float *p, float *y) {
+    const int nv = m.nv, NH = m.n_hard;
+    const int *hcon = si + m.L.hcon;
+    int *hon = si + m.L.hon, *ws = si + m.L.hws;
+    float *V = s + m.L.hV, *S = s + m.L.hS, *Lf = s + m.L.hL, *hlam = s + m.L.hlam, *rhs = s + m.L.hrhs;
+    const float *hx = s + m.L.hx;
+    int any = 0;
+    for (int h = 0; h < nhard_act; h++) {
+      if (hon[h] != 1) continue;
+      any = 1;
+      const float *jn = g.J3 + (3*hcon[h])*nv;
+      for (int v = lane; v < nv; v += TEAM) V[h*nv + v] = jn[v];
+      sync();
+      if (npair_act > 0) dense_solve(V + h*nv); else solve_ld(V + h*nv, y);
+    }
+    if (!any) return;
+    for (int a = 0; a < nhard_act; a++) {
+      if (hon[a] != 1) continue;
+      const float *jn = g.J3 + (3*hcon[a])*nv;
+      for (int b = 0; b <= a; b++) {
+        if (hon[b] != 1) continue;
+        float part = 0.f;
+        for (int v = lane; v < nv; v += TEAM) part += jn[v]*V[b*nv + v];
+        part = T::sum(mask, part);
+        if (lane == 0) S[a*NH + b] = part;
+      }
+      float part = 0.f;                       /* Jn_a u = -Jn_a p */
+      for (int v = lane; v < nv; v += TEAM) part -= jn[v]*p[v];
+      part = T::sum(mask, part);
+      if (lane == 0) rhs[a] = part - hx[a];
+    }
+    sync();
+    if (lane == 0) {
+      /* Cholesky of S on W (compact order ws); a row whose pivot collapses leaves W */
+      for (;;) {
+        int k = 0;
+        for (int h = 0; h < nhard_act; h++) if (hon[h] == 1) ws[k++] = h;
+        int drop = -1;
+        for (int a = 0; a < k && drop < 0; a++) {
+          for (int b = 0; b <= a; b++) {
+            float sum = S[ws[a]*NH + ws[b]];
+            for (int c = 0; c < b; c++) sum -= Lf[a*NH + c]*Lf[b*NH + c];
+            if (b < a) { Lf[a*NH + b] = sum/Lf[b*NH + b]; continue; }
+            if (!(sum > FB_HARD_PIVOT*S[ws[a]*NH + ws[a]])) { drop = ws[a]; break; }
+            Lf[a*NH + a] = sqrtf(sum);
+          }
+        }
+        if (drop >= 0) { hon[drop] = -1; hlam[drop] = 0.f; continue; }
+        for (int a = 0; a < k; a++) {
+          float sum = rhs[ws[a]];
+          for (int c = 0; c < a; c++) sum -= Lf[a*NH + c]*hlam[ws[c]];
+          hlam[ws[a]] = sum/Lf[a*NH + a];
+        }
+        for (int a = k - 1; a >= 0; a--) {
+          float sum = hlam[ws[a]];
+          for (int c = a + 1; c < k; c++) sum -= Lf[c*NH + a]*hlam[ws[c]];
+          hlam[ws[a]] = sum/Lf[a*NH + a];
+        }
+        break;
+      }
+    }
+    sync();
+    for (int v = lane; v < nv; v += TEAM) {
+      float acc = p[v];
+      for (int h = 0; h < nhard_act; h++) if (hon[h] == 1) acc += hlam[h]*V[h*nv + v];
+      p[v] = acc;
+    }
+    sync();
+  }
+
+  /* ratio test: alpha shrinks to where the first hard row outside W would become violated along p
+   * (prod3 holds J3 p); returns that row (it joins W after the step) or -1 */
+  FB_MEM int hard_ratio_test(float *alpha) {
+    const int *hcon = si + m.L.hcon, *hon = si + m.L.hon;
+    const float *hx = s + m.L.hx;
+    int block = -1;
+    for (int h = 0; h < nhard_act; h++) {
+      if (hon[h] != 0) continue;
+      const float jp = g.prod3[3*hcon[h]];
+      if (!(jp < 0.f)) continue;
+      const float ah = fmaxf(0.f, -hx[h]/jp);
+      if (ah < *alpha) { *alpha = ah; block = h; }
+    }
+    return block;
+  }
+
   /* ------------------------------------ A.8 primal Newton, exact line search */
   FB_MEM void solve_constraints(float *tmp1, float *tmp2) {
     const int nv = m.nv, nj = m.njnt;
@@ -1011,6 +1234,13 @@ FB_UNROLL
     float *aref = g.efc, *D = g.efc + m.maxefc, *res = g.efc + 2*m.maxefc,
           *jp = g.efc + 3*m.maxefc, *frc = g.efc + 4*m.maxefc;
     int maxit = m.solver_iterations < 50 ? m.solver_iterations : 50;
+    /* hard rows of frictionless pairs: W starts empty; `done` once the multipliers of W are >= 0,
+     * W's rows hold and no other row is violated */
+    int done = 0;
+    if (nhard_act > 0) {
+      for (int h = lane; h < nhard_act; h += TEAM) { si[m.L.hon + h] = 0; s[m.L.hlam + h] = 0.f; }
+      sync();
+    }
     for (int it = 0; it < maxit; it++) {
       rows_apply(qacc, res);
       for (int r = lane; r < nrow; r += TEAM) {
@@ -1019,6 +1249,7 @@ FB_UNROLL
         frc[r] = (rr < 0.f) ? D[r]*rr : 0.f;   /* y = D min(0, res) */
       }
       sync();
+      if (nhard_act > 0) hard_residuals(qacc);   /* prod3 = J3 qacc */
       mul_m(qacc, tmp1);                         /* tmp1 = M a */
       float gref = 0.f;                          /* magnitude of the terms the gradient is the difference of */
       for (int v = lane; v < nv; v += TEAM) {
@@ -1028,13 +1259,25 @@ FB_UNROLL
       gref = T::sum(mask, gref);
       sync();
       rows_tapply(frc, grad, 1);                 /* grad = M a - fsm + J' y */
-      float gn = 0.f;
-      for (int v = lane; v < nv; v += TEAM) gn += grad[v]*grad[v];
-      gn = T::sum(mask, gn);
-      /* MuJoCo's test (scaled gradient < tolerance, 1e-8 by default) is out of reach of fp32:
-       * once the active set is right the gradient is rounding noise, ~5e-6 of the terms it is
-       * the difference of.  Stop at whichever floor comes first. */
-      if (sqrtf(gn)*m.solver_scale < fmaxf(m.tolerance, 2e-5f*sqrtf(gref)*m.solver_scale)) break;
+      int added = 0, feasible = 1;
+      if (nhard_act == 0) {
+        float gn = 0.f;
+        for (int v = lane; v < nv; v += TEAM) gn += grad[v]*grad[v];
+        gn = T::sum(mask, gn);
+        /* MuJoCo's test (scaled gradient < tolerance, 1e-8 by default) is out of reach of fp32:
+         * once the active set is right the gradient is rounding noise, ~5e-6 of the terms it is
+         * the difference of.  Stop at whichever floor comes first. */
+        if (sqrtf(gn)*m.solver_scale < fmaxf(m.tolerance, 2e-5f*sqrtf(gref)*m.solver_scale)) break;
+      } else {
+        /* the same test on the Lagrangian gradient, once W is settled and its rows hold; then a
+         * negative multiplier leaves W, or the solve is done */
+        added = hard_add_violated();
+        feasible = hard_feasible();
+        const float gn = hard_lagrangian_norm2(grad, &gref);
+        if (!added && feasible && sqrtf(gn)*m.solver_scale < fmaxf(m.tolerance, 2e-5f*sqrtf(gref)*m.solver_scale)) {
+          if (!hard_release()) { done = 1; break; }
+        }
+      }
       /* H = M + sum_active D J'J.  Every row of J is supported on the ancestors of ONE body
        * (limits: one dof; plane contacts: the chain of the touching body), so H has exactly the
        * tree sparsity of M: it is assembled in M's layout and factored by the same scheduled
@@ -1089,23 +1332,10 @@ FB_UNROLL
           }
           sync();
         }
-        /* p = -H^-1 grad: L y = -grad, L' p = y */
+        /* p = -H^-1 grad */
         for (int v = lane; v < nv; v += TEAM) p[v] = -grad[v];
         sync();
-        for (int k = 0; k < nv; k++) {
-          const float yk = p[k]/H[k*nv + k];
-          sync();
-          if (lane == 0) p[k] = yk;
-          for (int i = k + 1 + lane; i < nv; i += TEAM) p[i] -= H[i*nv + k]*yk;
-          sync();
-        }
-        for (int k = nv - 1; k >= 0; k--) {
-          const float xk = p[k]/H[k*nv + k];
-          sync();
-          if (lane == 0) p[k] = xk;
-          for (int i = lane; i < k; i += TEAM) p[i] -= H[k*nv + i]*xk;
-          sync();
-        }
+        dense_solve(p);
       } else {
         for (int e = lane; e < m.nM; e += TEAM) {
           const int u = MI(ent_i, e), v = MI(ent_j, e);      /* v is u or an ancestor of u */
@@ -1140,42 +1370,53 @@ FB_UNROLL
         sync();
         solve_ld(p, tmp2);
       }
-      /* exact line search on phi'(alpha) = g0 + alpha pMp + sum D jp min(0, res + alpha jp) */
-      rows_apply(p, jp);
-      mul_m(p, tmp2);
-      float pMp = 0.f, g0 = 0.f;
-      for (int v = lane; v < nv; v += TEAM) { pMp += p[v]*tmp2[v]; g0 += p[v]*tmp1[v]; }
-      pMp = T::sum(mask, pMp);
-      g0 = T::sum(mask, g0);
-      float lo = 0.f, hi = 3.0e38f;
-      for (int r = lane; r < nrow; r += TEAM) {
-        float dr = D[r], jr = jp[r];
-        if (dr <= 0.f || jr == 0.f) continue;
-        float al = -res[r]/jr;
-        if (!(al > 0.f)) continue;
-        float gv = g0 + al*pMp;
-        for (int q = 0; q < nrow; q++) {
-          float dq = D[q];
-          if (dq > 0.f) gv += dq*jp[q]*fminf(0.f, res[q] + al*jp[q]);
+      if (nhard_act > 0) hard_step(p, tmp2);
+      float alpha = 1.0f;
+      if (nhard_act > 0 && (added || !feasible)) {
+        /* W grew or its rows do not hold yet: the full step onto them */
+        j3_times(p);
+      } else {
+        /* exact line search on phi'(alpha) = g0 + alpha pMp + sum D jp min(0, res + alpha jp).  With
+         * hard rows it runs on the Lagrangian, lambda of W held: g0 loses lambda Jn_W p (Jn_W p =
+         * -x_W, rounding noise once the rows hold, which would otherwise steer alpha) */
+        rows_apply(p, jp);
+        mul_m(p, tmp2);
+        float pMp = 0.f, g0 = 0.f;
+        for (int v = lane; v < nv; v += TEAM) { pMp += p[v]*tmp2[v]; g0 += p[v]*tmp1[v]; }
+        pMp = T::sum(mask, pMp);
+        g0 = T::sum(mask, g0);
+        if (nhard_act > 0) g0 -= hard_lambda_jp();
+        float lo = 0.f, hi = 3.0e38f;
+        for (int r = lane; r < nrow; r += TEAM) {
+          float dr = D[r], jr = jp[r];
+          if (dr <= 0.f || jr == 0.f) continue;
+          float al = -res[r]/jr;
+          if (!(al > 0.f)) continue;
+          float gv = g0 + al*pMp;
+          for (int q = 0; q < nrow; q++) {
+            float dq = D[q];
+            if (dq > 0.f) gv += dq*jp[q]*fminf(0.f, res[q] + al*jp[q]);
+          }
+          if (gv <= 0.f) lo = fmaxf(lo, al); else hi = fminf(hi, al);
         }
-        if (gv <= 0.f) lo = fmaxf(lo, al); else hi = fminf(hi, al);
+        lo = T::max(mask, lo);
+        hi = T::min(mask, hi);
+        float am = hi < 1.0e38f ? 0.5f*(lo + hi) : lo + 1.0f;
+        float glo = 0.f, slope = 0.f;
+        for (int r = lane; r < nrow; r += TEAM) {
+          float dr = D[r];
+          if (dr <= 0.f) continue;
+          float jr = jp[r];
+          glo += dr*jr*fminf(0.f, res[r] + lo*jr);
+          if (res[r] + am*jr < 0.f) slope += dr*jr*jr;
+        }
+        glo = T::sum(mask, glo) + g0 + lo*pMp;
+        slope = T::sum(mask, slope) + pMp;
+        alpha = slope > 0.f ? lo - glo/slope : 1.0f;
+        if (!(alpha > 0.f) || alpha != alpha) alpha = lo > 0.f ? lo : 1.0f;
+        if (hi < 1.0e38f && alpha > hi) alpha = hi;
       }
-      lo = T::max(mask, lo);
-      hi = T::min(mask, hi);
-      float am = hi < 1.0e38f ? 0.5f*(lo + hi) : lo + 1.0f;
-      float glo = 0.f, slope = 0.f;
-      for (int r = lane; r < nrow; r += TEAM) {
-        float dr = D[r];
-        if (dr <= 0.f) continue;
-        float jr = jp[r];
-        glo += dr*jr*fminf(0.f, res[r] + lo*jr);
-        if (res[r] + am*jr < 0.f) slope += dr*jr*jr;
-      }
-      glo = T::sum(mask, glo) + g0 + lo*pMp;
-      slope = T::sum(mask, slope) + pMp;
-      float alpha = slope > 0.f ? lo - glo/slope : 1.0f;
-      if (!(alpha > 0.f) || alpha != alpha) alpha = lo > 0.f ? lo : 1.0f;
-      if (hi < 1.0e38f && alpha > hi) alpha = hi;
+      const int block = nhard_act > 0 ? hard_ratio_test(&alpha) : -1;   /* prod3 = J3 p */
       float st = 0.f, a2 = 0.f;
       for (int v = lane; v < nv; v += TEAM) {
         float dv = alpha*p[v], nvv = qacc[v] + dv;
@@ -1185,9 +1426,17 @@ FB_UNROLL
       a2 = T::sum(mask, a2);
       sync();
       for (int v = lane; v < nv; v += TEAM) qacc[v] += alpha*p[v];
+      if (block >= 0 && lane == 0) si[m.L.hon + block] = 1;
       sync();
-      if (st <= 1e-14f*a2) break;
+      if (nhard_act == 0) {
+        if (st <= 1e-14f*a2) break;
+      } else if (st <= FB_HARD_STALL*a2 && !added && feasible && block < 0) {
+        /* a vanishing Newton step on a settled W: the multipliers of this step decide */
+        if (!hard_release()) { done = 1; break; }
+      }
     }
+    /* the hard rows' solve did not settle within the iteration cap */
+    if (nhard_act > 0 && !done && lane == 0) FB_FLAG_OR(g.flags, FB_FLAG_SOLVER);
 
     /* constraint forces */
     rows_apply(qacc, res);
@@ -1196,6 +1445,14 @@ FB_UNROLL
       frc[r] = (rr < 0.f) ? -D[r]*rr : 0.f;
     }
     sync();
+    /* a hard row's normal force lambda, a quarter on each of its four slots: J' frc adds Jn' lambda
+     * and the contact force reads (lambda, 0, 0) */
+    for (int h = lane; h < nhard_act; h += TEAM) {
+      const int i = si[m.L.hcon + h];
+      const float q = 0.25f*s[m.L.hlam + h];
+      for (int k = 0; k < 4; k++) frc[2*nj + 4*i + k] = q;
+    }
+    if (nhard_act > 0) sync();
     rows_tapply(frc, fcon, 0);
     float *limf = s + m.L.limf;
     for (int j = lane; j < nj; j += TEAM) {

@@ -172,8 +172,13 @@ struct DevLayout {
       qM, qLD, dinv, fsm, qacc, fcon, grad, pvec, tmp1, tmp2, limf, scratch;
   /* aliases inside scratch */
   int crb, cacc, cfrc, buf, altB, Md, H;
+  /* hard normal rows of frictionless pairs (n_hard of them): V = H^-1 Jn' [n_hard][nv], S = Jn V and
+   * its Cholesky factor [n_hard][n_hard] each, multipliers, residuals Jn a - aref, their tolerances
+   * and the right-hand side of S lambda = Jn u - x [n_hard] each */
+  int hV, hS, hL, hlam, hx, htol, hrhs;
   int n_float;   /* floats per env */
   int con_cand;  /* int region: con_cand[maxcon] */
+  int hcon, hon, hws;   /* int regions [n_hard]: contact of each active hard row, working-set flags, compact working set */
   int n_int;
 };
 
@@ -184,6 +189,7 @@ struct DevModel {
   int n_links, n_joints, n_contacts, n_xfrc, n_swim, n_wc;
   int maxcon, maxefc, npack; /* npack = nv*(nv+1)/2 */
   int n_pair;                /* candidates of explicit <pair>s (two-body rows: team kernel only, dense Newton Hessian) */
+  int n_hard;                /* ... of them frictionless, solved as hard normal rows (kind 10; H stays tree-sparse) */
   int solver_iterations, any_damping, any_stiffness, any_limit;
   int col_jpos, col_jvel, col_jtrq, col_jlim;
   int link_cols, joint_cols, contact_cols, xfrc_cols;
@@ -518,21 +524,25 @@ inline bool fb_build_model(const FbModel *fm, const FbFarms *ff, const FbWaveCon
   std::vector<int32_t> cbody(nc), ccaps(nc), cbody1(nc, 0);
   std::vector<double> lpos(3*nc), laxis(3*nc), rad(nc), pn(3*nc), pd(nc), cinvw(nc), gquat(4*nc, 0.0);
   m.n_pair = 0;
+  m.n_hard = 0;
   bool any_ellipsoid = false;      /* ... or cylinder: candidates whose contact point moves over the geom */
   for (int c = 0; c < nc; c++) {
     int g1 = fm->cand_geom1[c], g2 = fm->cand_geom2[c];
-    if (fm->cand_end[c] == 20) {
+    if (fm->cand_end[c] == 20 || fm->cand_end[c] == 21) {
       /* explicit <pair>, sphere-sphere (mjc_SphereSphere): kind 9.  cand_body / lpos / rad describe
        * geom2 as for a plane candidate; geom1 travels in the plane's slots: cand_body1 = its body,
        * pn = its centre in that body's frame, pd = its radius.  Rows of such a contact live on the
        * chains of TWO bodies: the model runs on the team kernel, whose Newton step takes a dense
-       * Hessian while one of them is active (fb_device.h). */
+       * Hessian while one of them is active (fb_device.h).
+       * cand_end 21, a frictionless pair: kind 10, the same geometry; its contact is one hard
+       * normal row with a multiplier, which leaves the Hessian tree-sparse. */
       if (fm->geom_type[g1] != FB_GEOM_SPHERE || fm->geom_type[g2] != FB_GEOM_SPHERE ||
           fm->geom_bodyid[g1] < 1 || fm->geom_bodyid[g2] < 1 || fm->geom_bodyid[g1] == fm->geom_bodyid[g2]) {
-        out.error = "pair candidates (cand_end 20) must be spheres on two different bodies of the tree"; return false;
+        out.error = "pair candidates (cand_end 20, 21) must be spheres on two different bodies of the tree"; return false;
       }
       cbody[c] = fm->geom_bodyid[g2]; cbody1[c] = fm->geom_bodyid[g1];
-      ccaps[c] = 9;
+      ccaps[c] = fm->cand_end[c] == 21 ? 10 : 9;
+      if (fm->cand_end[c] == 21) m.n_hard++;
       gquat[4*c] = 1.0;
       for (int k = 0; k < 3; k++) { lpos[3*c+k] = fm->geom_pos[3*g2+k]; laxis[3*c+k] = 0.0; pn[3*c+k] = fm->geom_pos[3*g1+k]; }
       rad[c] = fm->geom_size[3*g2];
@@ -1009,12 +1019,18 @@ inline bool fb_build_model(const FbModel *fm, const FbFarms *ff, const FbWaveCon
     L.H = L.scratch + pad4(m.npack);
     off += natural > need ? natural : need;
   }
-  /* models with explicit <pair>s: the dense Newton Hessian of the team kernel (nv x nv), a region of
-   * its own (the scratch aliases are live during the solve) */
-  if (m.n_pair > 0) L.H = take(nv*nv);
+  /* models with explicit <pair>s of kind 9: the dense Newton Hessian of the team kernel (nv x nv), a
+   * region of its own (the scratch aliases are live during the solve) */
+  if (m.n_pair - m.n_hard > 0) L.H = take(nv*nv);
+  /* frictionless pairs: the Schur-complement step on their hard normal rows */
+  const int nh = m.n_hard;
+  L.hV = take(nh*nv); L.hS = take(nh*nh); L.hL = take(nh*nh);
+  L.hlam = take(nh); L.hx = take(nh); L.htol = take(nh); L.hrhs = take(nh);
   L.n_float = off;
   L.con_cand = 0;
   L.n_int = (m.maxcon + 3) & ~3;
+  L.hcon = L.n_int; L.hon = L.hcon + ((nh + 3) & ~3); L.hws = L.hon + ((nh + 3) & ~3);
+  L.n_int = L.hws + ((nh + 3) & ~3);
   if (L.n_int == 0) L.n_int = 4;
   return true;
 }

@@ -216,9 +216,10 @@ class BatchedPhysics:
         self.iteration = 0
 
     @classmethod
-    def from_spec(cls, spec, n_envs, buffer_size=1, **kwargs):
-        """Build from an ``AnimatSpec`` (models.py): MJCF text + option objects."""
-        model = parse_mjcf(spec.mjcf)
+    def from_spec(cls, spec, n_envs, buffer_size=1, frictionless_pairs='refuse', **kwargs):
+        """Build from an ``AnimatSpec`` (models.py): MJCF text + option objects.
+        ``frictionless_pairs``: see ``mjcf_subset.parse_mjcf``."""
+        model = parse_mjcf(spec.mjcf, frictionless_pairs=frictionless_pairs)
         return cls(model, n_envs, spec.links_names, spec.joints_names, spec.contacts_names,
                    spec.xfrc_names, animat_options=spec.animat_options,
                    arena_options=spec.arena_options, units=spec.simulation_options.units,

@@ -19,6 +19,7 @@ cameras, lights, textures) is init-time or rendering and is ignored or rejected
 with an explicit error.
 """
 
+import copy
 import xml.etree.ElementTree as ET
 from dataclasses import dataclass, field
 from typing import Dict, List
@@ -232,7 +233,8 @@ class Model:
     # collision candidates (plane vs sphere / capsule end), compile-time
     cand_geom1: np.ndarray = None      # plane geom id
     cand_geom2: np.ndarray = None      # animat geom id
-    cand_end: np.ndarray = None        # 0 sphere centre, +1 / -1 capsule ends, 2..9 box corner (end - 2), 10 ellipsoid, 11..14 cylinder points
+    cand_end: np.ndarray = None        # 0 sphere centre, +1 / -1 capsule ends, 2..9 box corner (end - 2), 10 ellipsoid, 11..14 cylinder points,
+                                       # 20 sphere-sphere <pair>, 21 frictionless sphere-sphere <pair> solved as a hard normal row
     cand_friction: np.ndarray = None   # mixed sliding friction
     cand_solref: np.ndarray = None     # [ncand, 2]
     cand_solimp: np.ndarray = None     # [ncand, 5]
@@ -337,9 +339,19 @@ def _parse_body(elem, parent, bodies, anon):
     return body
 
 
-def parse_mjcf(xml_text: str) -> Model:
-    """Parse FARMS-schema MJCF text and compile it into a flat ``Model``."""
+FRICTIONLESS_PAIRS = ('refuse', 'hard')
+
+
+def parse_mjcf(xml_text: str, frictionless_pairs: str = 'refuse') -> Model:
+    """Parse FARMS-schema MJCF text and compile it into a flat ``Model``.
+
+    ``frictionless_pairs`` says what becomes of a ``<contact><pair>`` whose friction is at MuJoCo's
+    floor (``friction="0 ..."``, what the reference writes for every self-collision):
+    ``'refuse'`` (default) raises, ``'hard'`` compiles it to a hard normal row (candidate kind 21)
+    that drops the O(mu) terms of the pyramidal cone (DESIGN.md section 8)."""
     # pylint: disable=too-many-locals,too-many-branches,too-many-statements
+    if frictionless_pairs not in FRICTIONLESS_PAIRS:
+        raise ValueError(f'frictionless_pairs must be one of {FRICTIONLESS_PAIRS}, not {frictionless_pairs!r}')
     root = ET.fromstring(xml_text)
     if root.tag != 'mujoco':
         raise ValueError('not an MJCF document')
@@ -778,7 +790,7 @@ def parse_mjcf(xml_text: str) -> Model:
                 raise NotImplementedError(f'<contact><{elem.tag}> is outside the batched path')
             pairs.append(elem)
 
-    _compile_collision_candidates(model, pairs)
+    _compile_collision_candidates(model, pairs, frictionless_pairs)
     _compile_invweight0(model)
     return model
 
@@ -816,10 +828,12 @@ def _mix_contact_params(model, g1, g2):
 PAIR_MIN_FRICTION = 0.1
 
 
-def _compile_pair_candidates(model, pairs):
+def _compile_pair_candidates(model, pairs, frictionless_pairs='refuse'):
     """Explicit ``<contact><pair>`` self-collisions (mjcf.py:1012-1033: one pair per couple of
     collision geoms of the two links, ``condim=3``, ``friction=[0]*5``, optionally ``solref``).
-    Sphere-sphere only (candidate kind 20, ``mjc_SphereSphere``).  An explicit pair bypasses the
+    Sphere-sphere only (candidate kind 20, ``mjc_SphereSphere``; kind 21 for a pair at the friction
+    floor under ``frictionless_pairs='hard'``: the same geometry and parameters, solved as one hard
+    normal row per contact).  An explicit pair bypasses the
     contype / conaffinity and same-body / parent-child filters; attributes the element does not
     give come from the two geoms by the mixing rule, as MuJoCo's compiler fills them in."""
     cands = []
@@ -851,20 +865,28 @@ def _compile_pair_candidates(model, pairs):
             solimp = np.concatenate([given, np.array([0.9, 0.95, 0.001, 0.5, 2.0])[len(given):]])
         margin = float(elem.get('margin')) if elem.get('margin') is not None else max(model.geom_margin[g1], model.geom_margin[g2])
         gap = float(elem.get('gap')) if elem.get('gap') is not None else max(model.geom_gap[g1], model.geom_gap[g2])
+        if friction[0] <= MJ_MINMU and frictionless_pairs == 'hard':
+            # One hard row n.J.qacc >= aref per contact with the normal force as a multiplier
+            # (fb_device.h): drops the 1e-5 n of tangential force such a cone carries and the
+            # O(mu) softness of its normal.  mu stays at the floor for the record.
+            cands.append((g1, g2, 21, MJ_MINMU, solref, solimp, margin, gap))
+            continue
         if friction[0] < PAIR_MIN_FRICTION:
             # A pyramidal contact's rows carry D = 1/(2 mu^2 R) (mj_makeImpedance): at the floor
             # mu = 1e-5 that the reference's friction=[0]*5 pairs get (mjcf.py:1029), the normal
             # direction is 1e10 times stiffer than at mu = 1 and its residual J.qacc - aref has to
             # be resolved to 1e-11 relative -- out of reach of the fp32 primal Newton step
             # (DESIGN.md section 8).
+            hint = (" parse_mjcf(..., frictionless_pairs='hard') solves frictionless pairs as hard normal rows"
+                    if friction[0] <= MJ_MINMU else '')
             raise NotImplementedError(
                 f'<pair> {names}: friction {friction[0]:g} < {PAIR_MIN_FRICTION}: near-frictionless pyramidal '
-                'contacts are too stiff for the fp32 solver (DESIGN.md section 8)')
+                f'contacts are too stiff for the fp32 solver (DESIGN.md section 8).{hint}')
         cands.append((g1, g2, 20, max(MJ_MINMU, friction[0]), solref, solimp, margin, gap))
     return cands
 
 
-def _compile_collision_candidates(model, pairs=()):
+def _compile_collision_candidates(model, pairs=(), frictionless_pairs='refuse'):
     """Enumerate plane-vs-{sphere, capsule end, box corner, ellipsoid} candidates (and the four points of a cylinder) with mixed parameters.
 
     Pair filter ``(contype1 & conaffinity2) || (contype2 & conaffinity1)``,
@@ -905,7 +927,7 @@ def _compile_collision_candidates(model, pairs=()):
                 cands.append((g1, g2, end, max(MJ_MINMU, friction[0]), solref, solimp, margin, gap))
     # explicit pairs come last (MuJoCo's broad phase lists them ahead of the filtered ones; the
     # order of the contacts does not enter the solution, only the order of the rows)
-    cands += _compile_pair_candidates(model, pairs)
+    cands += _compile_pair_candidates(model, pairs, frictionless_pairs)
     n = len(cands)
     model.cand_geom1 = np.array([c[0] for c in cands], dtype=np.int32)
     model.cand_geom2 = np.array([c[1] for c in cands], dtype=np.int32)
@@ -915,6 +937,15 @@ def _compile_collision_candidates(model, pairs=()):
     model.cand_solimp = np.array([c[5] for c in cands], dtype=float).reshape(n, 5)
     model.cand_margin = np.array([c[6] for c in cands], dtype=float)
     model.cand_gap = np.array([c[7] for c in cands], dtype=float)
+
+
+def soft_pair_model(model):
+    """The model as MuJoCo solves it: a copy whose hard frictionless pairs (kind 21) are the soft
+    pyramidal pairs (kind 20, mu at the floor) the reference writes.  This is what a
+    double-precision reference solver takes to check the hard rows against."""
+    out = copy.copy(model)
+    out.cand_end = np.where(model.cand_end == 21, 20, model.cand_end).astype(np.int32)
+    return out
 
 
 def forward_kinematics(model, qpos):

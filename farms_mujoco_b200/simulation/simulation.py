@@ -49,6 +49,8 @@ class Simulation:
         self.options = simulation_options
         self.pause = not self.options.play
         self.handle_exceptions = kwargs.pop('handle_exceptions', False)
+        # frictionless <pair>s (the reference's self-collisions): see mjcf_subset.parse_mjcf
+        frictionless_pairs = kwargs.pop('frictionless_pairs', 'refuse')
         engine_kwargs = extract_sub_dict(kwargs, (
             'n_envs', 'links_names', 'joints_names', 'contacts_names', 'xfrc_names', 'arena_options',
             'device', 'team_lanes', 'library', 'qpos0', 'qvel0'))
@@ -65,7 +67,7 @@ class Simulation:
         self._qpos0, self._qvel0 = engine_kwargs.pop('qpos0', None), engine_kwargs.pop('qvel0', None)
         buffer_size = kwargs.get('buffer_size', 0) or self.options.buffer_size or self.options.n_iterations
         kwargs['buffer_size'] = buffer_size
-        model = parse_mjcf(mjcf_model) if isinstance(mjcf_model, str) else mjcf_model
+        model = parse_mjcf(mjcf_model, frictionless_pairs=frictionless_pairs) if isinstance(mjcf_model, str) else mjcf_model
         animat_options = kwargs.get('animat_options')
         self.physics = BatchedPhysics(
             model, engine_kwargs.pop('n_envs', 1),

@@ -35,6 +35,13 @@ from test_emu_parity import _pair_case
 spec, model, qpos0, qvel0, ctrl = _pair_case(3)
 ph = BatchedPhysics.from_spec(spec, 3, buffer_size=6, library=lib)
 ph.reset(qpos0, qvel0); ph.set_ctrl(ctrl); ph.step(5); assert ph.log_arrays()['contacts'].any(); print('pairs ok')
+# frictionless pairs as hard normal rows (the working-set regions), alone and beside a mu = 0.5 pair
+from test_frictionless_pairs import _case
+for kind in ('pair', 'ground', 'mixed'):
+    spec, model, qpos0, qvel0, ctrl, _ = _case(kind, 3)
+    ph = BatchedPhysics.from_spec(spec, 3, buffer_size=6, library=lib, frictionless_pairs='hard')
+    ph.reset(qpos0, qvel0); ph.set_ctrl(ctrl); ph.step(5); assert ph.log_arrays()['contacts'].any() and not ph.flags.any()
+    print('frictionless pairs', kind, 'ok')
 # the stand-alone drag operator
 from drag_cases import check_operator
 print('drag operator', check_operator(lib, n=33))

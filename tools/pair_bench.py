@@ -1,8 +1,11 @@
 """Throughput of the team kernel on a model with explicit <pair> self-collisions (dense Newton
-Hessian while a pair contact is active) next to the same model without the pairs, device-timed.
+Hessian while a pair contact is active), on the same model with the reference's frictionless pairs
+solved as hard normal rows (frictionless_pairs='hard', tree-sparse Hessian), and on the same pose
+without the pairs, device-timed in one process.
 usage: python tools/pair_bench.py [n_envs]"""
 import json
 import os
+import subprocess
 import sys
 
 import numpy as np
@@ -17,13 +20,21 @@ from farms_mujoco_b200.engine import BatchedPhysics  # noqa: E402
 n = int(sys.argv[1]) if len(sys.argv) > 1 else 4096
 inner, launches = 16, 6
 out = {'n_envs': n, 'steps_per_launch': inner, 'launches': launches}
-for name, spec, fast in (('salamander_foot_pairs (team kernel, pair contacts active)', variant_models.salamander_foot_pairs(), None),
-                         ('salamander_swim forced onto the team kernel, same pose', models.salamander(swimming=True), 0)):
-    model = mjcf_subset.parse_mjcf(spec.mjcf)
+try:
+    out['gpu'] = subprocess.run(['nvidia-smi', '--query-gpu=name,power.limit', '--format=csv,noheader'],
+                                capture_output=True, text=True, check=True).stdout.strip()
+except (OSError, subprocess.CalledProcessError):
+    out['gpu'] = 'unknown'
+for name, spec, fast, fp in (
+        ('salamander_foot_pairs (team kernel, pair contacts active)', variant_models.salamander_foot_pairs(), None, 'refuse'),
+        ('salamander_foot_pairs frictionless, hard normal rows (team kernel, pair contacts active)',
+         variant_models.salamander_foot_pairs(friction=0), None, 'hard'),
+        ('salamander_swim forced onto the team kernel, same pose', models.salamander(swimming=True), 0, 'refuse')):
+    model = mjcf_subset.parse_mjcf(spec.mjcf, frictionless_pairs=fp)
     rng = np.random.default_rng(0)
     qpos0 = np.tile(variant_models.folded_legs_qpos(model, 1.0), (n, 1))
     qpos0[:, 7:] += rng.uniform(-0.03, 0.03, (n, model.nq - 7))
-    ph = BatchedPhysics.from_spec(spec, n, buffer_size=inner + 1)
+    ph = BatchedPhysics.from_spec(spec, n, buffer_size=inner + 1, frictionless_pairs=fp)
     if fast is not None:
         ph.set_fast_path(fast)
     # hold the folded pose: the position actuators' targets are the initial joint angles
@@ -42,6 +53,6 @@ for name, spec, fast in (('salamander_foot_pairs (team kernel, pair contacts act
     pair = [i for i, c in enumerate(spec.contacts_names) if c[1]]
     active = float((np.abs(ph.log_row('contacts', inner)[:, pair, 6:9]).max(axis=(1, 2)) > 0).mean()) if pair else 0.0
     out[name] = {'ms_per_launch': float(np.median(ms)), 'env_steps_per_s': n*inner/(np.median(ms)*1e-3),
-                 'team_lanes': ph.team_lanes, 'fast_path': ph.fast_path,
+                 'team_lanes': ph.team_lanes, 'fast_path': ph.fast_path, 'envs_flagged': int(np.count_nonzero(ph.flags)),
                  'envs_with_an_active_pair_contact_in_the_last_row': active}
 print(json.dumps(out, indent=1))

@@ -1,7 +1,8 @@
 """Soak of the pair-contact path (team kernel, dense Newton Hessian): SALAMANDERs with explicit
 foot-foot <pair>s, the legs driven around the folded pose so that the feet meet and part again,
-on the ground (plane contacts and pair contacts in one solve).
-usage: python tools/pair_soak.py <n_envs> <launches of 16 steps>"""
+on the ground (plane contacts and pair contacts in one solve).  With --frictionless: the reference's
+frictionless pairs, solved as hard normal rows (frictionless_pairs='hard').
+usage: python tools/pair_soak.py <n_envs> <launches of 16 steps> [library] [--frictionless]"""
 import os
 import sys
 import time
@@ -15,18 +16,21 @@ import variant_models  # noqa: E402
 from farms_mujoco_b200 import mjcf_subset  # noqa: E402
 from farms_mujoco_b200.engine import BatchedPhysics  # noqa: E402
 
-n, launches = int(sys.argv[1]), int(sys.argv[2])
-library = sys.argv[3] if len(sys.argv) > 3 else None
+frictionless = '--frictionless' in sys.argv
+args = [a for a in sys.argv[1:] if a != '--frictionless']
+n, launches = int(args[0]), int(args[1])
+library = args[2] if len(args) > 2 else None
+fp = 'hard' if frictionless else 'refuse'
 # (in water the folded pose itself goes unstable after ~400 steps -- in the fp64 oracle too: explicit
 # Euler under the legs' drag -- so the soak runs on the ground, plane and pair contacts in one solve)
 for swimming in (False,):
-    spec = variant_models.salamander_foot_pairs(swimming=swimming)
-    model = mjcf_subset.parse_mjcf(spec.mjcf)
+    spec = variant_models.salamander_foot_pairs(swimming=swimming, **({'friction': 0} if frictionless else {}))
+    model = mjcf_subset.parse_mjcf(spec.mjcf, frictionless_pairs=fp)
     rng = np.random.default_rng(0)
     fold = variant_models.folded_legs_qpos(model, 1.0)
     qpos0 = np.tile(fold, (n, 1))
     qpos0[:, 7:] += rng.uniform(-0.03, 0.03, (n, model.nq - 7))
-    ph = BatchedPhysics.from_spec(spec, n, buffer_size=17, library=library)
+    ph = BatchedPhysics.from_spec(spec, n, buffer_size=17, library=library, frictionless_pairs=fp)
     ph.reset(qpos0, None)
     names = [tuple(c) for c in spec.contacts_names]
     pair = [i for i, c in enumerate(names) if c[1]]
@@ -52,7 +56,7 @@ for swimming in (False,):
         broken += int((~now & was).sum())
         was = now
     f = ph.flags
-    print('salamander_foot_pairs', 'water' if swimming else 'ground', n, 'envs', launches*16, 'steps', 'sec %.2f' % (time.time() - t0),
+    print('salamander_foot_pairs' + (' frictionless (hard rows)' if frictionless else ''), 'water' if swimming else 'ground', n, 'envs', launches*16, 'steps', 'sec %.2f' % (time.time() - t0),
           'nonfinite', int(np.count_nonzero(f & 1)), 'solver', int(np.count_nonzero(f & 4)),
           'pair contacts made', made, 'broken', broken, 'finite state', bool(np.isfinite(ph.qpos).all()),
           'max|qvel| %.2f' % np.abs(ph.qvel).max())
