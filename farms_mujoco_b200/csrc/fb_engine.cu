@@ -107,14 +107,11 @@ fb_fast_kernel(const __grid_constant__ FbFastParams Q) {
   const int valid = env < P.n_envs;
   if (!MULTI && !valid) return;
   const int n_float = SLIM ? P.m.X.n_float_slim : P.m.X.n_float;
-  /* multi-warp SLIM blocks stage the scratch through a TMA ring behind the warp's body blocks */
-  constexpr int TMA = FB_TMA_ENABLE && SLIM && MULTI;
-  const size_t warp_floats = (size_t)n_float*BLK + (TMA ? FB_RING_BYTES/sizeof(float) : 0);
+  const size_t warp_floats = (size_t)n_float*BLK;
   /* L2-resident scratch [warp][field][lane]: compile-time strides, coalesced */
-  FbFast<BLK, SLIM, TMA, LEAN> st(P, Q.rec, fb_smem + warp*warp_floats + lane,
-                            P.fast_scratch + (size_t)wid*(SLIM ? P.m.X.n_scratch_slim : P.m.X.n_scratch)*BLK + lane,
-                            valid ? env : 0);
-  if (TMA) st.ring_setup(fb_smem + warp*warp_floats + (size_t)n_float*BLK, lane);
+  FbFast<BLK, SLIM, LEAN> st(P, Q.rec, fb_smem + warp*warp_floats + lane,
+                             P.fast_scratch + (size_t)wid*(SLIM ? P.m.X.n_scratch_slim : P.m.X.n_scratch)*BLK + lane,
+                             valid ? env : 0);
   /* full warps move their state through a shared-memory tile (coalesced); a partial last
    * warp, or a model whose state rows do not fit the tile, uses per-thread accesses (the SLIM
    * layout's smaller blocks take the rows in two phases) */
@@ -152,8 +149,8 @@ fb_fast_split_kernel(const __grid_constant__ FbFastSplitParams Q) {
   if (blockIdx.x == 0 && threadIdx.x == 0) P.pending_count[P.parity ^ 1] = 0;   /* for the next launch */
   const int valid = env < P.n_envs;
   const int n_float = P.m.X.n_float;
-  FbFast<32, 0, 0, LEAN, 1> st(P, Q.rec, fb_smem + lane, P.fast_scratch + (size_t)wid*P.m.X.n_scratch*32 + lane,
-                               valid ? env : 0);
+  FbFast<32, 0, LEAN, 1> st(P, Q.rec, fb_smem + lane, P.fast_scratch + (size_t)wid*P.m.X.n_scratch*32 + lane,
+                            valid ? env : 0);
   float *extra = fb_smem + (size_t)n_float*32;
   st.split_setup(Q.split, role, extra + lane, reinterpret_cast<int *>(extra + 3*32) + lane);
   const int coop = (wid + 1)*32 <= P.n_envs ? P.m.X.coop_io : 0;
@@ -616,11 +613,11 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
         emu_split_run(sp.nwarps, [&](int role) {
           int d;
           if (lean) {
-            FbFast<1, 0, 0, 1, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env);
+            FbFast<1, 0, 1, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env);
             st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
             d = st.run_split(0, 0, 1);
           } else {
-            FbFast<1, 0, 0, 0, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env);
+            FbFast<1, 0, 0, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env);
             st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
             d = st.run_split(0, 0, 1);
           }
@@ -628,9 +625,9 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
         });
         done = done0;
       } else
-      if (h->fast_slim && lean) { FbFast<1, 1, 0, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env); done = st.run(0, 0); }
+      if (h->fast_slim && lean) { FbFast<1, 1, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env); done = st.run(0, 0); }
       else if (h->fast_slim) { FbFast<1, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env); done = st.run(0, 0); }
-      else if (lean) { FbFast<1, 0, 0, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env); done = st.run(0, 0); }
+      else if (lean) { FbFast<1, 0, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env); done = st.run(0, 0); }
       else { FbFast<1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env); done = st.run(0, 0); }
       if (done < n_steps) { P.steps_done[env] = done; P.pending[P.pending_count[P.parity]++] = env; }
     }
@@ -701,7 +698,6 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
       const int warps = (P.n_envs + 31)/32;
       const int wblocks = (warps + wpb - 1)/wpb;
       size_t bytes = (h->fast_slim ? h->fast_slim_smem_bytes : h->fast_smem_bytes)*(h->fast_block == 32 ? wpb : 1);
-      if (FB_TMA_ENABLE && h->fast_slim && wpb > 1) bytes += (size_t)wpb*FB_RING_BYTES;      /* TMA ring of every warp */
       /* LEAN variants: same arithmetic with the model's unused paths compiled out (smaller loops) */
       const bool lean = h->fast_lean && P.m.X.lean && !P.ctrl_seq;
       if (h->fast_split && h->fast_block == 32 && !h->fast_slim && h->hm.split.nwarps > 1 && warps <= h->split_capacity) {
@@ -886,15 +882,15 @@ static int fb_set_fast_block(FbHandle *h, int blk) {
 static int fb_slim_attributes(FbHandle *h, int max_smem) {
   h->fast_slim_smem_bytes = (size_t)h->hm.m.X.n_float_slim*sizeof(float)*32;
   const int b1 = (int)h->fast_slim_smem_bytes;
-  int fit = max_smem/(b1 + (FB_TMA_ENABLE ? FB_RING_BYTES : 0));     /* warps of one block (body blocks + TMA ring each) that fit an SM's shared memory */
+  int fit = max_smem/b1;     /* warps of one block that fit an SM's shared memory */
   if (fit > 8) fit = 8;
   cudaError_t ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, b1);
   if (ce == cudaSuccess) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 0>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (ce == cudaSuccess) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, b1);
   if (ce == cudaSuccess) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 0, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  if (ce == cudaSuccess && fit >= 2) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fit*(b1 + (FB_TMA_ENABLE ? FB_RING_BYTES : 0)));
+  if (ce == cudaSuccess && fit >= 2) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fit*b1);
   if (ce == cudaSuccess) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  if (ce == cudaSuccess && fit >= 2) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fit*(b1 + (FB_TMA_ENABLE ? FB_RING_BYTES : 0)));
+  if (ce == cudaSuccess && fit >= 2) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fit*b1);
   if (ce == cudaSuccess) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 1, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   if (ce != cudaSuccess) return fail(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ce));
   if (h->fast_wpb > fit) h->fast_wpb = fit;

@@ -190,102 +190,17 @@ FB_DEV void fb_sincos_half(float x, float *sn, float *cs) {
 #define FB_PIN_I(x) asm volatile("" :: "r"(x))
 #endif
 
-/* SLIM = 1 (large batches, unconstrained kernel only): the shared-memory block of a body holds
- * its pose only (7 floats); velocities and the accumulation slots of the branching bodies move to
- * the L2 scratch, fetched one body ahead like the rest of it.  203 instead of 431 floats of
- * shared memory per SALAMANDER: 8 warps of environments per SM instead of 4, i.e. two warps per
- * scheduler to hide each other's latencies, which pays once the batch has that many warps. */
-#ifndef FB_HOST_EMU
-/* ---- TMA bulk copies global -> shared memory with mbarrier completion (sm_90+ PTX; SASS UBLKCP /
- * SYNCS).  One elected lane arms the barrier with the byte count and issues the copy; every lane
- * of the warp waits on the barrier's phase and then reads the staged block with LDS. */
-FB_DEV unsigned fb_smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
-FB_DEV void fb_mbar_init(unsigned bar, unsigned count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(bar), "r"(count) : "memory");
-}
-FB_DEV void fb_mbar_expect_tx(unsigned bar, unsigned bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" :: "r"(bar), "r"(bytes) : "memory");
-}
-FB_DEV void fb_bulk_g2s(unsigned dst, const void *src, unsigned bytes, unsigned bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               :: "r"(dst), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-FB_DEV void fb_mbar_wait(unsigned bar, unsigned parity) {
-  asm volatile(
-      "{\n"
-      ".reg .pred P1;\n"
-      "LAB_WAIT:\n"
-      "mbarrier.try_wait.parity.shared::cta.b64 P1, [%0], %1;\n"
-      "@P1 bra DONE;\n"
-      "bra LAB_WAIT;\n"
-      "DONE:\n"
-      "}" :: "r"(bar), "r"(parity) : "memory");
-}
-/* generic-proxy writes (st.global of the scratch) before async-proxy reads (the bulk copies) */
-#ifndef FB_TMA_FENCE
-#define FB_TMA_FENCE 1
-#endif
-FB_DEV void fb_fence_proxy_async() {
-#if FB_TMA_FENCE == 2
-  asm volatile("fence.proxy.async;" ::: "memory");            /* + MEMBAR.ALL.GPU: measured, not needed */
-#elif FB_TMA_FENCE == 1
-  asm volatile("fence.proxy.async.global;" ::: "memory");     /* FENCE.VIEW.ASYNC.G */
-#endif
-}
-#endif
-
-/* stages of the TMA scratch ring (FbFast<.., TMA = 1>): a body's block is requested RING - 1
- * bodies before it is used */
-#ifndef FB_RING
-#define FB_RING 3
-#endif
-/* Off by default: measured r2d on B200, 65,536 SALAMANDERs, 7 warps per block -- 3.61 ms per launch
- * with the ring (bit-identical results; RING 2 or 3, with or without the proxy fences: 3.58 .. 3.61)
- * against 3.12 ms with the register prefetch.  A body's iteration then starts with
- * __syncwarp -> one lane arms the barrier and issues UBLKCP -> every lane polls the mbarrier -> 17 LDS,
- * a serial prefix of 100-200 cycles x 87 body visits per step that the register prefetch does not
- * have, and the ring's 6.5 KB per warp cost the eighth warp of a block.  Build with
- * -DFB_TMA_ENABLE=1 to reproduce (tools/variant_bench.sh). */
-#ifndef FB_TMA_ENABLE
-#define FB_TMA_ENABLE 0
-#endif
-#define FB_RING_FIELDS 17      /* W[6] U 1/d trq q qd V[6]: the fields the sweeps read, contiguous */
-/* shared memory of one warp's ring: the stages + one 8-byte mbarrier per stage, padded to 128 B */
-#define FB_RING_BYTES ((FB_RING*FB_RING_FIELDS*32*4 + 8*FB_RING + 127)/128*128)
-
-/* body loops of the three sweeps: -DFB_BODY_UNROLL=2 lets ptxas overlap the tail of one body with
- * the head of the next (measured, see DESIGN.md; default: not unrolled) */
-#if defined(FB_BODY_UNROLL) && !defined(FB_HOST_EMU)
-#define FB_STR_(x) #x
-#define FB_STR(x) FB_STR_(x)
-#define FB_BODY_LOOP _Pragma(FB_STR(unroll FB_BODY_UNROLL))
-#else
-#define FB_BODY_LOOP
-#endif
-
-/* Touch the record of the body visited NEXT (one word per 64-byte line of its 288 bytes) so that the
- * indexed constant loads of the next iteration hit the constant cache: the table (8 KB for 29
- * bodies) is larger than its first level, and a lone warp waits out every miss.  Off by default
- * (-DFB_REC_PREFETCH=1 compiles it in): measured r2q +0.2 .. 0.8 %, within noise. */
-#ifndef FB_REC_PREFETCH
-#define FB_REC_PREFETCH 0
-#endif
-#if FB_REC_PREFETCH && !defined(FB_HOST_EMU)
-#define FB_TOUCH_REC(r_) do { const int *w_ = reinterpret_cast<const int *>(&(r_)); \
-  FB_PIN_I(w_[0]); FB_PIN_I(w_[16]); FB_PIN_I(w_[32]); FB_PIN_I(w_[48]); FB_PIN_I(w_[64]); } while (0)
-#else
-#define FB_TOUCH_REC(r_) do { } while (0)
-#endif
-
 template <int SYNC> FB_DEV void fb_block_sync() {
 #ifndef FB_HOST_EMU
   if (SYNC) __syncthreads();
 #endif
 }
 
-/* TMA = 1 (SLIM layout in multi-warp blocks): the per-body scratch block is not fetched into
- * registers one body ahead (16-17 long-lived LDG results per thread that tie up a scoreboard:
- * r2a's top stalls) but staged in a small shared-memory ring by bulk copies, two bodies ahead. */
+/* SLIM = 1 (large batches, unconstrained kernel only): the shared-memory block of a body holds
+ * its pose only (7 floats); velocities and the accumulation slots of the branching bodies move to
+ * the L2 scratch, fetched one body ahead like the rest of it.  203 instead of 431 floats of
+ * shared memory per SALAMANDER: 8 warps of environments per SM instead of 4, i.e. two warps per
+ * scheduler to hide each other's latencies, which pays once the batch has that many warps. */
 /* LEAN = 1: the model (DevFastLayout::lean) has hinge joints only, anchors at the body origins,
  * axisymmetric inertias, the linear actuation form on every joint and the farms joints-row layout,
  * and the launch reads no control sequence: the slide-joint, general-inertia, generic-actuation,
@@ -296,7 +211,7 @@ template <int SYNC> FB_DEV void fb_block_sync() {
  * warps, each visiting its own bodies of the tree in two phases per sweep (FastSplit, fb_model.h);
  * the per-body code is the one every other variant runs, in the same order along every chain, so
  * the results are bit-identical to the single-warp kernel. */
-template <int BLK, int SLIM = 0, int TMA = 0, int LEAN = 0, int SPLIT = 0> struct FbFast {
+template <int BLK, int SLIM = 0, int LEAN = 0, int SPLIT = 0> struct FbFast {
   /* SLIM scratch block: W[6] U 1/d trq q qd V[6] tc tu -- the first 17 are one contiguous run */
   enum { NF = SLIM ? 7 : FB_NF, GNF = SLIM ? FG_NF + 6 : FG_NF, FG_V = SLIM ? 11 : FG_NF,
          FGTC = SLIM ? 17 : FG_TC, FGTU = SLIM ? 18 : FG_TU };
@@ -321,11 +236,6 @@ template <int BLK, int SLIM = 0, int TMA = 0, int LEAN = 0, int SPLIT = 0> struc
    * (FbParams::con_dirty), zfill = verdict for the current step */
   long long dirty_c;
   int zfill;
-  /* TMA ring of this warp: shared-memory stages, their mbarriers, the parity each barrier
-   * completes next, and the lane */
-  float *ring;
-  unsigned ring_bar, ring_phase;
-  int ring_lane;
   /* SPLIT: this warp's body list (ascending; phase A = [0, ord_bnd)), its role (0 = the trunk warp,
    * which also owns the root state and the state I/O), whether this lane's environment has left
    * the kernel (it still takes every barrier), the root position as warp 0 publishes it and the
@@ -340,7 +250,6 @@ template <int BLK, int SLIM = 0, int TMA = 0, int LEAN = 0, int SPLIT = 0> struc
     env_phase = P.env_phase[env];
     dirty_c = P.con_dirty[env];
     zfill = 1;
-    ring = 0; ring_bar = 0; ring_phase = 0; ring_lane = 0;
     ord = 0; ord_n = 0; ord_bnd = 0; role = 0; idle = 0; sroot = 0; sflag = 0;
     rootpos[0] = rootpos[1] = rootpos[2] = 0.f;
     rqn[0] = 1.f; rqn[1] = rqn[2] = rqn[3] = 0.f;
@@ -348,35 +257,6 @@ FB_UNROLL
     for (int k = 0; k < 13; k++) rt[k] = 0.f;
   }
 
-#ifndef FB_HOST_EMU
-  /* ---- TMA ring.  ring_setup: once per kernel, by every lane of the warp. */
-  FB_MEM void ring_setup(float *ring_base, int lane) {
-    ring = ring_base; ring_lane = lane; ring_phase = 0;
-    ring_bar = fb_smem_u32(ring_base + FB_RING*FB_RING_FIELDS*32);
-    if (lane == 0) {
-FB_UNROLL
-      for (int k = 0; k < FB_RING; k++) fb_mbar_init(ring_bar + 8*k, 1);
-      asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncwarp();
-  }
-  /* request the block of body b into stage st (the stage's previous content has been read:
-   * callers put a __syncwarp() between those reads and this call) */
-  FB_MEM void ring_issue(int leader, int b, int st, int f0, int nf) {
-    if (ring_lane == leader) {
-      const unsigned bar = ring_bar + 8*st, bytes = nf*32*sizeof(float);
-      fb_mbar_expect_tx(bar, bytes);
-      fb_bulk_g2s(fb_smem_u32(ring + (st*FB_RING_FIELDS + f0)*32),
-                  gs - ring_lane + ((size_t)GNF*(b - 1) + f0)*BLK, bytes, bar);
-    }
-  }
-  /* wait for stage st; returns this lane's view of it: field f at [f*32] */
-  FB_MEM const float *ring_wait(int st) {
-    fb_mbar_wait(ring_bar + 8*st, (ring_phase >> st) & 1u);
-    ring_phase ^= 1u << st;
-    return ring + st*FB_RING_FIELDS*32 + ring_lane;
-  }
-#endif
   FB_MEM void split_setup(const FastSplit &sp, int role_, float *sroot_, int *sflag_) {
     role = role_; ord = sp.order[role_]; ord_n = sp.n[role_]; ord_bnd = sp.boundary[role_];
     sroot = sroot_; sflag = sflag_;
@@ -459,6 +339,19 @@ FB_UNROLL
     if (P.n_spring <= 0) return;
     for (int b = 1; b < m.nbody; b++)
       if (FT_SREF(rec[b].flags) >= 0) P.qpos_spring[(size_t)env*m.nq + rec[b].qa] = last[(long long)(m.nu + FT_SREF(rec[b].flags))*P.env_pad];
+  }
+  /* end of a launch of n steps with a control sequence: ctrl ends as the last entry used, as if
+   * the host had set it step by step (the wave-driven actuators keep what the last step wrote) */
+  FB_MEM void store_seq_end(int n) const {
+    const size_t e = (size_t)env;
+    const float *last = P.ctrl_seq + ((size_t)(P.seq_pos + n - 1)*P.seq_stride)*P.env_pad + e;
+    for (int a = 0; a < m.nu; a++)
+      if (MI(ft_actwc, a) < 0) P.ctrl[e*m.nu + a] = last[(long long)a*P.env_pad];
+    store_springrefs(last);
+  }
+  /* no contact is active in this step: its contacts row is zero (sensors.pyx:140-190) */
+  FB_MEM void zero_contacts(float *row_contacts) const {
+    for (int i = 0; i < m.n_contacts*3; i++) fb_st4(row_contacts + i*(P.env_pad*FB_VEC_CONTACTS), 0.f, 0.f, 0.f, 0.f);
   }
 
   /* joint half of load_state: root state into registers, q / qd and the constant part of the
@@ -612,22 +505,8 @@ FB_UNROLL
     const int nb = m.nbody;
     int active = 0;
     /* scratch values are fetched one body ahead: the L2 round trip overlaps the arithmetic */
-    float nq = 0.f, nqd = 0.f;
-#ifndef FB_HOST_EMU
-    /* (TMA) the lanes that take this step: one of them issues the copies, all of them wait */
-    const unsigned live = TMA ? __activemask() : 0u;
-    const int leader = TMA ? __ffs(live) - 1 : 0;
-    int st = 0;
-    if (TMA) {
-FB_UNROLL
-      for (int d = 0; d < FB_RING - 1; d++)
-        if (1 + d < nb) ring_issue(leader, 1 + d, d, FG_Q, 2);
-    } else
-#endif
-    {
-      const int b0 = SPLIT ? (ord_n > 0 ? ord[0] : 1) : 1;
-      nq = fb_ld_scr(gblock(b0) + FG_Q*BLK); nqd = fb_ld_scr(gblock(b0) + FG_QD*BLK);
-    }
+    const int b0 = SPLIT ? (ord_n > 0 ? ord[0] : 1) : 1;
+    float nq = fb_ld_scr(gblock(b0) + FG_Q*BLK), nqd = fb_ld_scr(gblock(b0) + FG_QD*BLK);
     const int n_it = SPLIT ? ord_n : nb - 1;
     float *pb = block(1) - NF*BLK;
     float *pn = gblock(1);
@@ -638,7 +517,6 @@ FB_UNROLL
      * from the scratch while the previous body is computed -- issued at its use it cost a full L2
      * round trip per branch (r1aq: 6 % of the stall samples together with its pass-3 twin) */
     float nvp[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-FB_BODY_LOOP
     for (int i = 0; i <= n_it; i++) {
       if (SPLIT && i == ord_bnd) {
         split_barrier();                 /* the trunk is placed: the subtrees hanging off it start */
@@ -665,20 +543,9 @@ FB_UNROLL
       for (int k = 0; k < 3; k++) { FB_PIN_F(rc.dpos[k]); FB_PIN_F(rc.axis[k]); FB_PIN_F(rc.hloc[k]); }
 FB_UNROLL
       for (int k = 0; k < 4; k++) { FB_PIN_F(rc.bquat[k]); FB_PIN_F(rc.chk[k]); }
-      if (bn) FB_TOUCH_REC(rec[bn]);
       if (SPLIT) { pb = block(b); pn = gblock(bn ? bn : b); }
       else { pb += NF*BLK; pn += GNF*BLK; }
-      float cq = nq, cqd = nqd;
-#ifndef FB_HOST_EMU
-      if (TMA) {
-        __syncwarp(live);                 /* the stage requested next was read in the previous iteration */
-        const int sn = st == 0 ? FB_RING - 1 : st - 1;
-        if (b + FB_RING - 1 < nb) ring_issue(leader, b + FB_RING - 1, sn, FG_Q, 2);
-        const float *sb = ring_wait(st);
-        cq = sb[FG_Q*32]; cqd = sb[FG_QD*32];
-        st = st + 1 == FB_RING ? 0 : st + 1;
-      } else
-#endif
+      const float cq = nq, cqd = nqd;
       if (bn) { nq = fb_ld_scr(pn + FG_Q*BLK); nqd = fb_ld_scr(pn + FG_QD*BLK); }
       float *pgv = SPLIT ? gblock(b) : pn - GNF*BLK;       /* scratch block of this body (pn runs one ahead) */
       const int jtype = rc.jtype;
@@ -821,9 +688,6 @@ FB_UNROLL
         fb_st4(row + 4*ev, (v[5] + cr[2])*iv, v[0]*iw, v[1]*iw, v[2]*iw);
       }
     }
-#ifndef FB_HOST_EMU
-    if (TMA) fb_fence_proxy_async();      /* the velocities just stored are bulk-copied by pass 2 */
-#endif
     return active;
   }
 
@@ -847,33 +711,20 @@ FB_UNROLL
     for (int k = 0; k < 9; k++) C.H[k] = 0.f;
     float nx[10] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};        /* W[6], q, qd, tc, tu of the next body to visit */
     float nxv[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};     /* SLIM: its velocity */
-#ifndef FB_HOST_EMU
-    const unsigned live = TMA ? __activemask() : 0u;
-    const int leader = TMA ? __ffs(live) - 1 : 0;
-    int st = 0;
-    if (TMA) {
-FB_UNROLL
-      for (int d = 0; d < FB_RING - 1; d++)
-        if (nb - 1 - d >= 1) ring_issue(leader, nb - 1 - d, d, 0, FB_RING_FIELDS);
-    }
-#endif
     const int n_it = SPLIT ? ord_n : nb - 1;
     {
       const float *pn = gblock(SPLIT ? (ord_n > 0 ? ord[ord_n - 1] : 1) : nb - 1);
-      if (!TMA) {
 FB_UNROLL
-        for (int k = 0; k < 6; k++) nx[k] = fb_ld_scr(pn + (FG_W + k)*BLK);
-        nx[6] = fb_ld_scr(pn + FG_Q*BLK); nx[7] = fb_ld_scr(pn + FG_QD*BLK);
-      }
+      for (int k = 0; k < 6; k++) nx[k] = fb_ld_scr(pn + (FG_W + k)*BLK);
+      nx[6] = fb_ld_scr(pn + FG_Q*BLK); nx[7] = fb_ld_scr(pn + FG_QD*BLK);
       nx[8] = fb_ld_scr(pn + FGTC*BLK); nx[9] = fb_ld_scr(pn + FGTU*BLK);
-      if (SLIM && !TMA) {
+      if (SLIM) {
 FB_UNROLL
         for (int k = 0; k < 6; k++) nxv[k] = fb_ld_scr(pn + (FG_V + k)*BLK);
       }
     }
     float *pb = block(nb - 1) + NF*BLK;
     float *pg = gblock(nb - 1) + GNF*BLK;
-FB_BODY_LOOP
     for (int i = n_it; i >= 0; i--) {
       if (SPLIT && i == ord_bnd) split_barrier();      /* the subtrees have handed over: the trunk goes on */
       if (i == 0) break;
@@ -890,7 +741,6 @@ FB_UNROLL
       for (int k = 0; k < 3; k++) { FB_PIN_F(rc.hloc[k]); FB_PIN_F(rc.axis[k]); }
 FB_UNROLL
       for (int k = 0; k < 5; k++) FB_PIN_F(rc.Ib[k]);
-      if (bn) FB_TOUCH_REC(rec[bn]);
       if (SPLIT) { pb = block(b); pg = gblock(b); }
       else { pb -= NF*BLK; pg -= GNF*BLK; }
       const int jtype = rc.jtype, flags = rc.flags;
@@ -901,29 +751,15 @@ FB_UNROLL
       for (int k = 0; k < 6; k++) cxv[k] = nxv[k];
       if (bn) {
         const float *pn = SPLIT ? gblock(bn) : pg - GNF*BLK;
-        if (!TMA) {
 FB_UNROLL
-          for (int k = 0; k < 6; k++) nx[k] = fb_ld_scr(pn + (FG_W + k)*BLK);
-          nx[6] = fb_ld_scr(pn + FG_Q*BLK); nx[7] = fb_ld_scr(pn + FG_QD*BLK);
-        }
+        for (int k = 0; k < 6; k++) nx[k] = fb_ld_scr(pn + (FG_W + k)*BLK);
+        nx[6] = fb_ld_scr(pn + FG_Q*BLK); nx[7] = fb_ld_scr(pn + FG_QD*BLK);
         nx[8] = fb_ld_scr(pn + FGTC*BLK); nx[9] = fb_ld_scr(pn + FGTU*BLK);
-        if (SLIM && !TMA) {
+        if (SLIM) {
 FB_UNROLL
           for (int k = 0; k < 6; k++) nxv[k] = fb_ld_scr(pn + (FG_V + k)*BLK);
         }
       }
-#ifndef FB_HOST_EMU
-      if (TMA) {
-        __syncwarp(live);
-        const int sn = st == 0 ? FB_RING - 1 : st - 1;
-        if (b - (FB_RING - 1) >= 1) ring_issue(leader, b - (FB_RING - 1), sn, 0, FB_RING_FIELDS);
-        const float *sb = ring_wait(st);
-FB_UNROLL
-        for (int k = 0; k < 6; k++) { cx[k] = sb[(FG_W + k)*32]; cxv[k] = sb[(FG_V + k)*32]; }
-        cx[6] = sb[FG_Q*32]; cx[7] = sb[FG_QD*32];
-        st = st + 1 == FB_RING ? 0 : st + 1;
-      }
-#endif
       const Quat q = {pb[(FB_QUAT)*BLK], pb[(FB_QUAT + 1)*BLK], pb[(FB_QUAT + 2)*BLK], pb[(FB_QUAT + 3)*BLK]};
       float R[9], v[6], fx[6];
       q_mat(q, R);
@@ -1133,9 +969,6 @@ FB_UNROLL
         }
       }
     }
-#ifndef FB_HOST_EMU
-    if (TMA) fb_fence_proxy_async();      /* U, u, 1/d, trq just stored are bulk-copied by pass 3 */
-#endif
   }
 
   /* ---- pass 3: root -> leaves, accelerations, Euler, joints / xfrc rows, drag */
@@ -1151,18 +984,8 @@ FB_UNROLL
     int bad = 0;
     float nx[11] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};   /* U[6], u, 1/d, trq, q, qd of the next body to visit */
     float nxv[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};     /* SLIM: its velocity */
-#ifndef FB_HOST_EMU
-    const unsigned live = TMA ? __activemask() : 0u;
-    const int leader = TMA ? __ffs(live) - 1 : 0;
-    int st = 0;
-    if (TMA) {
-FB_UNROLL
-      for (int d = 0; d < FB_RING - 1; d++)
-        if (1 + d < nb) ring_issue(leader, 1 + d, d, 0, FB_RING_FIELDS);
-    }
-#endif
     const int n_it = SPLIT ? ord_n : nb - 1;
-    if (!TMA) {
+    {
       const float *pn = gblock(SPLIT ? (ord_n > 0 ? ord[0] : 1) : 1);
 FB_UNROLL
       for (int k = 0; k < 9; k++) nx[k] = fb_ld_scr(pn + (FG_W + k)*BLK);     /* W, U, DINV, TRQ are contiguous */
@@ -1175,7 +998,6 @@ FB_UNROLL
     float *pb = block(1) - NF*BLK;
     float *pg = gblock(1) - GNF*BLK;
     float nap[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};     /* SLIM: acceleration of the parent of the next body when that is a branch child */
-FB_BODY_LOOP
     for (int i = 0; i <= n_it; i++) {
       if (SPLIT && i == ord_bnd) split_barrier();      /* the trunk's accelerations are known */
       if (i == n_it) break;
@@ -1190,7 +1012,6 @@ FB_UNROLL
       for (int k = 0; k < 3; k++) { FB_PIN_F(rc.hloc[k]); FB_PIN_F(rc.axis[k]); }
 FB_UNROLL
       for (int k = 0; k < 6; k++) FB_PIN_F(rc.coef[k]);
-      if (bn) FB_TOUCH_REC(rec[bn]);
       if (SPLIT) { pb = block(b); pg = gblock(b); }
       else { pb += NF*BLK; pg += GNF*BLK; }
       const int jtype = rc.jtype, flags = rc.flags;
@@ -1199,7 +1020,7 @@ FB_UNROLL
       for (int k = 0; k < 11; k++) cx[k] = nx[k];
 FB_UNROLL
       for (int k = 0; k < 6; k++) cxv[k] = nxv[k];
-      if (!TMA && bn) {
+      if (bn) {
         const float *pn = SPLIT ? gblock(bn) : pg + GNF*BLK;
 FB_UNROLL
         for (int k = 0; k < 9; k++) nx[k] = fb_ld_scr(pn + (FG_W + k)*BLK);
@@ -1209,20 +1030,6 @@ FB_UNROLL
           for (int k = 0; k < 6; k++) nxv[k] = fb_ld_scr(pn + (FG_V + k)*BLK);
         }
       }
-#ifndef FB_HOST_EMU
-      if (TMA) {
-        __syncwarp(live);
-        const int sn = st == 0 ? FB_RING - 1 : st - 1;
-        if (b + FB_RING - 1 < nb) ring_issue(leader, b + FB_RING - 1, sn, 0, FB_RING_FIELDS);
-        const float *sb = ring_wait(st);
-FB_UNROLL
-        for (int k = 0; k < 9; k++) cx[k] = sb[(FG_W + k)*32];
-        cx[9] = sb[FG_Q*32]; cx[10] = sb[FG_QD*32];
-FB_UNROLL
-        for (int k = 0; k < 6; k++) cxv[k] = sb[(FG_V + k)*32];
-        st = st + 1 == FB_RING ? 0 : st + 1;
-      }
-#endif
       /* a body without an xfrc row keeps the user's wrench: fetched now, stored at the end of the
        * iteration (the slot held U during this step) */
       float uwr[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
@@ -1394,9 +1201,6 @@ FB_UNROLL
         for (int k = 0; k < 6; k++) fb_st_scr(pg + (FG_W + k)*BLK, uwr[k]);
       }
     }
-#ifndef FB_HOST_EMU
-    if (TMA) fb_fence_proxy_async();      /* q, qd, W just stored are bulk-copied by the next step's sweeps */
-#endif
     return bad;
   }
 
@@ -1411,9 +1215,6 @@ FB_UNROLL
   template <int SYNC>
   FB_MEM int run_t(int coop, int lane, int valid) {
     if (valid) load_state(coop, lane);
-#ifndef FB_HOST_EMU
-    if (TMA) fb_fence_proxy_async();      /* the scratch load_state filled is bulk-copied by the sweeps */
-#endif
     const size_t e = (size_t)env;
     const int n = P.n_steps;
     int kdone = n, dead = !valid;
@@ -1437,20 +1238,13 @@ FB_UNROLL
       fb_block_sync<SYNC>();
       if (dead) continue;
       int bad = pass_accel(aroot, row_joints, row_xfrc);
-      /* no contact is active on this path: the contacts rows are zero (sensors.pyx:140-190), which
-       * is what the log holds already unless a constrained step wrote this ring row before */
-      if (zfill)
-        for (int i = 0; i < m.n_contacts*3; i++) fb_st4(row_contacts + i*(P.env_pad*FB_VEC_CONTACTS), 0.f, 0.f, 0.f, 0.f);
+      /* the contacts rows are what the log holds already unless a constrained step wrote this ring
+       * row before */
+      if (zfill) zero_contacts(row_contacts);
       if (bad) FB_FLAG_OR(P.flags + env, FB_FLAG_NONFINITE);
     }
     if (!valid) return n;
-    if (P.ctrl_seq && kdone == n) {
-      /* ctrl ends as the last entry used, as if the host had set it step by step */
-      const float *last = P.ctrl_seq + ((size_t)(P.seq_pos + n - 1)*P.seq_stride)*P.env_pad + e;
-      for (int a = 0; a < m.nu; a++)
-        if (MI(ft_actwc, a) < 0) P.ctrl[e*m.nu + a] = last[(long long)a*P.env_pad];
-      this->store_springrefs(last);
-    }
+    if (P.ctrl_seq && kdone == n) store_seq_end(n);
     store_state(P.it0 + kdone, coop, lane);
     return kdone;
   }
@@ -1489,19 +1283,13 @@ FB_UNROLL
       FB_BLOCK_BARRIER();
       const int bad = pass_accel(aroot, row_joints, row_xfrc);
       if (!dead) {
-        if (zfill && role == 0)
-          for (int i = 0; i < m.n_contacts*3; i++) fb_st4(row_contacts + i*(P.env_pad*FB_VEC_CONTACTS), 0.f, 0.f, 0.f, 0.f);
+        if (zfill && role == 0) zero_contacts(row_contacts);
         if (bad) FB_FLAG_OR(P.flags + env, FB_FLAG_NONFINITE);
       }
     }
     FB_BLOCK_BARRIER();
     if (role != 0 || !valid) return n;
-    if (P.ctrl_seq && kdone == n) {
-      const float *last = P.ctrl_seq + ((size_t)(P.seq_pos + n - 1)*P.seq_stride)*P.env_pad + e;
-      for (int a = 0; a < m.nu; a++)
-        if (MI(ft_actwc, a) < 0) P.ctrl[e*m.nu + a] = last[(long long)a*P.env_pad];
-      this->store_springrefs(last);
-    }
+    if (P.ctrl_seq && kdone == n) store_seq_end(n);
     store_state(P.it0 + kdone, coop, lane);
     return kdone;
   }

@@ -68,17 +68,8 @@ static double *fb_emu_stats = 0;
  * another order than on one warp: results agree with the single-warp kernel to rounding, not bit
  * for bit. */
 #define FB_RED_MAX 8       /* values of one cross-warp reduction */
-/* Warm start of the constraint solver from the previous step's solution (steps of one launch).
- * OFF: on the bench workloads it takes the SALAMANDER from 3.38 Newton iterations per solve to one
- * line search along the guess + 1.82 iterations, the CENTIPEDE from 4.30 to 1 + 2.86 (host
- * emulation) -- but only the FIRST Newton step has its rounding error refined (sweep C), and after a
- * warm start that is no longer the large one: the CENTIPEDE's 12-step rollout error against the
- * oracle goes from 1.4e-6 to 1.4e-5 in qvel (SALAMANDER unchanged).  DESIGN.md section 4. */
-#ifndef FB_WARM_START
-#define FB_WARM_START 0
-#endif
-template <int BLK, int LEAN = 0, int SPLIT = 0> struct FbFastCon : FbFast<BLK, 0, 0, LEAN, SPLIT> {
-  typedef FbFast<BLK, 0, 0, LEAN, SPLIT> Base;
+template <int BLK, int LEAN = 0, int SPLIT = 0> struct FbFastCon : FbFast<BLK, 0, LEAN, SPLIT> {
+  typedef FbFast<BLK, 0, LEAN, SPLIT> Base;
   using Base::P; using Base::m; using Base::rec; using Base::s; using Base::env; using Base::gs;
   using Base::cs; using Base::csc; using Base::crec; using Base::hm; using Base::hany;
   using Base::rt; using Base::rootpos; using Base::rqn;
@@ -370,9 +361,7 @@ FB_UNROLL
    * space, classical MuJoCo qacc), and J a0 - aref of every candidate row.  Two carries: the
    * spatial acceleration with its velocity-product terms (what the recursion needs) and the
    * pure J a part (what the rows see). */
-  /* warm: this lane's previous step (of this launch) was a constrained one -- its solution is still
-   * in NB_A / NR_A, and p0 = a_prev - a0 goes where the solver keeps its direction (else p0 = 0) */
-  FB_MEM void smooth_accel(const float *aroot, int warm, int warm_any) {
+  FB_MEM void smooth_accel(const float *aroot) {
     const int nb = m.nbody;
     float ac[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, lc[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     float nx[9];      /* U[6], u, 1/d, qd of the next body to visit */
@@ -402,7 +391,6 @@ FB_UNROLL
         for (int k = 0; k < 8; k++) nx[k] = fb_ld_scr(pn1 + (NB_U + k)*BLK);
         nx[8] = fb_ld_scr(gblock(bn) + FG_QD*BLK);
       }
-      const float prev_a = warm_any ? fb_ld_scr(pn + NB_A*BLK) : 0.f;      /* the previous step's solution */
       const Quat q = {pb[(FB_QUAT)*BLK], pb[(FB_QUAT + 1)*BLK], pb[(FB_QUAT + 2)*BLK], pb[(FB_QUAT + 3)*BLK]};
       float R[9], v[6], a[6], al[6];
       q_mat(q, R);
@@ -416,10 +404,6 @@ FB_UNROLL
         for (int k = 0; k < 3; k++) {
           a[k] = aroot[k]; a[3 + k] = aroot[3 + k];
           al[k] = aroot[k]; al[3 + k] = aroot[3 + k] + m.grav[k] + cr[k];
-        }
-        if (warm_any) {
-FB_UNROLL
-          for (int k = 0; k < 6; k++) fb_st_scr(pr + (NR_P + k)*BLK, warm ? fb_ld_scr(pr + (NR_A + k)*BLK) - al[k] : 0.f);
         }
 FB_UNROLL
         for (int k = 0; k < 6; k++) { fb_st_scr(pr + (NR_A + k)*BLK, al[k]); fb_st_scr(pr + (NR_MD + k)*BLK, 0.f); }
@@ -469,7 +453,6 @@ FB_UNROLL
 FB_UNROLL
             for (int k = 0; k < 3; k++) { a[3 + k] += ax[k]*qdd; al[3 + k] += ax[k]*qdd; }
           }
-          if (warm_any) fb_st_scr(pn + NB_P*BLK, warm ? prev_a - qdd : 0.f);
           fb_st_scr(pn + NB_A*BLK, qdd);
           fb_st_scr(pn + NB_MD*BLK, 0.f);
         }
@@ -711,9 +694,7 @@ FB_UNROLL
 
   /* ---- Newton sweep B: root -> leaves.  p per joint, the bodies' pure accelerations, J p per
    * candidate row; g0 = p . g, pp = |p|^2 */
-  /* given = 1: the direction is already in NB_P / NR_P (warm start); only the bodies'
-   * accelerations, the rows' J p and |p|^2 are computed (p . g is left 0) */
-  FB_MEM void newton_b(float *g0_out, float *pp_out, int store_ap, int given) {
+  FB_MEM void newton_b(float *g0_out, float *pp_out, int store_ap) {
     const int nb = m.nbody;
     float lc[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
     float g0 = 0.f, pp = 0.f;
@@ -752,7 +733,7 @@ FB_UNROLL
 FB_UNROLL
         for (int k = 0; k < 6; k++) {
           al[k] = fb_ld_scr(pr + (NR_P + k)*BLK);
-          if (!given) g0 += al[k]*fb_ld_scr(pr + (NR_MD + k)*BLK);
+          g0 += al[k]*fb_ld_scr(pr + (NR_MD + k)*BLK);
           pp += al[k]*al[k];
         }
       } else {
@@ -780,10 +761,10 @@ FB_UNROLL
           m_rot(R, rc.axis[0], rc.axis[1], rc.axis[2], ax);
           const float *U = cx;
           const float ua = U[0]*al[0] + U[1]*al[1] + U[2]*al[2] + U[3]*al[3] + U[4]*al[4] + U[5]*al[5];
-          const float pj = given ? fb_ld_scr(pn + NB_P*BLK) : (cx[7] - ua)*cx[6];
+          const float pj = (cx[7] - ua)*cx[6];
           if (LEAN || jtype == FB_JNT_HINGE) { al[0] += ax[0]*pj; al[1] += ax[1]*pj; al[2] += ax[2]*pj; }
           else { al[3] += ax[0]*pj; al[4] += ax[1]*pj; al[5] += ax[2]*pj; }
-          if (!given) { fb_st_scr(pn + NB_P*BLK, pj); g0 += pj*cx[8]; }
+          fb_st_scr(pn + NB_P*BLK, pj); g0 += pj*cx[8];
           pp += pj*pj;
         }
       }
@@ -1062,23 +1043,17 @@ FB_UNROLL
   }
 
   /* ---- primal Newton with exact line search (SURVEY.md A.8), matrix-free */
-  /* warm_any (uniform over the warp, and over the warps of a SPLIT block): smooth_accel has left
-   * p0 = a_prev - a0 as the direction.  The first iteration is then the exact line search from a0
-   * along p0 (MuJoCo starts from qacc_warmstart; the search also covers a previous solution that has
-   * become a poor guess), with M p0 from sweep C; a lane without a previous solution has p0 = 0, takes
-   * a step of length 0 and enters the Newton iterations exactly as from a cold start. */
-  FB_MEM void solve(int mine, int warm_any) {      /* SPLIT: `mine` as combined over the warps */
+  FB_MEM void solve(int mine) {      /* SPLIT: `mine` as combined over the warps */
     int done = !mine;
     const int maxit = m.solver_iterations < 50 ? m.solver_iterations : 50;
     int it = 0;
     float prev_ratio = 3.0e38f, keep = 1.f;
-    if (!warm_any) newton_update(0.f, 1);        /* Delta = the constraint forces at a0: g = -J' f(a0) */
+    newton_update(0.f, 1);      /* Delta = the constraint forces at a0: g = -J' f(a0) */
     for (; it < maxit && FB_ANY(!done); it++) {
       float pg, pp, gv, sl;
       unsigned hash, hash0;
-      const int wit = warm_any && it == 0;
-      if (!wit) newton_a(keep);
-      newton_b(&pg, &pp, it == 0, wit);
+      newton_a(keep);
+      newton_b(&pg, &pp, it == 0);
       /* Line search on phi'(a) = p'M(a - a0) + a p'Mp + sum_active(a) D jp (res + a jp).  With
        * H p = -g:  p'M(a - a0) = p.g - S(0),  p'Mp = -p.g - Q(0).  First iteration: a = a0 and
        * p'Mp comes from sweep C.  phi'(0) = p.g and phi''(0) = -p.g, so the first trial step is
@@ -1093,7 +1068,6 @@ FB_UNROLL
         rcombine<6, 2>(f6, h2);
         pg = f6[0]; pp = f6[1]; S2[0] = f6[2]; S2[1] = f6[3]; Q2[0] = f6[4]; Q2[1] = f6[5];
       }
-      if (wit) pg = S2[0];                        /* phi'(0) along p0 = p0 . g */
       float g0 = pg - S2[0], pMp = fmaxf(-pg - Q2[0], 1e-7f*fabsf(pg));
       if (it == 0) {
         g0 = 0.f; pMp = newton_c();
@@ -1148,12 +1122,10 @@ FB_UNROLL
        * when the step has stopped shrinking below 1e-3: that is the floor of a worse-conditioned
        * model. */
       const float ratio = a*a*pp, lim = 1e-9f*a2 + 1e-30f;
-      /* (the warm step is a line search along a guess: neither its exactness nor its length says
-       * anything about convergence) */
-      if (!wit && !done && (exact || ratio <= lim || (it > 0 && ratio <= 1e-6f*a2 && ratio >= 0.25f*prev_ratio))) done = 1;
+      if (!done && (exact || ratio <= lim || (it > 0 && ratio <= 1e-6f*a2 && ratio >= 0.25f*prev_ratio))) done = 1;
       /* a diverged environment (non-finite state) must not hold its warp in the loop */
       if (!(a2 < 3.0e38f) || !(ratio < 3.0e38f)) done = 1;
-      prev_ratio = wit ? 3.0e38f : ratio;
+      prev_ratio = ratio;
 #ifdef FB_HOST_EMU
       if (fb_emu_stats && role == 0) { fb_emu_stats[0] += 1; fb_emu_stats[1] += nls; }
 #endif
@@ -1270,7 +1242,6 @@ FB_UNROLL
     const size_t e = (size_t)env;
     const int n = P.n_steps;
     long long row = (P.it0 + k0) % P.ring;
-    int warm = 0;
     for (int k = k0; k < n; k++) {
       row = row + 1 == P.ring ? 0 : row + 1;
       float *row_links = fb_log_row(P.log_links, row, m.n_links*20, P.env_pad, FB_VEC_LINKS, e);
@@ -1289,10 +1260,8 @@ FB_UNROLL
       if (FB_ANY(mine)) {
         this->dirty_c = P.it0 + k + 1;       /* every lane of the warp writes the constraint columns of this row */
         this->template pass_inertia_m<1>(time, aroot, 0, seqk);
-        const int warm_any = FB_WARM_START && FB_ANY(warm);
-        smooth_accel(aroot, warm, warm_any);
-        solve(mine, warm_any);
-        warm = 1;
+        smooth_accel(aroot);
+        solve(mine);
         final_forces();
 FB_UNROLL
         for (int i = 0; i < 3; i++) { aroot[i] = 0.f; aroot[3 + i] = -m.grav[i]; }
@@ -1300,20 +1269,13 @@ FB_UNROLL
         bad = this->template pass_accel_m<1>(aroot, row_joints, row_xfrc);
         write_contacts(row_contacts);
       } else {
-        warm = 0;
         this->template pass_inertia_m<0>(time, aroot, store_ctrl, seqk);
         bad = this->template pass_accel_m<0>(aroot, row_joints, row_xfrc);
-        if (this->zfill)
-          for (int i = 0; i < m.n_contacts*3; i++) fb_st4(row_contacts + i*(P.env_pad*FB_VEC_CONTACTS), 0.f, 0.f, 0.f, 0.f);
+        if (this->zfill) this->zero_contacts(row_contacts);
       }
       if (bad) FB_FLAG_OR(P.flags + env, FB_FLAG_NONFINITE);
     }
-    if (P.ctrl_seq) {
-      const float *last = P.ctrl_seq + ((size_t)(P.seq_pos + n - 1)*P.seq_stride)*P.env_pad + e;
-      for (int a = 0; a < m.nu; a++)
-        if (MI(ft_actwc, a) < 0) P.ctrl[e*m.nu + a] = last[(long long)a*P.env_pad];
-      this->store_springrefs(last);
-    }
+    if (P.ctrl_seq) this->store_seq_end(n);
     P.con_dirty[env] = this->dirty_c;
     this->store_state(P.it0 + n, coop, lane);
   }
@@ -1328,7 +1290,6 @@ FB_UNROLL
     const int n = P.n_steps;
     long long row = P.it0 % P.ring;
     idle = 0;
-    int warm = 0;
     for (int k = 0; k < n; k++) {
       row = row + 1 == P.ring ? 0 : row + 1;
       float *row_links = fb_log_row(P.log_links, row, m.n_links*20, P.env_pad, FB_VEC_LINKS, e);
@@ -1348,10 +1309,8 @@ FB_UNROLL
         this->dirty_c = P.it0 + k + 1;
         this->template pass_inertia_m<1>(time, aroot, 0, seqk);
         FB_BLOCK_BARRIER();
-        const int warm_any = FB_WARM_START && FB_ANY(warm);
-        smooth_accel(aroot, warm, warm_any);
-        solve(mine, warm_any);
-        warm = 1;
+        smooth_accel(aroot);
+        solve(mine);
         final_forces();
 FB_UNROLL
         for (int i = 0; i < 3; i++) { aroot[i] = 0.f; aroot[3 + i] = -m.grav[i]; }
@@ -1361,23 +1320,16 @@ FB_UNROLL
         bad = this->template pass_accel_m<1>(aroot, row_joints, row_xfrc);
         write_contacts(row_contacts);
       } else {
-        warm = 0;
         this->template pass_inertia_m<0>(time, aroot, store_ctrl, seqk);
         FB_BLOCK_BARRIER();
         bad = this->template pass_accel_m<0>(aroot, row_joints, row_xfrc);
-        if (this->zfill && role == 0)
-          for (int i = 0; i < m.n_contacts*3; i++) fb_st4(row_contacts + i*(P.env_pad*FB_VEC_CONTACTS), 0.f, 0.f, 0.f, 0.f);
+        if (this->zfill && role == 0) this->zero_contacts(row_contacts);
       }
       if (bad) FB_FLAG_OR(P.flags + env, FB_FLAG_NONFINITE);
       FB_BLOCK_BARRIER();
     }
     if (role != 0) return;
-    if (P.ctrl_seq) {
-      const float *last = P.ctrl_seq + ((size_t)(P.seq_pos + n - 1)*P.seq_stride)*P.env_pad + e;
-      for (int a = 0; a < m.nu; a++)
-        if (MI(ft_actwc, a) < 0) P.ctrl[e*m.nu + a] = last[(long long)a*P.env_pad];
-      this->store_springrefs(last);
-    }
+    if (P.ctrl_seq) this->store_seq_end(n);
     P.con_dirty[env] = this->dirty_c;
     this->store_state(P.it0 + n, coop, lane);
   }
