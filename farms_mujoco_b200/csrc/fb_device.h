@@ -87,6 +87,10 @@ struct EnvPtrs {
    * V lives at row[(item*(C/V) + col/V)*ev + col%V], ev = env_pad*V (FbLogView) */
   float *row_links, *row_joints, *row_contacts, *row_xfrc;
   long long ev_links, ev_joints, ev_contacts, ev_xfrc;
+  /* per-environment parameters (fb_set_env_param), already offset by the environment: value c of
+   * item i at ep_*[(i*k + c)*ep_pad]; NULL = the model's value */
+  const float *ep_stiffness, *ep_damping, *ep_coef, *ep_wvel;
+  long long ep_pad;
 };
 
 /* vector widths of the device log (floats of one row stored contiguously per environment) */
@@ -657,12 +661,12 @@ FB_UNROLL
       float f = fsm[d];
       if (MI(jnt_type, j) != FB_JNT_FREE) {
         int qa = MI(jnt_qposadr, j);
-        float stiff = MF(jnt_stiffness, j);
+        float stiff = g.ep_stiffness ? g.ep_stiffness[j*g.ep_pad] : MF(jnt_stiffness, j);
         if (stiff != 0.f) f -= stiff*(qpos[qa] - g.qpos_spring[qa]);
         int a0 = MI(jnt_actstart, j), a1 = MI(jnt_actstart, j + 1);
         for (int t = a0; t < a1; t++) { int a = MI(act_sorted, t); f += MF(act_gear, a)*actf[a]; }
       }
-      f -= MF(dof_damping, d)*qvel[d];
+      f -= (g.ep_damping ? g.ep_damping[d*g.ep_pad] : MF(dof_damping, d))*qvel[d];
       fsm[d] = f;
     }
     sync();
@@ -678,7 +682,7 @@ FB_UNROLL
     for (int e = lane; e < m.nM; e += TEAM) {
       int i = MI(ent_i, e);
       float v = qM[e];
-      if (hdamp != 0.f && i == MI(ent_j, e)) v += hdamp*MF(dof_damping, i);
+      if (hdamp != 0.f && i == MI(ent_j, e)) v += hdamp*(g.ep_damping ? g.ep_damping[i*g.ep_pad] : MF(dof_damping, i));
       qLD[e] = v;
     }
     sync();
@@ -1481,7 +1485,7 @@ FB_UNROLL
     detect_constraints();
     for (int v = lane; v < nv; v += TEAM) fcon[v] = 0.f;
     int active = (nlim + ncon) > 0;
-    if (active || want_qacc || !m.any_damping) {
+    if (active || want_qacc || !(m.any_damping || g.ep_damping)) {
       factor(0.f);
       for (int v = lane; v < nv; v += TEAM) qacc[v] = fsm[v];
       sync();
@@ -1500,7 +1504,7 @@ FB_UNROLL
     float *qpos = s + m.L.qpos, *qvel = s + m.L.qvel, *fsm = s + m.L.fsm, *fcon = s + m.L.fcon;
     float *x = s + m.L.grad;
     const float h = m.timestep;
-    if (m.any_damping) {
+    if (m.any_damping || g.ep_damping) {
       factor(h);
       for (int v = lane; v < nv; v += TEAM) x[v] = fsm[v] + fcon[v];
       sync();
@@ -1637,13 +1641,16 @@ FB_UNROLL
           float lift = -1000.f*mass*(-9.81f)/MF(swim_density, i)*frac;
           m_rot_t(R, 0.f, 0.f, lift, buoy);
         }
-        m_rot_t(R, m.water_velocity[0], m.water_velocity[1], m.water_velocity[2], uw);
+        if (g.ep_wvel) m_rot_t(R, g.ep_wvel[0], g.ep_wvel[g.ep_pad], g.ep_wvel[2*g.ep_pad], uw);
+        else m_rot_t(R, m.water_velocity[0], m.water_velocity[1], m.water_velocity[2], uw);
         float F[3], Tq[3];
         for (int k = 0; k < 3; k++) {
           float v = vl[k] - uw[k], w = wl[k];
           float sv = v < 0.f ? -v*v : v*v, sw = w < 0.f ? -w*w : w*w;
-          F[k] = sv*m.water_viscosity*MF(swim_coef, 6*i + k) + buoy[k];
-          Tq[k] = sw*MF(swim_coef, 6*i + 3 + k);
+          const float cl = g.ep_coef ? g.ep_coef[(6*i + k)*g.ep_pad] : MF(swim_coef, 6*i + k);
+          const float ca = g.ep_coef ? g.ep_coef[(6*i + 3 + k)*g.ep_pad] : MF(swim_coef, 6*i + 3 + k);
+          F[k] = sv*m.water_viscosity*cl + buoy[k];
+          Tq[k] = sw*ca;
         }
         float *row = g.row_xfrc + (long long)xi*(6/FB_VEC_XFRC)*g.ev_xfrc;
         for (int k = 0; k < 3; k++) {
@@ -1768,6 +1775,16 @@ struct FbParams {
   int *con_split_done;
 };
 
+/* Per-environment parameter tables (fb_set_env_param), float32 environment-minor: value c of item i
+ * of environment env at [(i*k + c)*env_pad + env] -- jnt_stiffness [njnt], dof_damping [nv], drag
+ * coefficients [n_swim][6], water velocity [3].  NULL: the model's value for every environment.
+ * A launch argument of its own (not a member of FbParams), so that the parameter blocks of the
+ * kernels that do not read it keep their layout: the team kernel tests the pointers at run time,
+ * the per-thread kernels read them in their ENVP twins only. */
+struct FbEnvTables {
+  const float *stiffness, *damping, *coef, *wvel;
+};
+
 #define FB_NEVER_DIRTY (-(1LL << 60))
 
 /* start of ring row `it` for one environment: floats_per_row = N*C of the kind */
@@ -1776,7 +1793,7 @@ FB_DEV float *fb_log_row(float *base, long long it, long long floats_per_row, lo
   return base + it*floats_per_row*env_pad + env*vec;
 }
 
-FB_DEV EnvPtrs fb_env_ptrs(const FbParams &P, int env) {
+FB_DEV EnvPtrs fb_env_ptrs(const FbParams &P, const FbEnvTables &T, int env) {
   const DevModel &m = P.m;
   EnvPtrs g;
   size_t e = (size_t)env;
@@ -1796,6 +1813,11 @@ FB_DEV EnvPtrs fb_env_ptrs(const FbParams &P, int env) {
   g.row_links = g.row_joints = g.row_contacts = g.row_xfrc = 0;
   g.ev_links = P.env_pad*FB_VEC_LINKS; g.ev_joints = P.env_pad*FB_VEC_JOINTS;
   g.ev_contacts = P.env_pad*FB_VEC_CONTACTS; g.ev_xfrc = P.env_pad*FB_VEC_XFRC;
+  g.ep_stiffness = T.stiffness ? T.stiffness + e : 0;
+  g.ep_damping = T.damping ? T.damping + e : 0;
+  g.ep_coef = T.coef ? T.coef + e : 0;
+  g.ep_wvel = T.wvel ? T.wvel + e : 0;
+  g.ep_pad = P.env_pad;
   return g;
 }
 
@@ -1804,10 +1826,10 @@ FB_DEV EnvPtrs fb_env_ptrs(const FbParams &P, int env) {
  * (it0+k+1) % ring = {derived of the pre-step state, qpos/qvel of the new
  * state} (SURVEY.md Appendix D-1), then the drag wrench for the next step. */
 template <int TEAM>
-FB_DEV void fb_run_env(const FbParams &P, int env, int k0, float *s, int *si, int lane, int base,
+FB_DEV void fb_run_env(const FbParams &P, const FbEnvTables &T, int env, int k0, float *s, int *si, int lane, int base,
                        unsigned mask) {
   const DevModel &m = P.m;
-  FbStep<TEAM> st(m, s, si, fb_env_ptrs(P, env), lane, base, mask);
+  FbStep<TEAM> st(m, s, si, fb_env_ptrs(P, T, env), lane, base, mask);
   st.init_world();
   st.load_state();
   const size_t e = (size_t)env;

@@ -12,6 +12,8 @@
  * so the arithmetic can be checked on the GPU-less development box.  The
  * product never loads that library.
  */
+#include <algorithm>
+#include <cmath>
 #include <cstdint>
 #include <cstdio>
 #include <cstdlib>
@@ -66,7 +68,7 @@ static const char *dev_error() { return cudaGetErrorString(cudaGetLastError()); 
 #ifndef FB_HOST_EMU
 template <int TEAM>
 __global__ void __launch_bounds__(128)
-fb_step_kernel(const __grid_constant__ FbParams P) {
+fb_step_kernel(const __grid_constant__ FbParams P, const __grid_constant__ FbEnvTables T) {
   extern __shared__ __align__(16) float fb_smem[];
   const DevModel &m = P.m;
   const int tid = threadIdx.x, team = tid/TEAM, lane = tid % TEAM;
@@ -83,7 +85,7 @@ fb_step_kernel(const __grid_constant__ FbParams P) {
   const unsigned mask = TEAM == 32 ? 0xffffffffu : (((1u << (TEAM & 31)) - 1u) << base);
   float *s = fb_smem + (size_t)team*(m.L.n_float + m.L.n_int);
   int *si = reinterpret_cast<int *>(s + m.L.n_float);
-  fb_run_env<TEAM>(P, env, k0, s, si, lane, base, mask);
+  fb_run_env<TEAM>(P, T, env, k0, s, si, lane, base, mask);
 }
 
 /* environment-per-thread kernel (fb_fast.h): no barriers, no shuffles; BLK threads =
@@ -95,33 +97,43 @@ struct FbFastParams {
 
 /* BLK environments per warp (32, or 16 in a half-filled warp).  MULTI: blocks of 2..8 warps
  * (blockDim.x/32) kept in step by a barrier per physics step (FbFast::run_t). */
+/* Every per-thread entry point has an ENVP twin (fb_*_envp_kernel, same template arguments) that reads
+ * the per-environment parameter tables of fb_set_env_param; launch() takes the twin while any table
+ * is set.  An entry point and its twin expand the same body (FB_*_BODY: ENVP is a template argument
+ * of FbFast / FbFastCon, T the tables); written out in each kernel rather than called as an inlined
+ * function, which ptxas was found to schedule differently.  A twin's parameters are the entry
+ * point's with the tables appended; the entry point's keep their layout. */
+struct FbFastEnvParams : FbFastParams { FbEnvTables T; };
+#define FB_FAST_BODY(ENVP, T) \
+  extern __shared__ __align__(16) float fb_smem[];                                                                    \
+  const FbParams &P = Q.P;                                                                                            \
+  const int warp = MULTI ? threadIdx.x >> 5 : 0, lane = MULTI ? threadIdx.x & 31 : threadIdx.x;                       \
+  const int wid = MULTI ? blockIdx.x*(blockDim.x >> 5) + warp : blockIdx.x;   /* warp index of the launch */          \
+  const int env = wid*BLK + lane;                                                                                     \
+  if (blockIdx.x == 0 && threadIdx.x == 0) P.pending_count[P.parity ^ 1] = 0;   /* for the next launch */             \
+  const int valid = env < P.n_envs;                                                                                   \
+  if (!MULTI && !valid) return;                                                                                       \
+  const int n_float = SLIM ? P.m.X.n_float_slim : P.m.X.n_float;                                                      \
+  const size_t warp_floats = (size_t)n_float*BLK;                                                                     \
+  /* L2-resident scratch [warp][field][lane]: compile-time strides, coalesced */                                      \
+  FbFast<BLK, SLIM, LEAN, 0, ENVP> st(P, Q.rec, fb_smem + warp*warp_floats + lane,                                    \
+                             P.fast_scratch + (size_t)wid*(SLIM ? P.m.X.n_scratch_slim : P.m.X.n_scratch)*BLK + lane, \
+                             valid ? env : 0, T);                                                                     \
+  /* full warps move their state through a shared-memory tile (coalesced); a partial last                             \
+   * warp, or a model whose state rows do not fit the tile, uses per-thread accesses (the SLIM                        \
+   * layout's smaller blocks take the rows in two phases) */                                                          \
+  const int coop = BLK == 32 && (wid + 1)*BLK <= P.n_envs ? (SLIM ? 2*P.m.X.coop_io2 : P.m.X.coop_io) : 0;            \
+  const int done = st.template run_t<MULTI>(coop, lane, valid);                                                       \
+  if (valid && done < P.n_steps) {                                                                                    \
+    P.steps_done[env] = done;                                                                                         \
+    P.pending[atomicAdd(P.pending_count + P.parity, 1)] = env;                                                        \
+  }
 template <int BLK, int SLIM, int MULTI, int LEAN = 0>
 __global__ void __launch_bounds__(MULTI ? 256 : 32)
-fb_fast_kernel(const __grid_constant__ FbFastParams Q) {
-  extern __shared__ __align__(16) float fb_smem[];
-  const FbParams &P = Q.P;
-  const int warp = MULTI ? threadIdx.x >> 5 : 0, lane = MULTI ? threadIdx.x & 31 : threadIdx.x;
-  const int wid = MULTI ? blockIdx.x*(blockDim.x >> 5) + warp : blockIdx.x;   /* warp index of the launch */
-  const int env = wid*BLK + lane;
-  if (blockIdx.x == 0 && threadIdx.x == 0) P.pending_count[P.parity ^ 1] = 0;   /* for the next launch */
-  const int valid = env < P.n_envs;
-  if (!MULTI && !valid) return;
-  const int n_float = SLIM ? P.m.X.n_float_slim : P.m.X.n_float;
-  const size_t warp_floats = (size_t)n_float*BLK;
-  /* L2-resident scratch [warp][field][lane]: compile-time strides, coalesced */
-  FbFast<BLK, SLIM, LEAN> st(P, Q.rec, fb_smem + warp*warp_floats + lane,
-                             P.fast_scratch + (size_t)wid*(SLIM ? P.m.X.n_scratch_slim : P.m.X.n_scratch)*BLK + lane,
-                             valid ? env : 0);
-  /* full warps move their state through a shared-memory tile (coalesced); a partial last
-   * warp, or a model whose state rows do not fit the tile, uses per-thread accesses (the SLIM
-   * layout's smaller blocks take the rows in two phases) */
-  const int coop = BLK == 32 && (wid + 1)*BLK <= P.n_envs ? (SLIM ? 2*P.m.X.coop_io2 : P.m.X.coop_io) : 0;
-  const int done = st.template run_t<MULTI>(coop, lane, valid);
-  if (valid && done < P.n_steps) {
-    P.steps_done[env] = done;
-    P.pending[atomicAdd(P.pending_count + P.parity, 1)] = env;
-  }
-}
+fb_fast_kernel(const __grid_constant__ FbFastParams Q) { FB_FAST_BODY(0, 0) }
+template <int BLK, int SLIM, int MULTI, int LEAN = 0>
+__global__ void __launch_bounds__(MULTI ? 256 : 32)
+fb_fast_envp_kernel(const __grid_constant__ FbFastEnvParams Q) { FB_FAST_BODY(1, &Q.T) }
 
 /* SPLIT variant (small batches): one block = 32 environments stepped by split.nwarps warps */
 struct FbFastSplitParams {
@@ -139,27 +151,31 @@ struct FbFastSplitParams {
 #ifndef FB_SPLIT_MINBLOCKS
 #define FB_SPLIT_MINBLOCKS 3
 #endif
+struct FbFastSplitEnvParams : FbFastSplitParams { FbEnvTables T; };
+#define FB_FAST_SPLIT_BODY(ENVP, T) \
+  extern __shared__ __align__(16) float fb_smem[];                                                                  \
+  const FbParams &P = Q.P;                                                                                          \
+  const int role = threadIdx.x >> 5, lane = threadIdx.x & 31, wid = blockIdx.x;                                     \
+  const int env = wid*32 + lane;                                                                                    \
+  if (blockIdx.x == 0 && threadIdx.x == 0) P.pending_count[P.parity ^ 1] = 0;   /* for the next launch */           \
+  const int valid = env < P.n_envs;                                                                                 \
+  const int n_float = P.m.X.n_float;                                                                                \
+  FbFast<32, 0, LEAN, 1, ENVP> st(P, Q.rec, fb_smem + lane, P.fast_scratch + (size_t)wid*P.m.X.n_scratch*32 + lane, \
+                            valid ? env : 0, T);                                                                    \
+  float *extra = fb_smem + (size_t)n_float*32;                                                                      \
+  st.split_setup(Q.split, role, extra + lane, reinterpret_cast<int *>(extra + 3*32) + lane);                        \
+  const int coop = (wid + 1)*32 <= P.n_envs ? P.m.X.coop_io : 0;                                                    \
+  const int done = st.run_split(coop, lane, valid);                                                                 \
+  if (role == 0 && valid && done < P.n_steps) {                                                                     \
+    P.steps_done[env] = done;                                                                                       \
+    P.pending[atomicAdd(P.pending_count + P.parity, 1)] = env;                                                      \
+  }
 template <int LEAN>
 __global__ void __launch_bounds__(32*FB_SPLIT_MAXW, FB_SPLIT_MINBLOCKS)
-fb_fast_split_kernel(const __grid_constant__ FbFastSplitParams Q) {
-  extern __shared__ __align__(16) float fb_smem[];
-  const FbParams &P = Q.P;
-  const int role = threadIdx.x >> 5, lane = threadIdx.x & 31, wid = blockIdx.x;
-  const int env = wid*32 + lane;
-  if (blockIdx.x == 0 && threadIdx.x == 0) P.pending_count[P.parity ^ 1] = 0;   /* for the next launch */
-  const int valid = env < P.n_envs;
-  const int n_float = P.m.X.n_float;
-  FbFast<32, 0, LEAN, 1> st(P, Q.rec, fb_smem + lane, P.fast_scratch + (size_t)wid*P.m.X.n_scratch*32 + lane,
-                            valid ? env : 0);
-  float *extra = fb_smem + (size_t)n_float*32;
-  st.split_setup(Q.split, role, extra + lane, reinterpret_cast<int *>(extra + 3*32) + lane);
-  const int coop = (wid + 1)*32 <= P.n_envs ? P.m.X.coop_io : 0;
-  const int done = st.run_split(coop, lane, valid);
-  if (role == 0 && valid && done < P.n_steps) {
-    P.steps_done[env] = done;
-    P.pending[atomicAdd(P.pending_count + P.parity, 1)] = env;
-  }
-}
+fb_fast_split_kernel(const __grid_constant__ FbFastSplitParams Q) { FB_FAST_SPLIT_BODY(0, 0) }
+template <int LEAN>
+__global__ void __launch_bounds__(32*FB_SPLIT_MAXW, FB_SPLIT_MINBLOCKS)
+fb_fast_split_envp_kernel(const __grid_constant__ FbFastSplitEnvParams Q) { FB_FAST_SPLIT_BODY(1, &Q.T) }
 
 struct FbFastConParams {
   FbParams P;
@@ -168,24 +184,29 @@ struct FbFastConParams {
 };
 static_assert(sizeof(FbFastConParams) <= 32764, "kernel parameters of fb_fastc_kernel exceed 32 KB");
 
+struct FbFastConEnvParams : FbFastConParams { FbEnvTables T; };
+static_assert(sizeof(FbFastConEnvParams) <= 32764, "kernel parameters of fb_fastc_envp_kernel exceed 32 KB");
+#define FB_FASTC_BODY(ENVP, T) \
+  extern __shared__ __align__(16) float fb_smem[];                                                                             \
+  const FbParams &P = Q.P;                                                                                                     \
+  const int i = blockIdx.x*BLK + threadIdx.x;                                                                                  \
+  const int count = P.use_pending ? P.pending_count[P.parity] : P.n_envs;                                                      \
+  if (i >= count) return;                                                                                                      \
+  if (P.con_split_done && P.con_split_done[blockIdx.x]) return;      /* stepped by the SPLIT variant */                        \
+  const int identity = !P.use_pending || count == P.n_envs;                                                                    \
+  const int env = identity ? i : P.pending[i];                                                                                 \
+  const int k0 = P.use_pending ? P.steps_done[env] : 0;                                                                        \
+  const size_t t0 = (size_t)blockIdx.x*BLK;                                                                                    \
+  FbFastCon<BLK, LEAN, 0, ENVP> st(P, Q.rec, Q.cand, fb_smem + threadIdx.x, P.fast_scratch + t0*P.m.X.n_scratch + threadIdx.x, \
+                    P.con_scratch + t0*P.m.X.n_con + threadIdx.x, env, T);                                                     \
+  const int coop = BLK == 32 && identity && P.m.X.coop_io && (blockIdx.x + 1)*BLK <= count;                                    \
+  st.run_con(k0, coop, threadIdx.x);                                                                                           
 template <int BLK, int LEAN = 0>
 __global__ void __launch_bounds__(BLK)
-fb_fastc_kernel(const __grid_constant__ FbFastConParams Q) {
-  extern __shared__ __align__(16) float fb_smem[];
-  const FbParams &P = Q.P;
-  const int i = blockIdx.x*BLK + threadIdx.x;
-  const int count = P.use_pending ? P.pending_count[P.parity] : P.n_envs;
-  if (i >= count) return;
-  if (P.con_split_done && P.con_split_done[blockIdx.x]) return;      /* stepped by the SPLIT variant */
-  const int identity = !P.use_pending || count == P.n_envs;
-  const int env = identity ? i : P.pending[i];
-  const int k0 = P.use_pending ? P.steps_done[env] : 0;
-  const size_t t0 = (size_t)blockIdx.x*BLK;
-  FbFastCon<BLK, LEAN> st(P, Q.rec, Q.cand, fb_smem + threadIdx.x, P.fast_scratch + t0*P.m.X.n_scratch + threadIdx.x,
-                    P.con_scratch + t0*P.m.X.n_con + threadIdx.x, env);
-  const int coop = BLK == 32 && identity && P.m.X.coop_io && (blockIdx.x + 1)*BLK <= count;
-  st.run_con(k0, coop, threadIdx.x);
-}
+fb_fastc_kernel(const __grid_constant__ FbFastConParams Q) { FB_FASTC_BODY(0, 0) }
+template <int BLK, int LEAN = 0>
+__global__ void __launch_bounds__(BLK)
+fb_fastc_envp_kernel(const __grid_constant__ FbFastConEnvParams Q) { FB_FASTC_BODY(1, &Q.T) }
 
 /* SPLIT variant of the constrained kernel: one block = the BLK environments of one group (the
  * lanes of a warp; the upper half-warp leaves at once when BLK = 16) stepped by split.nwarps
@@ -204,26 +225,53 @@ static_assert(sizeof(FbFastConSplitParams) <= 32764, "kernel parameters of fb_fa
 #ifndef FB_CSPLIT_MINBLOCKS
 #define FB_CSPLIT_MINBLOCKS 2
 #endif
+struct FbFastConSplitEnvParams : FbFastConSplitParams { FbEnvTables T; };
+static_assert(sizeof(FbFastConSplitEnvParams) <= 32764, "kernel parameters of fb_fastc_split_envp_kernel exceed 32 KB");
+#define FB_FASTC_SPLIT_BODY(ENVP, T) \
+  extern __shared__ __align__(16) float fb_smem[];                                                                       \
+  const FbParams &P = Q.P;                                                                                               \
+  const int role = threadIdx.x >> 5, lane = threadIdx.x & 31, grp = blockIdx.x;                                          \
+  const int env = grp*BLK + lane;                                                                                        \
+  if (lane >= BLK || env >= P.n_envs) return;                                                                            \
+  /* block-uniform: every warp sees the same lanes */                                                                    \
+  const int all0 = P.pending_count[P.parity] == P.n_envs && __ballot_sync(__activemask(), P.steps_done[env] != 0) == 0u; \
+  if (threadIdx.x == 0) P.con_split_done[grp] = all0;                                                                    \
+  if (!all0) return;                                                                                                     \
+  const size_t t0 = (size_t)grp*BLK;                                                                                     \
+  FbFastCon<BLK, LEAN, 1, ENVP> st(P, Q.rec, Q.cand, fb_smem + lane, P.fast_scratch + t0*P.m.X.n_scratch + lane,         \
+                             P.con_scratch + t0*P.m.X.n_con + lane, env, T);                                             \
+  float *extra = fb_smem + (size_t)P.m.X.n_float*BLK;                                                                    \
+  st.split_setup(Q.split, role, extra + lane, reinterpret_cast<int *>(extra + 3*BLK) + lane);                            \
+  st.con_split_setup(Q.split, extra + 4*BLK + lane);                                                                     \
+  const int coop = BLK == 32 && P.m.X.coop_io && (grp + 1)*BLK <= P.n_envs;                                              \
+  st.run_con_split(coop, lane);                                                                                          
 template <int BLK, int LEAN>
 __global__ void __launch_bounds__(32*FB_SPLIT_MAXW, FB_CSPLIT_MINBLOCKS)
-fb_fastc_split_kernel(const __grid_constant__ FbFastConSplitParams Q) {
-  extern __shared__ __align__(16) float fb_smem[];
-  const FbParams &P = Q.P;
-  const int role = threadIdx.x >> 5, lane = threadIdx.x & 31, grp = blockIdx.x;
-  const int env = grp*BLK + lane;
-  if (lane >= BLK || env >= P.n_envs) return;
-  /* block-uniform: every warp sees the same lanes */
-  const int all0 = P.pending_count[P.parity] == P.n_envs && __ballot_sync(__activemask(), P.steps_done[env] != 0) == 0u;
-  if (threadIdx.x == 0) P.con_split_done[grp] = all0;
-  if (!all0) return;
-  const size_t t0 = (size_t)grp*BLK;
-  FbFastCon<BLK, LEAN, 1> st(P, Q.rec, Q.cand, fb_smem + lane, P.fast_scratch + t0*P.m.X.n_scratch + lane,
-                             P.con_scratch + t0*P.m.X.n_con + lane, env);
-  float *extra = fb_smem + (size_t)P.m.X.n_float*BLK;
-  st.split_setup(Q.split, role, extra + lane, reinterpret_cast<int *>(extra + 3*BLK) + lane);
-  st.con_split_setup(Q.split, extra + 4*BLK + lane);
-  const int coop = BLK == 32 && P.m.X.coop_io && (grp + 1)*BLK <= P.n_envs;
-  st.run_con_split(coop, lane);
+fb_fastc_split_kernel(const __grid_constant__ FbFastConSplitParams Q) { FB_FASTC_SPLIT_BODY(0, 0) }
+template <int BLK, int LEAN>
+__global__ void __launch_bounds__(32*FB_SPLIT_MAXW, FB_CSPLIT_MINBLOCKS)
+fb_fastc_split_envp_kernel(const __grid_constant__ FbFastConSplitEnvParams Q) { FB_FASTC_SPLIT_BODY(1, &Q.T) }
+
+/* launch an entry point or its ENVP twin */
+template <int BLK, int SLIM, int MULTI, int LEAN>
+static void fb_launch_fast(bool envp, int grid, int threads, size_t bytes, cudaStream_t st, const FbFastEnvParams &Q) {
+  if (envp) fb_fast_envp_kernel<BLK, SLIM, MULTI, LEAN><<<grid, threads, bytes, st>>>(Q);
+  else fb_fast_kernel<BLK, SLIM, MULTI, LEAN><<<grid, threads, bytes, st>>>(static_cast<const FbFastParams &>(Q));
+}
+template <int LEAN>
+static void fb_launch_fast_split(bool envp, int grid, int threads, size_t bytes, cudaStream_t st, const FbFastSplitEnvParams &Q) {
+  if (envp) fb_fast_split_envp_kernel<LEAN><<<grid, threads, bytes, st>>>(Q);
+  else fb_fast_split_kernel<LEAN><<<grid, threads, bytes, st>>>(static_cast<const FbFastSplitParams &>(Q));
+}
+template <int BLK, int LEAN>
+static void fb_launch_fastc(bool envp, int grid, size_t bytes, cudaStream_t st, const FbFastConEnvParams &Q) {
+  if (envp) fb_fastc_envp_kernel<BLK, LEAN><<<grid, BLK, bytes, st>>>(Q);
+  else fb_fastc_kernel<BLK, LEAN><<<grid, BLK, bytes, st>>>(static_cast<const FbFastConParams &>(Q));
+}
+template <int BLK, int LEAN>
+static void fb_launch_fastc_split(bool envp, int grid, int threads, size_t bytes, cudaStream_t st, const FbFastConSplitEnvParams &Q) {
+  if (envp) fb_fastc_split_envp_kernel<BLK, LEAN><<<grid, threads, bytes, st>>>(Q);
+  else fb_fastc_split_kernel<BLK, LEAN><<<grid, threads, bytes, st>>>(static_cast<const FbFastConSplitParams &>(Q));
 }
 
 /* Stand-alone drag operator (fb_drag_forces, fb_drag.h): one thread = one link row */
@@ -361,15 +409,20 @@ struct FbHandle {
   long long launch_parity;
   int log_used;                     /* 0 until the first reset: the log is as fb_create zeroed it */
 #ifndef FB_HOST_EMU
-  FbFastParams *fastQ;               /* host staging of the per-thread kernel's parameters */
-  FbFastSplitParams *splitQ;         /* ... of its SPLIT variant */
-  FbFastConParams *conQ;             /* ... and of the per-thread constrained kernel's */
-  FbFastConSplitParams *csplitQ;     /* ... and of its SPLIT variant */
+  FbFastEnvParams *fastQ;            /* host staging of the per-thread kernel's parameters (+ the ENVP twin's tables) */
+  FbFastSplitEnvParams *splitQ;      /* ... of its SPLIT variant */
+  FbFastConEnvParams *conQ;          /* ... and of the per-thread constrained kernel's */
+  FbFastConSplitEnvParams *csplitQ;  /* ... and of its SPLIT variant */
 #endif
   fbStream stream;
   std::vector<void *> allocs;
   int32_t *I_dev;
   float *F_dev;
+  /* per-environment parameter tables (fb_set_env_param), indexed by FB_ENV_*: the device copy
+   * (FbParams::ep_*, float32 [item*k + c][env_pad]) and the values as set ([n_envs][width]) */
+  float *ep_dev[4];
+  std::vector<double> ep_host[4];
+  FbEnvTables ep;                   /* ep_dev as the kernels take it */
   long long launches;
   long long it;            /* physics steps since reset */
   float last_ms;
@@ -505,17 +558,17 @@ static int upload_model(FbHandle *h) {
         h->hm.rec[b].flags |= (int32_t)(sx + 1) << FT_SREF_SHIFT;
 #ifndef FB_HOST_EMU
   if (h->hm.m.X.ok) {
-    if (!h->fastQ) h->fastQ = new FbFastParams();
+    if (!h->fastQ) h->fastQ = new FbFastEnvParams();
     memset(h->fastQ->rec, 0, sizeof(h->fastQ->rec));
     memcpy(h->fastQ->rec, h->hm.rec.data(), sizeof(FastRec)*h->hm.rec.size());
-    if (!h->splitQ) h->splitQ = new FbFastSplitParams();
+    if (!h->splitQ) h->splitQ = new FbFastSplitEnvParams();
     memcpy(h->splitQ->rec, h->fastQ->rec, sizeof(h->splitQ->rec));
     h->splitQ->split = h->hm.split;
-    if (!h->conQ) h->conQ = new FbFastConParams();
+    if (!h->conQ) h->conQ = new FbFastConEnvParams();
     memcpy(h->conQ->rec, h->fastQ->rec, sizeof(h->conQ->rec));
     memset(h->conQ->cand, 0, sizeof(h->conQ->cand));
     if (h->hm.m.X.con_ok) memcpy(h->conQ->cand, h->hm.crec.data(), sizeof(CandRec)*h->hm.crec.size());
-    if (!h->csplitQ) h->csplitQ = new FbFastConSplitParams();
+    if (!h->csplitQ) h->csplitQ = new FbFastConSplitEnvParams();
     memcpy(h->csplitQ->rec, h->conQ->rec, sizeof(h->csplitQ->rec));
     memcpy(h->csplitQ->cand, h->conQ->cand, sizeof(h->csplitQ->cand));
     h->csplitQ->split = h->hm.split;
@@ -562,6 +615,79 @@ template <class F> static void emu_split_run(int nw, F body) {
 }
 #endif
 
+#ifdef FB_HOST_EMU
+/* test harness: the per-thread kernels (ENVP: their twins) run serially on the host */
+template <int ENVP> static void emu_per_thread(FbHandle *h, FbParams &P, int n_steps, int con_thread) {
+  const DevModel &m = P.m;
+  const FbEnvTables *T = ENVP ? &h->ep : nullptr;
+  P.pending_count[P.parity ^ 1] = 0;
+  std::vector<float> fs((size_t)m.X.n_float + 8, 0.f);
+  std::vector<float> fg((size_t)(m.X.n_scratch > m.X.n_scratch_slim ? m.X.n_scratch : m.X.n_scratch_slim) + 8, 0.f);
+  const FastSplit &sp = h->hm.split;
+  const int n_extra = 4 + 2*FB_SPLIT_MAXW*FB_RED_MAX;      /* root position, flag, reduction buffers (one lane) */
+  for (int env = 0; env < P.n_envs; env++) {
+    int done;
+    const bool lean = h->fast_lean && m.X.lean && !P.ctrl_seq;
+    if (h->fast_split && !h->fast_slim && sp.nwarps > 1) {
+      /* SPLIT variant: the warps of the block are host threads */
+      std::vector<float> extra(n_extra, 0.f);
+      int done0 = 0;
+      emu_split_run(sp.nwarps, [&](int role) {
+        int d;
+        if (lean) {
+          FbFast<1, 0, 1, 1, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T);
+          st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
+          d = st.run_split(0, 0, 1);
+        } else {
+          FbFast<1, 0, 0, 1, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T);
+          st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
+          d = st.run_split(0, 0, 1);
+        }
+        if (role == 0) done0 = d;
+      });
+      done = done0;
+    } else
+    if (h->fast_slim && lean) { FbFast<1, 1, 1, 0, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T); done = st.run(0, 0); }
+    else if (h->fast_slim) { FbFast<1, 1, 0, 0, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T); done = st.run(0, 0); }
+    else if (lean) { FbFast<1, 0, 1, 0, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T); done = st.run(0, 0); }
+    else { FbFast<1, 0, 0, 0, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T); done = st.run(0, 0); }
+    if (done < n_steps) { P.steps_done[env] = done; P.pending[P.pending_count[P.parity]++] = env; }
+  }
+  if (con_thread) {
+    std::vector<float> fc((size_t)m.X.n_con + 8, 0.f);
+    for (int i = 0; i < P.pending_count[P.parity]; i++) {
+      const int env = P.pending[i];
+      if (h->con_split && !h->fast_slim && sp.nwarps > 1 && P.steps_done[env] == 0) {
+        /* SPLIT variant of the constrained kernel (a group = this environment) */
+        std::vector<float> extra(n_extra, 0.f);
+        const bool lean = h->fast_lean && m.X.lean && !P.ctrl_seq;
+        emu_split_run(sp.nwarps, [&](int role) {
+          if (lean) {
+            FbFastCon<1, 1, 1, ENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, T);
+            st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
+            st.con_split_setup(sp, extra.data() + 4);
+            st.run_con_split(0, 0);
+          } else {
+            FbFastCon<1, 0, 1, ENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, T);
+            st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
+            st.con_split_setup(sp, extra.data() + 4);
+            st.run_con_split(0, 0);
+          }
+        });
+        continue;
+      }
+      if (h->fast_lean && m.X.lean && !P.ctrl_seq) {
+        FbFastCon<1, 1, 0, ENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, T);
+        st.run_con(P.steps_done[env], 0, 0);
+      } else {
+        FbFastCon<1, 0, 0, ENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, T);
+        st.run_con(P.steps_done[env], 0, 0);
+      }
+    }
+  }
+}
+#endif
+
 static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
   FbParams &P = h->P;
   P.mode = mode; P.n_steps = n_steps; P.want_derived = want_derived; P.it0 = h->it;
@@ -591,6 +717,8 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
     if (h->seq_pos == h->seq_len) h->seq_len = h->seq_pos = 0;     /* consumed: ctrl is held again */
   }
   const int use_fast = h->fast_enabled && P.m.X.ok && mode == FB_MODE_STEP && !want_derived;
+  /* the per-thread kernels' ENVP twins while a per-environment parameter table is set */
+  const bool envp = h->ep.stiffness || h->ep.damping || h->ep.coef || h->ep.wvel;
   const int con_thread = use_fast && h->con_thread && P.m.X.con_ok;
   P.use_pending = use_fast;
   P.parity = (int)(h->launch_parity & 1);
@@ -598,78 +726,15 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
 #ifdef FB_HOST_EMU
   const DevModel &m = P.m;
   if (use_fast) {
-    P.pending_count[P.parity ^ 1] = 0;
-    std::vector<float> fs((size_t)m.X.n_float + 8, 0.f);
-    std::vector<float> fg((size_t)(m.X.n_scratch > m.X.n_scratch_slim ? m.X.n_scratch : m.X.n_scratch_slim) + 8, 0.f);
-    const FastSplit &sp = h->hm.split;
-    const int n_extra = 4 + 2*FB_SPLIT_MAXW*FB_RED_MAX;      /* root position, flag, reduction buffers (one lane) */
-    for (int env = 0; env < P.n_envs; env++) {
-      int done;
-      const bool lean = h->fast_lean && m.X.lean && !P.ctrl_seq;
-      if (h->fast_split && !h->fast_slim && sp.nwarps > 1) {
-        /* SPLIT variant: the warps of the block are host threads */
-        std::vector<float> extra(n_extra, 0.f);
-        int done0 = 0;
-        emu_split_run(sp.nwarps, [&](int role) {
-          int d;
-          if (lean) {
-            FbFast<1, 0, 1, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env);
-            st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
-            d = st.run_split(0, 0, 1);
-          } else {
-            FbFast<1, 0, 0, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env);
-            st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
-            d = st.run_split(0, 0, 1);
-          }
-          if (role == 0) done0 = d;
-        });
-        done = done0;
-      } else
-      if (h->fast_slim && lean) { FbFast<1, 1, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env); done = st.run(0, 0); }
-      else if (h->fast_slim) { FbFast<1, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env); done = st.run(0, 0); }
-      else if (lean) { FbFast<1, 0, 1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env); done = st.run(0, 0); }
-      else { FbFast<1> st(P, h->hm.rec.data(), fs.data(), fg.data(), env); done = st.run(0, 0); }
-      if (done < n_steps) { P.steps_done[env] = done; P.pending[P.pending_count[P.parity]++] = env; }
-    }
-    if (con_thread) {
-      std::vector<float> fc((size_t)m.X.n_con + 8, 0.f);
-      for (int i = 0; i < P.pending_count[P.parity]; i++) {
-        const int env = P.pending[i];
-        if (h->con_split && !h->fast_slim && sp.nwarps > 1 && P.steps_done[env] == 0) {
-          /* SPLIT variant of the constrained kernel (a group = this environment) */
-          std::vector<float> extra(n_extra, 0.f);
-          const bool lean = h->fast_lean && m.X.lean && !P.ctrl_seq;
-          emu_split_run(sp.nwarps, [&](int role) {
-            if (lean) {
-              FbFastCon<1, 1, 1> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env);
-              st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
-              st.con_split_setup(sp, extra.data() + 4);
-              st.run_con_split(0, 0);
-            } else {
-              FbFastCon<1, 0, 1> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env);
-              st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
-              st.con_split_setup(sp, extra.data() + 4);
-              st.run_con_split(0, 0);
-            }
-          });
-          continue;
-        }
-        if (h->fast_lean && m.X.lean && !P.ctrl_seq) {
-          FbFastCon<1, 1> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env);
-          st.run_con(P.steps_done[env], 0, 0);
-        } else {
-          FbFastCon<1> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env);
-          st.run_con(P.steps_done[env], 0, 0);
-        }
-      }
-    }
+    if (envp) emu_per_thread<1>(h, P, n_steps, con_thread);
+    else emu_per_thread<0>(h, P, n_steps, con_thread);
   }
   std::vector<float> s((size_t)m.L.n_float + 8, 0.f);
   std::vector<int> si((size_t)m.L.n_int + 8, 0);
   const int count = use_fast ? (con_thread ? 0 : P.pending_count[P.parity]) : P.n_envs;
   for (int i = 0; i < count; i++) {
     int env = use_fast ? P.pending[i] : i;
-    fb_run_env<1>(P, env, use_fast ? P.steps_done[env] : 0, s.data(), si.data(), 0, 0, 1u);
+    fb_run_env<1>(P, h->ep, env, use_fast ? P.steps_done[env] : 0, s.data(), si.data(), 0, 0, 1u);
   }
   h->last_ms = 0.f;
 #else
@@ -691,7 +756,7 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
   cudaEventRecord(h->ev0, h->stream);
   if (use_fast) {
     int fblocks = (P.n_envs + h->fast_block - 1)/h->fast_block;
-    h->fastQ->P = P;
+    h->fastQ->P = P; h->fastQ->T = h->ep;
     {
       int wpb = h->fast_block == 32 ? h->fast_wpb : 1;
       if (!h->fast_slim || wpb < 2 || wpb > 8) wpb = 1;      /* multi-warp blocks: SLIM layout only (measured 3-5 % slower on the regular one) */
@@ -702,23 +767,23 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
       const bool lean = h->fast_lean && P.m.X.lean && !P.ctrl_seq;
       if (h->fast_split && h->fast_block == 32 && !h->fast_slim && h->hm.split.nwarps > 1 && warps <= h->split_capacity) {
         /* small batch: the tree of every 32 environments split over several warps */
-        h->splitQ->P = P;
+        h->splitQ->P = P; h->splitQ->T = h->ep;
         const size_t sbytes = h->fast_smem_bytes + FB_SPLIT_EXTRA_BYTES;
         const int threads = 32*h->hm.split.nwarps;
-        if (lean) fb_fast_split_kernel<1><<<warps, threads, sbytes, h->stream>>>(*h->splitQ);
-        else fb_fast_split_kernel<0><<<warps, threads, sbytes, h->stream>>>(*h->splitQ);
+        if (lean) fb_launch_fast_split<1>(envp, warps, threads, sbytes, h->stream, *h->splitQ);
+        else fb_launch_fast_split<0>(envp, warps, threads, sbytes, h->stream, *h->splitQ);
       } else if (h->fast_block == 16) {
-        if (lean) fb_fast_kernel<16, 0, 0, 1><<<fblocks, 16, bytes, h->stream>>>(*h->fastQ);
-        else fb_fast_kernel<16, 0, 0><<<fblocks, 16, bytes, h->stream>>>(*h->fastQ);
+        if (lean) fb_launch_fast<16, 0, 0, 1>(envp, fblocks, 16, bytes, h->stream, *h->fastQ);
+        else fb_launch_fast<16, 0, 0, 0>(envp, fblocks, 16, bytes, h->stream, *h->fastQ);
       } else if (h->fast_slim && wpb > 1) {
-        if (lean) fb_fast_kernel<32, 1, 1, 1><<<wblocks, 32*wpb, bytes, h->stream>>>(*h->fastQ);
-        else fb_fast_kernel<32, 1, 1><<<wblocks, 32*wpb, bytes, h->stream>>>(*h->fastQ);
+        if (lean) fb_launch_fast<32, 1, 1, 1>(envp, wblocks, 32*wpb, bytes, h->stream, *h->fastQ);
+        else fb_launch_fast<32, 1, 1, 0>(envp, wblocks, 32*wpb, bytes, h->stream, *h->fastQ);
       } else if (h->fast_slim) {
-        if (lean) fb_fast_kernel<32, 1, 0, 1><<<warps, 32, bytes, h->stream>>>(*h->fastQ);
-        else fb_fast_kernel<32, 1, 0><<<warps, 32, bytes, h->stream>>>(*h->fastQ);
+        if (lean) fb_launch_fast<32, 1, 0, 1>(envp, warps, 32, bytes, h->stream, *h->fastQ);
+        else fb_launch_fast<32, 1, 0, 0>(envp, warps, 32, bytes, h->stream, *h->fastQ);
       } else {
-        if (lean) fb_fast_kernel<32, 0, 0, 1><<<warps, 32, bytes, h->stream>>>(*h->fastQ);
-        else fb_fast_kernel<32, 0, 0><<<warps, 32, bytes, h->stream>>>(*h->fastQ);
+        if (lean) fb_launch_fast<32, 0, 0, 1>(envp, warps, 32, bytes, h->stream, *h->fastQ);
+        else fb_launch_fast<32, 0, 0, 0>(envp, warps, 32, bytes, h->stream, *h->fastQ);
       }
     }
     h->launches++;
@@ -728,32 +793,32 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
       if (h->con_split && P.use_pending && !h->fast_slim && h->hm.split.nwarps > 1 && fb_con_split_pays(h)) {
         /* small ground-contact batch: the tree of every group split over several warps */
         P.con_split_done = h->con_split_done;
-        h->csplitQ->P = P;
+        h->csplitQ->P = P; h->csplitQ->T = h->ep;
         const size_t sbytes = h->fast_smem_bytes + (size_t)FB_CSPLIT_EXTRA*h->fast_block*sizeof(float);
         const int threads = 32*h->hm.split.nwarps;
         if (h->fast_block == 16) {
-          if (clean) fb_fastc_split_kernel<16, 1><<<fblocks, threads, sbytes, h->stream>>>(*h->csplitQ);
-          else fb_fastc_split_kernel<16, 0><<<fblocks, threads, sbytes, h->stream>>>(*h->csplitQ);
+          if (clean) fb_launch_fastc_split<16, 1>(envp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
+          else fb_launch_fastc_split<16, 0>(envp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
         } else {
-          if (clean) fb_fastc_split_kernel<32, 1><<<fblocks, threads, sbytes, h->stream>>>(*h->csplitQ);
-          else fb_fastc_split_kernel<32, 0><<<fblocks, threads, sbytes, h->stream>>>(*h->csplitQ);
+          if (clean) fb_launch_fastc_split<32, 1>(envp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
+          else fb_launch_fastc_split<32, 0>(envp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
         }
         h->launches++;
       }
-      h->conQ->P = P;
+      h->conQ->P = P; h->conQ->T = h->ep;
       if (h->fast_block == 16) {
-        if (clean) fb_fastc_kernel<16, 1><<<fblocks, 16, h->fast_smem_bytes, h->stream>>>(*h->conQ);
-        else fb_fastc_kernel<16><<<fblocks, 16, h->fast_smem_bytes, h->stream>>>(*h->conQ);
+        if (clean) fb_launch_fastc<16, 1>(envp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
+        else fb_launch_fastc<16, 0>(envp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
       } else {
-        if (clean) fb_fastc_kernel<32, 1><<<fblocks, 32, h->fast_smem_bytes, h->stream>>>(*h->conQ);
-        else fb_fastc_kernel<32><<<fblocks, 32, h->fast_smem_bytes, h->stream>>>(*h->conQ);
+        if (clean) fb_launch_fastc<32, 1>(envp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
+        else fb_launch_fastc<32, 0>(envp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
       }
     }
   }
   if (!con_thread) switch (h->team) {
-    case 8: fb_step_kernel<8><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P); break;
-    case 16: fb_step_kernel<16><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P); break;
-    default: fb_step_kernel<32><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P); break;
+    case 8: fb_step_kernel<8><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep); break;
+    case 16: fb_step_kernel<16><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep); break;
+    default: fb_step_kernel<32><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep); break;
   }
   cudaEventRecord(h->ev1, h->stream);
   {
@@ -799,9 +864,12 @@ static long long fb_con_split_blocks(FbHandle *h, int blk, cudaError_t *ce) {
   const size_t sbytes = ((size_t)h->hm.m.X.n_float + FB_CSPLIT_EXTRA)*blk*sizeof(float);
   if (!h->hm.m.X.con_ok || h->hm.split.nwarps < 2 || sbytes > (size_t)h->max_smem) return 0;
   int per_sm = 1 << 30;
-  for (int lean = 0; lean < 2 && *ce == cudaSuccess; lean++) {
-    const void *k = blk == 16 ? (lean ? (const void *)fb_fastc_split_kernel<16, 1> : (const void *)fb_fastc_split_kernel<16, 0>)
-                              : (lean ? (const void *)fb_fastc_split_kernel<32, 1> : (const void *)fb_fastc_split_kernel<32, 0>);
+  for (int v = 0; v < 4 && *ce == cudaSuccess; v++) {      /* LEAN x ENVP */
+    const void *k16[4] = {(const void *)fb_fastc_split_kernel<16, 0>, (const void *)fb_fastc_split_kernel<16, 1>,
+                          (const void *)fb_fastc_split_envp_kernel<16, 0>, (const void *)fb_fastc_split_envp_kernel<16, 1>};
+    const void *k32[4] = {(const void *)fb_fastc_split_kernel<32, 0>, (const void *)fb_fastc_split_kernel<32, 1>,
+                          (const void *)fb_fastc_split_envp_kernel<32, 0>, (const void *)fb_fastc_split_envp_kernel<32, 1>};
+    const void *k = blk == 16 ? k16[v] : k32[v];
     *ce = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
     if (*ce == cudaSuccess) *ce = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     int nb = 0;
@@ -816,9 +884,12 @@ static long long fb_con_single_blocks(FbHandle *h, int blk, cudaError_t *ce) {
   const size_t sbytes = (size_t)h->hm.m.X.n_float*blk*sizeof(float);
   if (!h->hm.m.X.con_ok || sbytes > (size_t)h->max_smem) return 0;
   int per_sm = 1 << 30;
-  for (int lean = 0; lean < 2 && *ce == cudaSuccess; lean++) {
-    const void *k = blk == 16 ? (lean ? (const void *)fb_fastc_kernel<16, 1> : (const void *)fb_fastc_kernel<16, 0>)
-                              : (lean ? (const void *)fb_fastc_kernel<32, 1> : (const void *)fb_fastc_kernel<32, 0>);
+  for (int v = 0; v < 4 && *ce == cudaSuccess; v++) {      /* LEAN x ENVP */
+    const void *k16[4] = {(const void *)fb_fastc_kernel<16, 0>, (const void *)fb_fastc_kernel<16, 1>,
+                          (const void *)fb_fastc_envp_kernel<16, 0>, (const void *)fb_fastc_envp_kernel<16, 1>};
+    const void *k32[4] = {(const void *)fb_fastc_kernel<32, 0>, (const void *)fb_fastc_kernel<32, 1>,
+                          (const void *)fb_fastc_envp_kernel<32, 0>, (const void *)fb_fastc_envp_kernel<32, 1>};
+    const void *k = blk == 16 ? k16[v] : k32[v];
     *ce = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
     if (*ce == cudaSuccess) *ce = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     int nb = 0;
@@ -855,15 +926,19 @@ static int fb_set_fast_block(FbHandle *h, int blk) {
   if (ce == cudaSuccess) ce = cudaFuncSetAttribute(K_, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes); \
   if (ce == cudaSuccess) ce = cudaFuncSetAttribute(K_, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
   switch (blk) {
-    case 16: FB_SET_SMEM((fb_fast_kernel<16, 0, 0>)) FB_SET_SMEM((fb_fast_kernel<16, 0, 0, 1>)) FB_SET_SMEM(fb_fastc_kernel<16>) FB_SET_SMEM((fb_fastc_kernel<16, 1>)) break;
-    default: FB_SET_SMEM((fb_fast_kernel<32, 0, 0>)) FB_SET_SMEM((fb_fast_kernel<32, 0, 0, 1>)) FB_SET_SMEM(fb_fastc_kernel<32>) FB_SET_SMEM((fb_fastc_kernel<32, 1>)) break;
+    case 16: FB_SET_SMEM((fb_fast_kernel<16, 0, 0>)) FB_SET_SMEM((fb_fast_kernel<16, 0, 0, 1>)) FB_SET_SMEM(fb_fastc_kernel<16>) FB_SET_SMEM((fb_fastc_kernel<16, 1>))
+             FB_SET_SMEM((fb_fast_envp_kernel<16, 0, 0>)) FB_SET_SMEM((fb_fast_envp_kernel<16, 0, 0, 1>)) FB_SET_SMEM(fb_fastc_envp_kernel<16>) FB_SET_SMEM((fb_fastc_envp_kernel<16, 1>)) break;
+    default: FB_SET_SMEM((fb_fast_kernel<32, 0, 0>)) FB_SET_SMEM((fb_fast_kernel<32, 0, 0, 1>)) FB_SET_SMEM(fb_fastc_kernel<32>) FB_SET_SMEM((fb_fastc_kernel<32, 1>))
+             FB_SET_SMEM((fb_fast_envp_kernel<32, 0, 0>)) FB_SET_SMEM((fb_fast_envp_kernel<32, 0, 0, 1>)) FB_SET_SMEM(fb_fastc_envp_kernel<32>) FB_SET_SMEM((fb_fastc_envp_kernel<32, 1>)) break;
   }
 #undef FB_SET_SMEM
   h->split_capacity = 0;
   if (blk == 32 && h->hm.split.nwarps > 1 && (size_t)bytes + FB_SPLIT_EXTRA_BYTES <= (size_t)h->max_smem) {
     int per_sm = 1 << 30;
-    for (int lean = 0; lean < 2 && ce == cudaSuccess; lean++) {
-      const void *k = lean ? (const void *)fb_fast_split_kernel<1> : (const void *)fb_fast_split_kernel<0>;
+    for (int v = 0; v < 4 && ce == cudaSuccess; v++) {      /* LEAN x ENVP */
+      const void *split_k[4] = {(const void *)fb_fast_split_kernel<0>, (const void *)fb_fast_split_kernel<1>,
+                                (const void *)fb_fast_split_envp_kernel<0>, (const void *)fb_fast_split_envp_kernel<1>};
+      const void *k = split_k[v];
       ce = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes + FB_SPLIT_EXTRA_BYTES);
       if (ce == cudaSuccess) ce = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
       int nb = 0;
@@ -884,14 +959,17 @@ static int fb_slim_attributes(FbHandle *h, int max_smem) {
   const int b1 = (int)h->fast_slim_smem_bytes;
   int fit = max_smem/b1;     /* warps of one block that fit an SM's shared memory */
   if (fit > 8) fit = 8;
-  cudaError_t ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, b1);
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 0>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 0, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, b1);
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 0, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  if (ce == cudaSuccess && fit >= 2) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fit*b1);
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  if (ce == cudaSuccess && fit >= 2) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 1, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fit*b1);
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(fb_fast_kernel<32, 1, 1, 1>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  const void *one[4] = {(const void *)fb_fast_kernel<32, 1, 0>, (const void *)fb_fast_kernel<32, 1, 0, 1>,
+                        (const void *)fb_fast_envp_kernel<32, 1, 0>, (const void *)fb_fast_envp_kernel<32, 1, 0, 1>};
+  const void *multi[4] = {(const void *)fb_fast_kernel<32, 1, 1>, (const void *)fb_fast_kernel<32, 1, 1, 1>,
+                          (const void *)fb_fast_envp_kernel<32, 1, 1>, (const void *)fb_fast_envp_kernel<32, 1, 1, 1>};
+  cudaError_t ce = cudaSuccess;
+  for (int v = 0; v < 4; v++) {      /* LEAN x ENVP */
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute(one[v], cudaFuncAttributeMaxDynamicSharedMemorySize, b1);
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute(one[v], cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+    if (ce == cudaSuccess && fit >= 2) ce = cudaFuncSetAttribute(multi[v], cudaFuncAttributeMaxDynamicSharedMemorySize, fit*b1);
+    if (ce == cudaSuccess) ce = cudaFuncSetAttribute(multi[v], cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+  }
   if (ce != cudaSuccess) return fail(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ce));
   if (h->fast_wpb > fit) h->fast_wpb = fit;
   if (h->fast_wpb < 2) h->fast_wpb = 1;
@@ -946,6 +1024,7 @@ void fb_destroy(FbHandle *h) {
   if (h->seq_dev) { dev_free(h->seq_dev); dev_free(h->seq_stage); }
   if (h->I_dev) dev_free(h->I_dev);
   if (h->F_dev) dev_free(h->F_dev);
+  for (float *p : h->ep_dev) if (p) dev_free(p);
 #ifndef FB_HOST_EMU
   cudaEventDestroy(h->ev0); cudaEventDestroy(h->ev1);
   cudaStreamSynchronize(h->copy_stream);
@@ -974,6 +1053,8 @@ int fb_create(const FbModel *model, const FbFarms *farms, int n_envs, int device
   FbHandle *h = new (std::nothrow) FbHandle();
   if (!h) return fail("out of host memory");
   h->device = device; h->I_dev = nullptr; h->F_dev = nullptr; h->launches = 0; h->it = 0;
+  for (float *&p : h->ep_dev) p = nullptr;
+  memset(&h->ep, 0, sizeof(h->ep));
   h->last_ms = 0.f; h->has_wc = false; h->gather_links = h->gather_joints = h->gather_env = nullptr;
   h->seq_dev = h->seq_stage = nullptr; h->seq_len = h->seq_pos = h->seq_cap = h->seq_rows = 0;
   h->cpg_on = false; memset(&h->cpg, 0, sizeof(h->cpg));
@@ -1404,9 +1485,99 @@ int fb_set_actuator_forcerange(FbHandle *h, int n, const int32_t *actuator, cons
 int fb_set_water_velocity(FbHandle *h, double vx, double vy, double vz) {
   if (!h) return fail("null handle");
   if (!h->has_farms) return fail("no farms tables");
+  if (h->ep_dev[FB_ENV_WATER_VELOCITY])
+    return fail("fb_set_water_velocity: a per-environment water velocity is set; change it with "
+                "fb_set_env_param(FB_ENV_WATER_VELOCITY, ...), or clear it with fb_set_env_param(FB_ENV_WATER_VELOCITY, NULL) first");
   h->ff_shallow.water_velocity[0] = vx; h->ff_shallow.water_velocity[1] = vy; h->ff_shallow.water_velocity[2] = vz;
   h->P.m.water_velocity[0] = (float)vx; h->P.m.water_velocity[1] = (float)vy; h->P.m.water_velocity[2] = (float)vz;
   h->hm.m.water_velocity[0] = (float)vx; h->hm.m.water_velocity[1] = (float)vy; h->hm.m.water_velocity[2] = (float)vz;
+  return 0;
+}
+
+/* ---- per-environment parameters (fb_set_env_param) */
+static const char *const kEnvParamName[4] = {"FB_ENV_JNT_STIFFNESS", "FB_ENV_DOF_DAMPING", "FB_ENV_DRAG_COEF",
+                                             "FB_ENV_WATER_VELOCITY"};
+
+/* values per environment of a field: njnt, nv, 6*n_swim, 3 */
+static int env_param_width(const FbHandle *h, int field) {
+  switch (field) {
+    case FB_ENV_JNT_STIFFNESS: return h->fm_shallow.njnt;
+    case FB_ENV_DOF_DAMPING: return h->fm_shallow.nv;
+    case FB_ENV_DRAG_COEF: return h->has_farms ? 6*h->ff_shallow.n_swim : 0;
+    default: return 3;
+  }
+}
+
+/* the model's value of entry c of a field */
+static double env_param_model(const FbHandle *h, int field, int c) {
+  switch (field) {
+    case FB_ENV_JNT_STIFFNESS: return h->fm_shallow.jnt_stiffness[c];
+    case FB_ENV_DOF_DAMPING: return h->fm_shallow.dof_damping[c];
+    case FB_ENV_DRAG_COEF: return h->ff_shallow.swim_coefficients[c];
+    default: return h->has_farms ? h->ff_shallow.water_velocity[c] : 0.0;
+  }
+}
+
+static void env_param_bind(FbHandle *h) {
+  h->ep.stiffness = h->ep_dev[FB_ENV_JNT_STIFFNESS];
+  h->ep.damping = h->ep_dev[FB_ENV_DOF_DAMPING];
+  h->ep.coef = h->ep_dev[FB_ENV_DRAG_COEF];
+  h->ep.wvel = h->ep_dev[FB_ENV_WATER_VELOCITY];
+}
+
+int fb_set_env_param(FbHandle *h, int field, const double *values) {
+  if (!h) return fail("null handle");
+  if (field < FB_ENV_JNT_STIFFNESS || field > FB_ENV_WATER_VELOCITY) return fail("fb_set_env_param: unknown field " + std::to_string(field));
+  const std::string name = std::string("fb_set_env_param(") + kEnvParamName[field] + ")";
+  if (!values) {                                    /* back to the model's value */
+    if (h->ep_dev[field]) { dev_sync(h->stream); dev_free(h->ep_dev[field]); h->ep_dev[field] = nullptr; }
+    h->ep_host[field].clear();
+    env_param_bind(h);
+    return 0;
+  }
+  if ((field == FB_ENV_DRAG_COEF || field == FB_ENV_WATER_VELOCITY) && (!h->has_farms || h->ff_shallow.n_swim <= 0))
+    return fail(name + ": the model has no swimming links");
+  const FbModel &fm = h->fm_shallow;
+  const int n = h->P.n_envs, w = env_param_width(h, field);
+  const long long pad = h->P.env_pad;
+  for (int e = 0; e < n; e++)
+    for (int c = 0; c < w; c++) {
+      const double v = values[(size_t)e*w + c];
+      const std::string at = " at environment " + std::to_string(e) + ", index " + std::to_string(c);
+      /* drag coefficients are negative in FARMS (the force opposes the motion) and a water velocity is
+       * a vector: only stiffness and damping have a sign to check */
+      const int signed_field = field == FB_ENV_DRAG_COEF || field == FB_ENV_WATER_VELOCITY;
+      if (!std::isfinite(v)) return fail(name + ": non-finite value" + at);
+      if (!signed_field && v < 0.0) return fail(name + ": negative value" + at);
+      const int free_entry = (field == FB_ENV_JNT_STIFFNESS && fm.jnt_type[c] == FB_JNT_FREE) ||
+                             (field == FB_ENV_DOF_DAMPING && fm.jnt_type[fm.dof_jntid[c]] == FB_JNT_FREE);
+      if (free_entry && v != 0.0) return fail(name + ": non-zero value on the free joint" + at);
+    }
+  std::vector<float> dev((size_t)w*pad, 0.f);
+  for (int e = 0; e < n; e++)
+    for (int c = 0; c < w; c++) dev[(size_t)c*pad + e] = (float)values[(size_t)e*w + c];
+  if (!h->ep_dev[field]) {
+    void *p = nullptr;
+    if (dev_alloc(&p, dev.size()*sizeof(float))) return fail(name + ": device allocation failed");
+    h->ep_dev[field] = static_cast<float *>(p);
+  }
+  if (h2d(h->ep_dev[field], dev.data(), dev.size()*sizeof(float), h->stream) || dev_sync(h->stream))
+    return fail(name + ": upload failed: " + dev_error());
+  h->ep_host[field].assign(values, values + (size_t)n*w);
+  env_param_bind(h);
+  return 0;
+}
+
+int fb_get_env_param(FbHandle *h, int field, double *out) {
+  if (!h || !out) return fail("null argument");
+  if (field < FB_ENV_JNT_STIFFNESS || field > FB_ENV_WATER_VELOCITY) return fail("fb_get_env_param: unknown field " + std::to_string(field));
+  const int n = h->P.n_envs, w = env_param_width(h, field);
+  if (h->ep_dev[field]) {
+    std::copy(h->ep_host[field].begin(), h->ep_host[field].end(), out);
+    return 0;
+  }
+  for (int e = 0; e < n; e++)
+    for (int c = 0; c < w; c++) out[(size_t)e*w + c] = env_param_model(h, field, c);
   return 0;
 }
 

@@ -211,7 +211,19 @@ template <int SYNC> FB_DEV void fb_block_sync() {
  * warps, each visiting its own bodies of the tree in two phases per sweep (FastSplit, fb_model.h);
  * the per-body code is the one every other variant runs, in the same order along every chain, so
  * the results are bit-identical to the single-warp kernel. */
-template <int BLK, int SLIM = 0, int LEAN = 0, int SPLIT = 0> struct FbFast {
+/* ENVP = 1 (fb_set_env_param): joint stiffness and damping, drag coefficients and water velocity
+ * come from the per-environment tables (FbEnvTables, `ept`) where one is set (a uniform null test
+ * per table), else from the records / the model as with ENVP = 0.  Same arithmetic on the values. */
+/* the tables' pointer is a member of the ENVP variants only: a member that the other variants never
+ * read still changed how ptxas scheduled the SLIM kernels */
+template <int ENVP> struct FbEnvRef {
+  const FbEnvTables *ept;   /* the per-environment parameter tables (kernel parameters) */
+  FB_MEM FbEnvRef(const FbEnvTables *ept_) : ept(ept_) {}
+};
+template <> struct FbEnvRef<0> {
+  FB_MEM FbEnvRef(const FbEnvTables *) {}
+};
+template <int BLK, int SLIM = 0, int LEAN = 0, int SPLIT = 0, int ENVP = 0> struct FbFast : FbEnvRef<ENVP> {
   /* SLIM scratch block: W[6] U 1/d trq q qd V[6] tc tu -- the first 17 are one contiguous run */
   enum { NF = SLIM ? 7 : FB_NF, GNF = SLIM ? FG_NF + 6 : FG_NF, FG_V = SLIM ? 11 : FG_NF,
          FGTC = SLIM ? 17 : FG_TC, FGTU = SLIM ? 18 : FG_TU };
@@ -245,8 +257,8 @@ template <int BLK, int SLIM = 0, int LEAN = 0, int SPLIT = 0> struct FbFast {
   float *sroot;
   int *sflag;
 
-  FB_MEM FbFast(const FbParams &P_, const FastRec *rec_, float *s_, float *gs_, int env_)
-      : P(P_), m(P_.m), rec(rec_), s(s_), env(env_), gs(gs_), cs(0), csc(0), crec(0) {
+  FB_MEM FbFast(const FbParams &P_, const FastRec *rec_, float *s_, float *gs_, int env_, const FbEnvTables *ept_ = 0)
+      : FbEnvRef<ENVP>(ept_), P(P_), m(P_.m), rec(rec_), s(s_), env(env_), gs(gs_), cs(0), csc(0), crec(0) {
     env_phase = P.env_phase[env];
     dirty_c = P.con_dirty[env];
     zfill = 1;
@@ -741,6 +753,16 @@ FB_UNROLL
       for (int k = 0; k < 3; k++) { FB_PIN_F(rc.hloc[k]); FB_PIN_F(rc.axis[k]); }
 FB_UNROLL
       for (int k = 0; k < 5; k++) FB_PIN_F(rc.Ib[k]);
+      float estiff = 0.f, edamp = 0.f;       /* ENVP: this environment's values, loads issued here */
+      if constexpr (ENVP) {
+        const FbEnvTables *ept = this->ept;
+        estiff = rc.stiffness; edamp = rc.damping;
+        if (rc.jtype > FB_JNT_FREE) {
+          if (ept->stiffness) estiff = ept->stiffness[(size_t)rc.jid*P.env_pad + env];
+          if (ept->damping) edamp = ept->damping[(size_t)rc.da*P.env_pad + env];
+        }
+        FB_PIN_F(estiff); FB_PIN_F(edamp);
+      }
       if (SPLIT) { pb = block(b); pg = gblock(b); }
       else { pb -= NF*BLK; pg -= GNF*BLK; }
       const int jtype = rc.jtype, flags = rc.flags;
@@ -885,13 +907,13 @@ FB_UNROLL
         } else {
           actuation_generic(rc, qj, qd, time, store_ctrl, seqk, &tau, &trq);
         }
-        if (rc.stiffness != 0.f) {
+        if ((ENVP ? estiff : rc.stiffness) != 0.f) {
           /* spring reference of this step: a row of the control sequence (on-device CPG), else held */
           const float ref = (!LEAN && seqk && FT_SREF(flags) >= 0) ? seqk[(long long)(m.nu + FT_SREF(flags))*P.env_pad]
                                                            : P.qpos_spring[(size_t)env*m.nq + rc.qa];
-          tau -= rc.stiffness*(qj - ref);
+          tau -= (ENVP ? estiff : rc.stiffness)*(qj - ref);
         }
-        tau -= rc.damping*qd;
+        tau -= (ENVP ? edamp : rc.damping)*qd;
         if (MODE == 2) tau += fb_ld_scr(nblock(b) + NB_TAUC*BLK);
         float d, u;
         float aq[3] = {ax[0]*qd, ax[1]*qd, ax[2]*qd};
@@ -910,7 +932,7 @@ FB_UNROLL
           c[0] = c[1] = c[2] = 0.f;
           v_cross(v, aq, c + 3);
         }
-        d += MODE == 1 ? rc.armature : rc.armature + hdt*rc.damping;
+        d += MODE == 1 ? rc.armature : rc.armature + hdt*(ENVP ? edamp : rc.damping);
         const float dinv = fb_rcp(d);
         /* Ia = I - U U'/d */
         sym_rank1(I.A, U, dinv);
@@ -1012,6 +1034,18 @@ FB_UNROLL
       for (int k = 0; k < 3; k++) { FB_PIN_F(rc.hloc[k]); FB_PIN_F(rc.axis[k]); }
 FB_UNROLL
       for (int k = 0; k < 6; k++) FB_PIN_F(rc.coef[k]);
+      float ecoef[6], ewv[3];                /* ENVP: this environment's drag values, loads issued here */
+      if constexpr (ENVP) if (rc.swim >= 0) {
+        const FbEnvTables *ept = this->ept;
+FB_UNROLL
+        for (int k = 0; k < 6; k++) ecoef[k] = ept->coef ? ept->coef[(size_t)(6*rc.swim + k)*P.env_pad + env] : rc.coef[k];
+FB_UNROLL
+        for (int k = 0; k < 3; k++) ewv[k] = ept->wvel ? ept->wvel[(size_t)k*P.env_pad + env] : m.water_velocity[k];
+FB_UNROLL
+        for (int k = 0; k < 6; k++) FB_PIN_F(ecoef[k]);
+FB_UNROLL
+        for (int k = 0; k < 3; k++) FB_PIN_F(ewv[k]);
+      }
       if (SPLIT) { pb = block(b); pg = gblock(b); }
       else { pb += NF*BLK; pg += GNF*BLK; }
       const int jtype = rc.jtype, flags = rc.flags;
@@ -1176,13 +1210,14 @@ FB_UNROLL
               float frac = fminf(fmaxf(m.water_surface - pz, 0.f)/rc.height, 1.f);
               m_rot_t(R, 0.f, 0.f, rc.lift*frac, buoy);
             }
-            m_rot_t(R, m.water_velocity[0], m.water_velocity[1], m.water_velocity[2], uw);
+            if (ENVP) m_rot_t(R, ewv[0], ewv[1], ewv[2], uw);
+            else m_rot_t(R, m.water_velocity[0], m.water_velocity[1], m.water_velocity[2], uw);
 FB_UNROLL
             for (int k = 0; k < 3; k++) {
               float vv = vl[k] - uw[k], w = wl[k];
               float sv = vv < 0.f ? -vv*vv : vv*vv, sw = w < 0.f ? -w*w : w*w;
-              F[k] = sv*m.water_viscosity*rc.coef[k] + buoy[k];
-              Tq[k] = sw*rc.coef[3 + k];
+              F[k] = sv*m.water_viscosity*(ENVP ? ecoef[k] : rc.coef[k]) + buoy[k];
+              Tq[k] = sw*(ENVP ? ecoef[3 + k] : rc.coef[3 + k]);
             }
             m_rot(R, F[0], F[1], F[2], wf);
             m_rot(R, Tq[0], Tq[1], Tq[2], wt);

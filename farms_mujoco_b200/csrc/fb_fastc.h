@@ -68,8 +68,9 @@ static double *fb_emu_stats = 0;
  * another order than on one warp: results agree with the single-warp kernel to rounding, not bit
  * for bit. */
 #define FB_RED_MAX 8       /* values of one cross-warp reduction */
-template <int BLK, int LEAN = 0, int SPLIT = 0> struct FbFastCon : FbFast<BLK, 0, LEAN, SPLIT> {
-  typedef FbFast<BLK, 0, LEAN, SPLIT> Base;
+/* ENVP: as in FbFast (per-environment stiffness, damping, drag coefficients, water velocity). */
+template <int BLK, int LEAN = 0, int SPLIT = 0, int ENVP = 0> struct FbFastCon : FbFast<BLK, 0, LEAN, SPLIT, ENVP> {
+  typedef FbFast<BLK, 0, LEAN, SPLIT, ENVP> Base;
   using Base::P; using Base::m; using Base::rec; using Base::s; using Base::env; using Base::gs;
   using Base::cs; using Base::csc; using Base::crec; using Base::hm; using Base::hany;
   using Base::rt; using Base::rootpos; using Base::rqn;
@@ -135,8 +136,8 @@ FB_UNROLL
   FB_MEM float *wslot(int i) const { return csw + 6*BLK*i; }
 
   FB_MEM FbFastCon(const FbParams &P_, const FastRec *rec_, const CandRec *crec_, float *s_, float *gs_,
-                   float *cs_, int env_)
-      : Base(P_, rec_, s_, gs_, env_) {
+                   float *cs_, int env_, const FbEnvTables *ept_ = 0)
+      : Base(P_, rec_, s_, gs_, env_, ept_) {
     cs = cs_; crec = crec_;
     csc = cs_ + (NB_NF*(P_.m.nbody - 1) + NR_NF)*BLK;
     csw = csc + NC_NF*P_.m.ncand*BLK;

@@ -45,6 +45,8 @@ ABI_SYMBOLS = {
     'fb_set_actuator_forcerange': (ct.c_int, [_H, ct.c_int, ct.POINTER(ct.c_int32), ct.POINTER(ct.c_int32), cabi.c_double_p]),
     'fb_set_water_velocity': (ct.c_int, [_H, ct.c_double, ct.c_double, ct.c_double]),
     'fb_set_swimming': (ct.c_int, [_H, ct.c_int, ct.c_int]),
+    'fb_set_env_param': (ct.c_int, [_H, ct.c_int, cabi.c_double_p]),
+    'fb_get_env_param': (ct.c_int, [_H, ct.c_int, cabi.c_double_p]),
     'fb_step': (ct.c_int, [_H, ct.c_int, ct.c_int, ct.c_int]),
     'fb_synchronize': (ct.c_int, [_H]),
     'fb_last_step_ms': (ct.c_int, [_H, ct.POINTER(ct.c_float)]),
@@ -391,6 +393,49 @@ class BatchedPhysics:
 
     def set_swimming(self, drag, buoyancy):
         self._check(self.lib.fb_set_swimming(self._handle, int(bool(drag)), int(bool(buoyancy))))
+
+    # fb_set_env_param fields (include/farms_b200.h FB_ENV_*): keyword -> (field, shape of one environment)
+    def _env_param_fields(self):
+        n_swim = len(self.tables.swim_links_index)
+        return {'jnt_stiffness': (0, (self.model.njnt,)), 'dof_damping': (1, (self.model.nv,)),
+                'drag_coefficients': (2, (n_swim, 2, 3)), 'water_velocity': (3, (3,))}
+
+    def set_env_params(self, **fields):
+        """Per-environment physical parameters (fb_set_env_param): ``jnt_stiffness [n_envs, njnt]``,
+        ``dof_damping [n_envs, nv]``, ``drag_coefficients [n_envs, n_swim, 2, 3]`` (the layout of
+        ``FarmsTables.swim_coefficients``) and ``water_velocity [n_envs, 3]``.  Environment ``e`` then
+        steps as the model edited to its values.  Only the keywords passed change; ``None`` returns a
+        field to the model's value; an array without the environment axis is broadcast to every
+        environment.  The tables survive ``reset``."""
+        known = self._env_param_fields()
+        for name in fields:
+            if name not in known:
+                raise TypeError(f'set_env_params: unknown field {name!r} (one of {", ".join(known)})')
+        for name, values in fields.items():
+            field, shape = known[name]
+            if values is None:
+                self._check(self.lib.fb_set_env_param(self._handle, field, None))
+                continue
+            arr = np.asarray(values, dtype=np.float64)
+            if arr.shape != (self.n_envs,) + shape:
+                try:
+                    arr = np.broadcast_to(arr, (self.n_envs,) + shape)
+                except ValueError:
+                    raise ValueError(f'set_env_params: {name} must be {list(shape)} or '
+                                     f'{[self.n_envs] + list(shape)}, got {list(arr.shape)}') from None
+            arr = np.ascontiguousarray(arr)
+            self._check(self.lib.fb_set_env_param(self._handle, field, arr.ctypes.data_as(cabi.c_double_p)))
+
+    def env_params(self):
+        """The four fields of ``set_env_params`` as float64 ``[n_envs, ...]`` arrays (the model's value
+        broadcast for a field that is not set)."""
+        out = {}
+        for name, (field, shape) in self._env_param_fields().items():
+            arr = np.zeros((self.n_envs,) + shape, dtype=np.float64)
+            if arr.size:
+                self._check(self.lib.fb_get_env_param(self._handle, field, arr.ctypes.data_as(cabi.c_double_p)))
+            out[name] = arr
+        return out
 
     # --------------------------------------------------------------- views
     @property

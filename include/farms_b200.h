@@ -229,6 +229,24 @@ int fb_set_water_velocity(FbHandle *h, double vx, double vy, double vz);
 /* Drag on/off overrides for the fused swimming step (drag.pyx:393-395). */
 int fb_set_swimming(FbHandle *h, int drag, int buoyancy);
 
+/* Per-environment physical parameters (parameter sweeps, domain randomisation): each field is either
+ * the model's value for every environment (default) or a table of one value set per environment.
+ *   FB_ENV_JNT_STIFFNESS   [n_envs][njnt]     model.jnt_stiffness
+ *   FB_ENV_DOF_DAMPING     [n_envs][nv]       model.dof_damping
+ *   FB_ENV_DRAG_COEF       [n_envs][n_swim][2][3]  FbFarms.swim_coefficients (linear xyz, angular xyz)
+ *   FB_ENV_WATER_VELOCITY  [n_envs][3]        FbFarms.water_velocity
+ * Environment e then steps exactly as the model edited to e's values.  values: host float64; NULL
+ * returns the field to the model's value.  Refused, with the field and the first bad index named:
+ * non-finite values, negative stiffness or damping (drag coefficients are negative in FARMS and a
+ * water velocity has any sign), a non-zero stiffness or damping
+ * on the free joint, drag coefficients or water velocity on a model without swimming links.  The
+ * tables survive fb_reset and are freed by fb_destroy; while FB_ENV_WATER_VELOCITY is set,
+ * fb_set_water_velocity is refused.  fb_get_env_param returns the values in the same layout (the
+ * model's value broadcast for a field that is not set). */
+enum { FB_ENV_JNT_STIFFNESS = 0, FB_ENV_DOF_DAMPING = 1, FB_ENV_DRAG_COEF = 2, FB_ENV_WATER_VELOCITY = 3 };
+int fb_set_env_param(FbHandle *h, int field, const double *values);
+int fb_get_env_param(FbHandle *h, int field, double *out);
+
 /* Advance every environment by n_steps physics steps (simulation.py:155-156
  * env.step -> mj_step, with task.before_step's sensor logging, the swimming
  * callback and the controller fused in).  Step j writes log row (j+1) % ring.
