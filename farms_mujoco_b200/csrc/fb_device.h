@@ -91,6 +91,10 @@ struct EnvPtrs {
    * item i at ep_*[(i*k + c)*ep_pad]; NULL = the model's value */
   const float *ep_stiffness, *ep_damping, *ep_coef, *ep_wvel;
   long long ep_pad;
+  /* sliding friction of candidate c at fric[c*fric_stride]: this environment's column of the
+   * FB_ENV_CAND_FRICTION table (stride env_pad), else the model's cand_friction (stride 1) */
+  const float *fric;
+  int fric_stride;
 };
 
 /* vector widths of the device log (floats of one row stored contiguously per environment) */
@@ -297,6 +301,10 @@ template <int TEAM> struct FbStep {
         comx(0.f), comy(0.f), comz(0.f), ncon(0), nlim(0), npair_act(0), nhard_act(0) {}
 
   FB_MEM void sync() { T::sync(mask); }
+
+  /* sliding friction of candidate c: this environment's where FB_ENV_CAND_FRICTION is set (one load
+   * without a branch either way: the branch cost the table-free team kernel 1 %) */
+  FB_MEM float cand_mu(int c) const { return FB_LDG(g.fric + c*g.fric_stride); }
 
   /* ------------------------------------------------------------ init */
   FB_MEM void init_world() {
@@ -915,7 +923,7 @@ FB_UNROLL
     j3_times(qvel);  /* prod3 <- J3 qvel */
     for (int i = lane; i < ncon; i += TEAM) {
       int c = con_cand[i];
-      float mu = MF(cand_friction, c), dist = g.d_con_dist[i];
+      float mu = cand_mu(c), dist = g.d_con_dist[i];
       float includemargin = MF(cand_margin, c) - MF(cand_gap, c);
       float sr[2] = {MF(cand_solref, 2*c), MF(cand_solref, 2*c+1)}, si5[5];
       for (int k = 0; k < 5; k++) si5[k] = MF(cand_solimp, 5*c + k);
@@ -975,7 +983,7 @@ FB_UNROLL
     }
     const int *con_cand = si + m.L.con_cand;
     for (int i = lane; i < ncon; i += TEAM) {
-      float mu = MF(cand_friction, con_cand[i]);
+      float mu = cand_mu(con_cand[i]);
       float pn = g.prod3[3*i], p1 = g.prod3[3*i+1], p2 = g.prod3[3*i+2];
       int r = 2*nj + 4*i;
       out[r] = pn + mu*p1; out[r+1] = pn - mu*p1; out[r+2] = pn + mu*p2; out[r+3] = pn - mu*p2;
@@ -989,7 +997,7 @@ FB_UNROLL
     const int *con_cand = si + m.L.con_cand;
     float *y3 = g.prod3 + 3*m.maxcon;
     for (int i = lane; i < ncon; i += TEAM) {
-      float mu = MF(cand_friction, con_cand[i]);
+      float mu = cand_mu(con_cand[i]);
       const float *yy = y + 2*nj + 4*i;
       y3[3*i] = yy[0] + yy[1] + yy[2] + yy[3];
       y3[3*i+1] = mu*(yy[0] - yy[1]);
@@ -1313,7 +1321,7 @@ FB_UNROLL
           float h = H[idx];
           for (int i = 0; i < ncon; i++) {
             const int r = 2*nj + 4*i;
-            const float d = D[r], mu = MF(cand_friction, con_cand[i]);
+            const float d = D[r], mu = cand_mu(con_cand[i]);
             const float nu_ = g.J3[(3*i)*nv + u], nv_ = g.J3[(3*i)*nv + v];
             const float t1u = mu*g.J3[(3*i+1)*nv + u], t1v = mu*g.J3[(3*i+1)*nv + v];
             const float t2u = mu*g.J3[(3*i+2)*nv + u], t2v = mu*g.J3[(3*i+2)*nv + v];
@@ -1356,7 +1364,7 @@ FB_UNROLL
             /* u on the chain of b implies v on it too */
             if (!(((unsigned)MI(body_ancmask, b*m.nmaskw + (u >> 5)) >> (u & 31)) & 1u)) continue;
             int r = 2*nj + 4*i;
-            float d = D[r], mu = MF(cand_friction, c);
+            float d = D[r], mu = cand_mu(c);
             float nu_ = g.J3[(3*i)*nv + u], nv_ = g.J3[(3*i)*nv + v];
             float t1u = mu*g.J3[(3*i+1)*nv + u], t1v = mu*g.J3[(3*i+1)*nv + v];
             float t2u = mu*g.J3[(3*i+2)*nv + u], t2v = mu*g.J3[(3*i+2)*nv + v];
@@ -1464,7 +1472,7 @@ FB_UNROLL
       limf[j] = D[2*j] > 0.f ? frc[2*j] : (D[2*j+1] > 0.f ? frc[2*j+1] : 0.f);
     }
     for (int i = lane; i < ncon; i += TEAM) {
-      float mu = MF(cand_friction, con_cand[i]);
+      float mu = cand_mu(con_cand[i]);
       const float *f = frc + 2*nj + 4*i;
       g.d_con_force[3*i] = f[0] + f[1] + f[2] + f[3];
       g.d_con_force[3*i+1] = (f[0] - f[1])*mu;
@@ -1777,12 +1785,15 @@ struct FbParams {
 
 /* Per-environment parameter tables (fb_set_env_param), float32 environment-minor: value c of item i
  * of environment env at [(i*k + c)*env_pad + env] -- jnt_stiffness [njnt], dof_damping [nv], drag
- * coefficients [n_swim][6], water velocity [3].  NULL: the model's value for every environment.
+ * coefficients [n_swim][6], water velocity [3], candidate friction [ncand].  NULL: the model's value
+ * for every environment.
  * A launch argument of its own (not a member of FbParams), so that the parameter blocks of the
  * kernels that do not read it keep their layout: the team kernel tests the pointers at run time,
- * the per-thread kernels read them in their ENVP twins only. */
+ * the per-thread kernels read them in their ENVP twins only (the unconstrained twins never read
+ * `fric`: the member is last, so the members they read keep their offsets). */
 struct FbEnvTables {
   const float *stiffness, *damping, *coef, *wvel;
+  const float *fric;
 };
 
 #define FB_NEVER_DIRTY (-(1LL << 60))
@@ -1818,6 +1829,8 @@ FB_DEV EnvPtrs fb_env_ptrs(const FbParams &P, const FbEnvTables &T, int env) {
   g.ep_coef = T.coef ? T.coef + e : 0;
   g.ep_wvel = T.wvel ? T.wvel + e : 0;
   g.ep_pad = P.env_pad;
+  g.fric = T.fric ? T.fric + e : m.F + m.o.cand_friction;
+  g.fric_stride = T.fric ? (int)P.env_pad : 1;
   return g;
 }
 

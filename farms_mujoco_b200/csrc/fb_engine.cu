@@ -98,8 +98,10 @@ struct FbFastParams {
 /* BLK environments per warp (32, or 16 in a half-filled warp).  MULTI: blocks of 2..8 warps
  * (blockDim.x/32) kept in step by a barrier per physics step (FbFast::run_t). */
 /* Every per-thread entry point has an ENVP twin (fb_*_envp_kernel, same template arguments) that reads
- * the per-environment parameter tables of fb_set_env_param; launch() takes the twin while any table
- * is set.  An entry point and its twin expand the same body (FB_*_BODY: ENVP is a template argument
+ * the per-environment parameter tables of fb_set_env_param; launch() takes the twin while a table the
+ * kernel reads is set: any table for the constrained kernels, any but the candidate friction for the
+ * unconstrained ones (they have no contacts).  An entry point and its twin expand the same body
+ * (FB_*_BODY: ENVP is a template argument
  * of FbFast / FbFastCon, T the tables); written out in each kernel rather than called as an inlined
  * function, which ptxas was found to schedule differently.  A twin's parameters are the entry
  * point's with the tables appended; the entry point's keep their layout. */
@@ -385,6 +387,8 @@ __global__ void fb_gather_env_kernel(const float *__restrict__ log, int ring, in
 #endif
 
 /* ---------------------------------------------------------------- handle */
+enum { FB_N_ENV_PARAM = FB_ENV_CAND_FRICTION + 1 };     /* fields of fb_set_env_param */
+
 struct FbHandle {
   FbHostModel hm;
   FbParams P;
@@ -420,8 +424,8 @@ struct FbHandle {
   float *F_dev;
   /* per-environment parameter tables (fb_set_env_param), indexed by FB_ENV_*: the device copy
    * (FbParams::ep_*, float32 [item*k + c][env_pad]) and the values as set ([n_envs][width]) */
-  float *ep_dev[4];
-  std::vector<double> ep_host[4];
+  float *ep_dev[FB_N_ENV_PARAM];
+  std::vector<double> ep_host[FB_N_ENV_PARAM];
   FbEnvTables ep;                   /* ep_dev as the kernels take it */
   long long launches;
   long long it;            /* physics steps since reset */
@@ -580,6 +584,7 @@ static int upload_model(FbHandle *h) {
 #ifndef FB_HOST_EMU
 static int fb_set_fast_block(FbHandle *h, int blk);
 static long long fb_con_split_blocks(FbHandle *h, int blk, cudaError_t *ce);
+
 static long long fb_con_cost(long long n_envs, int blk, long long capacity, int split);
 static bool fb_con_split_pays(FbHandle *h);
 #endif
@@ -616,10 +621,11 @@ template <class F> static void emu_split_run(int nw, F body) {
 #endif
 
 #ifdef FB_HOST_EMU
-/* test harness: the per-thread kernels (ENVP: their twins) run serially on the host */
-template <int ENVP> static void emu_per_thread(FbHandle *h, FbParams &P, int n_steps, int con_thread) {
+/* test harness: the per-thread kernels run serially on the host (ENVP: the unconstrained kernels'
+ * twins, CENVP: the constrained kernels') */
+template <int ENVP, int CENVP> static void emu_per_thread(FbHandle *h, FbParams &P, int n_steps, int con_thread) {
   const DevModel &m = P.m;
-  const FbEnvTables *T = ENVP ? &h->ep : nullptr;
+  const FbEnvTables *T = ENVP ? &h->ep : nullptr, *CT = CENVP ? &h->ep : nullptr;
   P.pending_count[P.parity ^ 1] = 0;
   std::vector<float> fs((size_t)m.X.n_float + 8, 0.f);
   std::vector<float> fg((size_t)(m.X.n_scratch > m.X.n_scratch_slim ? m.X.n_scratch : m.X.n_scratch_slim) + 8, 0.f);
@@ -663,12 +669,12 @@ template <int ENVP> static void emu_per_thread(FbHandle *h, FbParams &P, int n_s
         const bool lean = h->fast_lean && m.X.lean && !P.ctrl_seq;
         emu_split_run(sp.nwarps, [&](int role) {
           if (lean) {
-            FbFastCon<1, 1, 1, ENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, T);
+            FbFastCon<1, 1, 1, CENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, CT);
             st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
             st.con_split_setup(sp, extra.data() + 4);
             st.run_con_split(0, 0);
           } else {
-            FbFastCon<1, 0, 1, ENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, T);
+            FbFastCon<1, 0, 1, CENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, CT);
             st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
             st.con_split_setup(sp, extra.data() + 4);
             st.run_con_split(0, 0);
@@ -677,10 +683,10 @@ template <int ENVP> static void emu_per_thread(FbHandle *h, FbParams &P, int n_s
         continue;
       }
       if (h->fast_lean && m.X.lean && !P.ctrl_seq) {
-        FbFastCon<1, 1, 0, ENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, T);
+        FbFastCon<1, 1, 0, CENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, CT);
         st.run_con(P.steps_done[env], 0, 0);
       } else {
-        FbFastCon<1, 0, 0, ENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, T);
+        FbFastCon<1, 0, 0, CENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, CT);
         st.run_con(P.steps_done[env], 0, 0);
       }
     }
@@ -717,8 +723,10 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
     if (h->seq_pos == h->seq_len) h->seq_len = h->seq_pos = 0;     /* consumed: ctrl is held again */
   }
   const int use_fast = h->fast_enabled && P.m.X.ok && mode == FB_MODE_STEP && !want_derived;
-  /* the per-thread kernels' ENVP twins while a per-environment parameter table is set */
+  /* the per-thread kernels' ENVP twins while a per-environment parameter table they read is set: the
+   * unconstrained kernels never read the candidate friction */
   const bool envp = h->ep.stiffness || h->ep.damping || h->ep.coef || h->ep.wvel;
+  const bool cenvp = envp || h->ep.fric;
   const int con_thread = use_fast && h->con_thread && P.m.X.con_ok;
   P.use_pending = use_fast;
   P.parity = (int)(h->launch_parity & 1);
@@ -726,8 +734,9 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
 #ifdef FB_HOST_EMU
   const DevModel &m = P.m;
   if (use_fast) {
-    if (envp) emu_per_thread<1>(h, P, n_steps, con_thread);
-    else emu_per_thread<0>(h, P, n_steps, con_thread);
+    if (envp) emu_per_thread<1, 1>(h, P, n_steps, con_thread);
+    else if (cenvp) emu_per_thread<0, 1>(h, P, n_steps, con_thread);
+    else emu_per_thread<0, 0>(h, P, n_steps, con_thread);
   }
   std::vector<float> s((size_t)m.L.n_float + 8, 0.f);
   std::vector<int> si((size_t)m.L.n_int + 8, 0);
@@ -797,21 +806,21 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
         const size_t sbytes = h->fast_smem_bytes + (size_t)FB_CSPLIT_EXTRA*h->fast_block*sizeof(float);
         const int threads = 32*h->hm.split.nwarps;
         if (h->fast_block == 16) {
-          if (clean) fb_launch_fastc_split<16, 1>(envp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
-          else fb_launch_fastc_split<16, 0>(envp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
+          if (clean) fb_launch_fastc_split<16, 1>(cenvp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
+          else fb_launch_fastc_split<16, 0>(cenvp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
         } else {
-          if (clean) fb_launch_fastc_split<32, 1>(envp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
-          else fb_launch_fastc_split<32, 0>(envp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
+          if (clean) fb_launch_fastc_split<32, 1>(cenvp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
+          else fb_launch_fastc_split<32, 0>(cenvp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
         }
         h->launches++;
       }
       h->conQ->P = P; h->conQ->T = h->ep;
       if (h->fast_block == 16) {
-        if (clean) fb_launch_fastc<16, 1>(envp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
-        else fb_launch_fastc<16, 0>(envp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
+        if (clean) fb_launch_fastc<16, 1>(cenvp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
+        else fb_launch_fastc<16, 0>(cenvp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
       } else {
-        if (clean) fb_launch_fastc<32, 1>(envp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
-        else fb_launch_fastc<32, 0>(envp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
+        if (clean) fb_launch_fastc<32, 1>(cenvp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
+        else fb_launch_fastc<32, 0>(cenvp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
       }
     }
   }
@@ -1495,15 +1504,20 @@ int fb_set_water_velocity(FbHandle *h, double vx, double vy, double vz) {
 }
 
 /* ---- per-environment parameters (fb_set_env_param) */
-static const char *const kEnvParamName[4] = {"FB_ENV_JNT_STIFFNESS", "FB_ENV_DOF_DAMPING", "FB_ENV_DRAG_COEF",
-                                             "FB_ENV_WATER_VELOCITY"};
+static const char *const kEnvParamName[FB_N_ENV_PARAM] = {"FB_ENV_JNT_STIFFNESS", "FB_ENV_DOF_DAMPING", "FB_ENV_DRAG_COEF",
+                                                          "FB_ENV_WATER_VELOCITY", "FB_ENV_CAND_FRICTION"};
 
-/* values per environment of a field: njnt, nv, 6*n_swim, 3 */
+/* Lowest candidate friction a table may hold (mjcf_subset.PAIR_MIN_FRICTION): the pyramid rows'
+ * D = 1/(2 mu^2 R) stiffens as 1/mu^2, and the fp32 solver's error grows with it (DESIGN.md section 8) */
+#define FB_MIN_ENV_FRICTION 0.1
+
+/* values per environment of a field: njnt, nv, 6*n_swim, 3, ncand */
 static int env_param_width(const FbHandle *h, int field) {
   switch (field) {
     case FB_ENV_JNT_STIFFNESS: return h->fm_shallow.njnt;
     case FB_ENV_DOF_DAMPING: return h->fm_shallow.nv;
     case FB_ENV_DRAG_COEF: return h->has_farms ? 6*h->ff_shallow.n_swim : 0;
+    case FB_ENV_CAND_FRICTION: return h->fm_shallow.ncand;
     default: return 3;
   }
 }
@@ -1514,6 +1528,7 @@ static double env_param_model(const FbHandle *h, int field, int c) {
     case FB_ENV_JNT_STIFFNESS: return h->fm_shallow.jnt_stiffness[c];
     case FB_ENV_DOF_DAMPING: return h->fm_shallow.dof_damping[c];
     case FB_ENV_DRAG_COEF: return h->ff_shallow.swim_coefficients[c];
+    case FB_ENV_CAND_FRICTION: return h->fm_shallow.cand_friction[c];
     default: return h->has_farms ? h->ff_shallow.water_velocity[c] : 0.0;
   }
 }
@@ -1523,11 +1538,12 @@ static void env_param_bind(FbHandle *h) {
   h->ep.damping = h->ep_dev[FB_ENV_DOF_DAMPING];
   h->ep.coef = h->ep_dev[FB_ENV_DRAG_COEF];
   h->ep.wvel = h->ep_dev[FB_ENV_WATER_VELOCITY];
+  h->ep.fric = h->ep_dev[FB_ENV_CAND_FRICTION];
 }
 
 int fb_set_env_param(FbHandle *h, int field, const double *values) {
   if (!h) return fail("null handle");
-  if (field < FB_ENV_JNT_STIFFNESS || field > FB_ENV_WATER_VELOCITY) return fail("fb_set_env_param: unknown field " + std::to_string(field));
+  if (field < 0 || field >= FB_N_ENV_PARAM) return fail("fb_set_env_param: unknown field " + std::to_string(field));
   const std::string name = std::string("fb_set_env_param(") + kEnvParamName[field] + ")";
   if (!values) {                                    /* back to the model's value */
     if (h->ep_dev[field]) { dev_sync(h->stream); dev_free(h->ep_dev[field]); h->ep_dev[field] = nullptr; }
@@ -1537,13 +1553,15 @@ int fb_set_env_param(FbHandle *h, int field, const double *values) {
   }
   if ((field == FB_ENV_DRAG_COEF || field == FB_ENV_WATER_VELOCITY) && (!h->has_farms || h->ff_shallow.n_swim <= 0))
     return fail(name + ": the model has no swimming links");
+  if (field == FB_ENV_CAND_FRICTION && h->fm_shallow.ncand <= 0) return fail(name + ": the model has no collision candidates");
   const FbModel &fm = h->fm_shallow;
   const int n = h->P.n_envs, w = env_param_width(h, field);
   const long long pad = h->P.env_pad;
   for (int e = 0; e < n; e++)
     for (int c = 0; c < w; c++) {
       const double v = values[(size_t)e*w + c];
-      const std::string at = " at environment " + std::to_string(e) + ", index " + std::to_string(c);
+      const std::string at = " at environment " + std::to_string(e) +
+                             (field == FB_ENV_CAND_FRICTION ? ", candidate " : ", index ") + std::to_string(c);
       /* drag coefficients are negative in FARMS (the force opposes the motion) and a water velocity is
        * a vector: only stiffness and damping have a sign to check */
       const int signed_field = field == FB_ENV_DRAG_COEF || field == FB_ENV_WATER_VELOCITY;
@@ -1552,6 +1570,17 @@ int fb_set_env_param(FbHandle *h, int field, const double *values) {
       const int free_entry = (field == FB_ENV_JNT_STIFFNESS && fm.jnt_type[c] == FB_JNT_FREE) ||
                              (field == FB_ENV_DOF_DAMPING && fm.jnt_type[fm.dof_jntid[c]] == FB_JNT_FREE);
       if (free_entry && v != 0.0) return fail(name + ": non-zero value on the free joint" + at);
+      if (field == FB_ENV_CAND_FRICTION) {
+        /* an explicit <pair> takes its friction from the pair element, not from the geoms */
+        const int pair = fm.cand_end[c] == 20 || fm.cand_end[c] == 21;
+        if (pair && v != fm.cand_friction[c])
+          return fail(name + ": " + std::to_string(v) + " differs from the <pair> candidate's friction " +
+                      std::to_string(fm.cand_friction[c]) + at + " (pair frictions stay per model)");
+        if (!pair && v < FB_MIN_ENV_FRICTION)
+          return fail(name + ": friction " + std::to_string(v) + " below 0.1" + at + ": the pyramid rows stiffen as "
+                      "1/mu^2 and the fp32 solver's error grows with them (3e-4 at mu = 0.1, 2.6e-3 at 0.05, "
+                      "measured for pairs)");
+      }
     }
   std::vector<float> dev((size_t)w*pad, 0.f);
   for (int e = 0; e < n; e++)
@@ -1570,7 +1599,7 @@ int fb_set_env_param(FbHandle *h, int field, const double *values) {
 
 int fb_get_env_param(FbHandle *h, int field, double *out) {
   if (!h || !out) return fail("null argument");
-  if (field < FB_ENV_JNT_STIFFNESS || field > FB_ENV_WATER_VELOCITY) return fail("fb_get_env_param: unknown field " + std::to_string(field));
+  if (field < 0 || field >= FB_N_ENV_PARAM) return fail("fb_get_env_param: unknown field " + std::to_string(field));
   const int n = h->P.n_envs, w = env_param_width(h, field);
   if (h->ep_dev[field]) {
     std::copy(h->ep_host[field].begin(), h->ep_host[field].end(), out);

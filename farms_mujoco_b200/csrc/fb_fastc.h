@@ -68,7 +68,8 @@ static double *fb_emu_stats = 0;
  * another order than on one warp: results agree with the single-warp kernel to rounding, not bit
  * for bit. */
 #define FB_RED_MAX 8       /* values of one cross-warp reduction */
-/* ENVP: as in FbFast (per-environment stiffness, damping, drag coefficients, water velocity). */
+/* ENVP: as in FbFast (per-environment stiffness, damping, drag coefficients, water velocity), and the
+ * candidates' friction from the FB_ENV_CAND_FRICTION table where it is set (cand_mu). */
 template <int BLK, int LEAN = 0, int SPLIT = 0, int ENVP = 0> struct FbFastCon : FbFast<BLK, 0, LEAN, SPLIT, ENVP> {
   typedef FbFast<BLK, 0, LEAN, SPLIT, ENVP> Base;
   using Base::P; using Base::m; using Base::rec; using Base::s; using Base::env; using Base::gs;
@@ -144,6 +145,18 @@ FB_UNROLL
     hm[0] = hm[1] = hany[0] = hany[1] = 0ull;
     lany[0] = lany[1] = 0u;
     own = ~0ull; nroles = 1; red_par = 0; sred = 0; hmul = 1u;
+  }
+
+  /* sliding friction of a candidate: ENVP, this environment's where FB_ENV_CAND_FRICTION is set (a
+   * uniform null test; the table is indexed by the model's candidate id cid, not the slot).  One load
+   * per use site, no copy in the candidate's scratch: so the twins compile without spills, as the
+   * kernels without ENVP do. */
+  FB_MEM float cand_mu(const CandRec &cr_) const {
+    if constexpr (ENVP) {
+      const float *fr = this->ept->fric;
+      if (fr) return fr[(size_t)cr_.cid*P.env_pad + env];
+    }
+    return cr_.mu;
   }
 
   FB_MEM int lane_on(int fc) const { return fb_bit128(hm, fc); }
@@ -307,7 +320,7 @@ FB_UNROLL
         f[3] -= dt*f[0]; f[4] -= dt*f[1]; f[5] -= dt*f[2];
         v_normalize3(f + 3);
         v_cross(f, f + 3, f + 6);
-        const float mu = cr_.mu;
+        const float mu = cand_mu(cr_);
         const int c = cr_.cid;
         float sr[2] = {MF(cand_solref, 2*c), MF(cand_solref, 2*c + 1)}, si5[5];
         for (int k = 0; k < 5; k++) si5[k] = MF(cand_solimp, 5*c + k);
@@ -352,7 +365,7 @@ FB_UNROLL
     v_cross(al, r, cr);
 FB_UNROLL
     for (int k = 0; k < 3; k++) pa[k] = al[3 + k] + cr[k];
-    const float mu = cr_.mu;
+    const float mu = cand_mu(cr_);
     out[0] = n[0]*pa[0] + n[1]*pa[1] + n[2]*pa[2];
     out[1] = mu*(t1[0]*pa[0] + t1[1]*pa[1] + t1[2]*pa[2]);
     out[2] = mu*(t2[0]*pa[0] + t2[1]*pa[1] + t2[2]*pa[2]);
@@ -542,7 +555,7 @@ FB_UNROLL
 FB_UNROLL
         for (int k = 0; k < 3; k++) { t1[k] = fb_ld_scr(pc + (NC_T1 + k)*BLK); r[k] = fb_ld_scr(pc + (NC_R + k)*BLK); }
         v_cross(n, t1, t2);
-        const float mu = cr_.mu;
+        const float mu = cand_mu(cr_);
         ArtInertia Kc;
         float p6[6] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
 FB_UNROLL
@@ -1016,7 +1029,7 @@ FB_UNROLL
     CandIter it = cand_begin();
     for (int fc = cand_next(it); fc >= 0; fc = cand_next(it)) {
       float *pc = ncand(fc);
-      const float mu = crec[fc].mu;
+      const float mu = cand_mu(crec[fc]);
       float v[7];
 FB_UNROLL
       for (int k = 0; k < 7; k++) v[k] = fb_ld_scr(pc + (NC_D + k)*BLK);     /* D, res[3], jp[3] */
@@ -1169,7 +1182,7 @@ FB_UNROLL
 FB_UNROLL
       for (int k = 0; k < 3; k++) t1[k] = fb_ld_scr(pc + (NC_T1 + k)*BLK);
       v_cross(n, t1, t2);
-      const float mu = cr_.mu;
+      const float mu = cand_mu(cr_);
       const float rn = fb_ld_scr(pc + NC_RES*BLK), r1 = fb_ld_scr(pc + (NC_RES + 1)*BLK), r2 = fb_ld_scr(pc + (NC_RES + 2)*BLK);
       float f4[4];
 FB_UNROLL

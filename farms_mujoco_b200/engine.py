@@ -16,7 +16,7 @@ import numpy as np
 from . import cabi
 from .data import AnimatData
 from .layout import sc
-from .mjcf_subset import parse_mjcf
+from .mjcf_subset import PAIR_MIN_FRICTION, candidate_friction, parse_mjcf
 from .simulation.physics import FarmsTables, get_sensor_maps, get_physics2data_maps
 from .units import SimulationUnitScaling
 
@@ -209,6 +209,7 @@ class BatchedPhysics:
                                        ct.byref(handle)))
         self._handle = handle
         self._cpg_n_osc = 0
+        self._geom_friction = None      # set_env_params(geom_friction=...) as last set
         self._log = cabi.FbLogView()
         self._state = cabi.FbStateView()
         self._derived = cabi.FbDerivedView()
@@ -394,19 +395,24 @@ class BatchedPhysics:
     def set_swimming(self, drag, buoyancy):
         self._check(self.lib.fb_set_swimming(self._handle, int(bool(drag)), int(bool(buoyancy))))
 
-    # fb_set_env_param fields (include/farms_b200.h FB_ENV_*): keyword -> (field, shape of one environment)
+    # fb_set_env_param fields (include/farms_b200.h FB_ENV_*): keyword -> (field, shape of one environment).
+    # geom_friction is given per geom and set per collision candidate (FB_ENV_CAND_FRICTION).
     def _env_param_fields(self):
         n_swim = len(self.tables.swim_links_index)
         return {'jnt_stiffness': (0, (self.model.njnt,)), 'dof_damping': (1, (self.model.nv,)),
-                'drag_coefficients': (2, (n_swim, 2, 3)), 'water_velocity': (3, (3,))}
+                'drag_coefficients': (2, (n_swim, 2, 3)), 'water_velocity': (3, (3,)),
+                'geom_friction': (4, (self.model.ngeom,))}
 
     def set_env_params(self, **fields):
         """Per-environment physical parameters (fb_set_env_param): ``jnt_stiffness [n_envs, njnt]``,
         ``dof_damping [n_envs, nv]``, ``drag_coefficients [n_envs, n_swim, 2, 3]`` (the layout of
-        ``FarmsTables.swim_coefficients``) and ``water_velocity [n_envs, 3]``.  Environment ``e`` then
-        steps as the model edited to its values.  Only the keywords passed change; ``None`` returns a
-        field to the model's value; an array without the environment axis is broadcast to every
-        environment.  The tables survive ``reset``."""
+        ``FarmsTables.swim_coefficients``), ``water_velocity [n_envs, 3]`` and ``geom_friction [n_envs,
+        ngeom]`` (the sliding friction ``model.geom_friction[:, 0]``; each collision candidate gets the
+        two geoms' values mixed as the compiler mixes them, ``mjcf_subset.candidate_friction``, and
+        explicit ``<pair>`` candidates keep the pair's friction).  Environment ``e`` then steps as the
+        model edited to its values.  Only the keywords passed change; ``None`` returns a field to the
+        model's value; an array without the environment axis is broadcast to every environment.  The
+        tables survive ``reset``."""
         known = self._env_param_fields()
         for name in fields:
             if name not in known:
@@ -415,6 +421,8 @@ class BatchedPhysics:
             field, shape = known[name]
             if values is None:
                 self._check(self.lib.fb_set_env_param(self._handle, field, None))
+                if name == 'geom_friction':
+                    self._geom_friction = None
                 continue
             arr = np.asarray(values, dtype=np.float64)
             if arr.shape != (self.n_envs,) + shape:
@@ -424,13 +432,43 @@ class BatchedPhysics:
                     raise ValueError(f'set_env_params: {name} must be {list(shape)} or '
                                      f'{[self.n_envs] + list(shape)}, got {list(arr.shape)}') from None
             arr = np.ascontiguousarray(arr)
+            if name == 'geom_friction':
+                self._set_geom_friction(arr)
+                continue
             self._check(self.lib.fb_set_env_param(self._handle, field, arr.ctypes.data_as(cabi.c_double_p)))
 
+    def _set_geom_friction(self, geom_friction):
+        """FB_ENV_CAND_FRICTION from per-geom sliding frictions [n_envs, ngeom]."""
+        bad = np.argwhere(~(np.isfinite(geom_friction) & (geom_friction >= 0.0)))
+        if len(bad):
+            e, g = bad[0]
+            raise ValueError(f'set_env_params: geom_friction of environment {e}, geom {g} '
+                             f'("{self.model.geom_names[g]}") is {float(geom_friction[e, g])!r}: '
+                             'a friction must be finite and non-negative')
+        cand = np.ascontiguousarray(candidate_friction(self.model, geom_friction))
+        try:
+            self._check(self.lib.fb_set_env_param(self._handle, 4, cand.ctypes.data_as(cabi.c_double_p)))
+        except EngineError as err:
+            pair = np.isin(self.model.cand_end, (20, 21))
+            low = np.argwhere((cand < PAIR_MIN_FRICTION) & ~pair)
+            if not len(low):
+                raise
+            e, c = low[0]
+            g1, g2 = (self.model.geom_names[g[c]] for g in (self.model.cand_geom1, self.model.cand_geom2))
+            raise EngineError(f'set_env_params: geom_friction of environment {e} mixes to {cand[e, c]:g} on '
+                              f'candidate {c}, geoms "{g1}" and "{g2}" (the larger of the two, or the '
+                              f'higher-priority one, is what counts): {err}') from None
+        self._geom_friction = geom_friction.copy()
+
     def env_params(self):
-        """The four fields of ``set_env_params`` as float64 ``[n_envs, ...]`` arrays (the model's value
+        """The fields of ``set_env_params`` as float64 ``[n_envs, ...]`` arrays (the model's value
         broadcast for a field that is not set)."""
         out = {}
         for name, (field, shape) in self._env_param_fields().items():
+            if name == 'geom_friction':
+                out[name] = (self._geom_friction.copy() if self._geom_friction is not None else
+                             np.tile(np.asarray(self.model.geom_friction, dtype=np.float64)[:, 0], (self.n_envs, 1)))
+                continue
             arr = np.zeros((self.n_envs,) + shape, dtype=np.float64)
             if arr.size:
                 self._check(self.lib.fb_get_env_param(self._handle, field, arr.ctypes.data_as(cabi.c_double_p)))

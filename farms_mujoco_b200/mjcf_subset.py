@@ -799,14 +799,21 @@ def parse_mjcf(xml_text: str, frictionless_pairs: str = 'refuse') -> Model:
 # Compile-time numerics
 # --------------------------------------------------------------------------
 
+def _mix_friction(priority1, priority2, friction1, friction2):
+    """mj_contactParam's friction of a geom pair: the higher-priority geom's, else the larger of the
+    two, floored at MJ_MINMU, element-wise (arrays broadcast).  The one copy of the rule: the compiler
+    (_mix_contact_params) and the per-environment tables (candidate_friction) both call it."""
+    return np.maximum(MJ_MINMU, np.where(priority1 > priority2, friction1,
+                                         np.where(priority2 > priority1, friction2, np.maximum(friction1, friction2))))
+
+
 def _mix_contact_params(model, g1, g2):
     """mj_contactParam for equal priorities (SURVEY.md Appendix A.6)."""
     p1, p2 = model.geom_priority[g1], model.geom_priority[g2]
+    friction = _mix_friction(p1, p2, model.geom_friction[g1], model.geom_friction[g2])
     if p1 != p2:
         g = g1 if p1 > p2 else g2
-        return (model.geom_friction[g].copy(), model.geom_solref[g].copy(),
-                model.geom_solimp[g].copy())
-    friction = np.maximum(model.geom_friction[g1], model.geom_friction[g2])
+        return friction, model.geom_solref[g].copy(), model.geom_solimp[g].copy()
     m1, m2 = model.geom_solmix[g1], model.geom_solmix[g2]
     if m1 >= MJ_MINVAL and m2 >= MJ_MINVAL:
         mix = m1/(m1 + m2)
@@ -924,7 +931,7 @@ def _compile_collision_candidates(model, pairs=(), frictionless_pairs='refuse'):
             ends = {GEOM_SPHERE: [0], GEOM_CAPSULE: [1, -1], GEOM_BOX: list(range(2, 10)), GEOM_ELLIPSOID: [10],
                     GEOM_CYLINDER: [11, 12, 13, 14]}[int(model.geom_type[g2])]
             for end in ends:
-                cands.append((g1, g2, end, max(MJ_MINMU, friction[0]), solref, solimp, margin, gap))
+                cands.append((g1, g2, end, float(friction[0]), solref, solimp, margin, gap))
     # explicit pairs come last (MuJoCo's broad phase lists them ahead of the filtered ones; the
     # order of the contacts does not enter the solution, only the order of the rows)
     cands += _compile_pair_candidates(model, pairs, frictionless_pairs)
@@ -937,6 +944,20 @@ def _compile_collision_candidates(model, pairs=(), frictionless_pairs='refuse'):
     model.cand_solimp = np.array([c[5] for c in cands], dtype=float).reshape(n, 5)
     model.cand_margin = np.array([c[6] for c in cands], dtype=float)
     model.cand_gap = np.array([c[7] for c in cands], dtype=float)
+
+
+def candidate_friction(model, geom_friction):
+    """The mixed sliding friction of every collision candidate, ``[..., ncand]``, for the sliding
+    frictions ``geom_friction [..., ngeom]`` (``model.geom_friction[:, 0]`` edited): what
+    ``parse_mjcf`` compiles into ``cand_friction`` for a model with those frictions -- the
+    candidate's two geoms mixed by priority or max, floored at ``MJ_MINMU``.  Explicit ``<pair>``
+    candidates (kinds 20 and 21) keep the model's value: a pair takes its friction from the pair
+    element."""
+    geom_friction = np.asarray(geom_friction, dtype=np.float64)
+    g1, g2 = model.cand_geom1, model.cand_geom2
+    mixed = _mix_friction(model.geom_priority[g1], model.geom_priority[g2], geom_friction[..., g1], geom_friction[..., g2])
+    pair = (model.cand_end == 20) | (model.cand_end == 21)
+    return np.where(pair, model.cand_friction, mixed)
 
 
 def soft_pair_model(model):

@@ -4,14 +4,20 @@ Alternates, round after round in one process, device-timed windows of
   swim/none    65,536 SALAMANDERs in water, 16 steps a launch (bench.py's headline configuration)
   swim/drag    the same with per-environment drag coefficients
   swim/all     the same with all four fields (stiffness, damping, drag coefficients, water velocity)
+  swim/friction  the headline batch with per-environment contact friction (the swimming path does
+               not read it: the unconstrained kernels keep their entry points)
   ground/none  4,096 SALAMANDERs on the ground (every step constrained)
   ground/sd    the same with per-environment stiffness and damping
-so that every configuration sees the same machine state; the tables of one engine are set and
-cleared between its windows.  Prints one JSON object (median / min / max env-steps/s of each
+  ground/friction  the same with per-environment contact friction
+  ground/all   friction, stiffness and damping
+  centipede/none, centipede/friction  8,192 CENTIPEDEs on the ground, without and with friction
+so that every configuration sees the same machine state (the CENTIPEDE pair alternates in a group of
+its own, after the SALAMANDER engines are closed); the tables of one engine are set and cleared
+between its windows.  Prints one JSON object (median / min / max env-steps/s of each
 configuration, the cost against its table-free run, the card and its power limit) and writes it to
 --out when given.
 
-    python tools/env_params_bench.py --rounds 5 --launches 30 --out profiles/r6_env_params_bench.json
+    python tools/env_params_bench.py --rounds 5 --launches 30 --out profiles/r7_env_friction_bench.json
 """
 
 import argparse
@@ -55,7 +61,14 @@ def table_values(model, tables, n_envs, fields, seed=11):
         out['drag_coefficients'] = base*rng.uniform(0.5, 2.0, size=(n_envs, n_swim, 2, 3))
     if 'water_velocity' in fields:
         out['water_velocity'] = rng.uniform(-0.05, 0.05, size=(n_envs, 3))
+    if 'geom_friction' in fields:
+        out['geom_friction'] = rng.uniform(0.5, 1.5, size=(n_envs, model.ngeom))
     return out
+
+
+def table_width(model, field, values):
+    """Device table entries per environment: one per collision candidate for the friction."""
+    return model.ncand if field == 'geom_friction' else int(np.prod(values.shape[1:]))
 
 
 def engine(name, n_envs, ring):
@@ -97,53 +110,67 @@ def main():
     ap.add_argument('--ring', type=int, default=64)
     ap.add_argument('--swim-envs', type=int, default=65536)
     ap.add_argument('--ground-envs', type=int, default=4096)
+    ap.add_argument('--centipede-envs', type=int, default=8192)
     ap.add_argument('--out', default=None)
     args = ap.parse_args()
     import torch
     if not torch.cuda.is_available():
         raise SystemExit('env_params_bench.py: no CUDA device')
-    all_fields = ('jnt_stiffness', 'dof_damping', 'drag_coefficients', 'water_velocity')
-    configs = [('swim', 'none', ()), ('swim', 'drag', ('drag_coefficients',)), ('swim', 'all', all_fields),
-               ('ground', 'none', ()), ('ground', 'sd', ('jnt_stiffness', 'dof_damping'))]
-    engines = {'swim': engine('salamander_swim', args.swim_envs, args.ring),
-               'ground': engine('salamander', args.ground_envs, args.ring)}
-    streams, tables = {}, {}
-    for key, (physics, model, _) in engines.items():
-        ptr = ctypes.c_void_p()
-        physics._check(physics.lib.fb_device_ptr_stream(physics._handle, ctypes.byref(ptr)))  # pylint: disable=protected-access
-        streams[key] = torch.cuda.ExternalStream(ptr.value, device=0)
-        tables[key] = table_values(model, physics.tables, physics.n_envs, all_fields)
-    rates = {f'{e}/{c}': [] for e, c, _ in configs}
-    for _ in range(args.rounds):
-        for eng, cfg, fields in configs:
-            physics, _, (qpos0, qvel0) = engines[eng]
-            physics.set_env_params(**{f: (tables[eng][f] if f in fields else None) for f in all_fields})
-            physics.reset(qpos0, qvel0)
-            rates[f'{eng}/{cfg}'].append(timed(physics, streams[eng], args.inner, args.launches, args.warmup))
-            assert not physics.flags.any(), f'{eng}/{cfg}: flags set'
+    all_fields = ('jnt_stiffness', 'dof_damping', 'drag_coefficients', 'water_velocity', 'geom_friction')
+    # Two groups, each alternated round after round: the SALAMANDER engines, then the CENTIPEDE
+    # engine once they are closed.  A kernel's shared-memory limit is an attribute of the function,
+    # which every engine of the process shares, and a SALAMANDER engine's block-size review sets it
+    # for its smaller model: the CENTIPEDE's launches need the engines of the other model gone.
+    groups = [
+        ({'swim': ('salamander_swim', args.swim_envs), 'ground': ('salamander', args.ground_envs)},
+         [('swim', 'none', ()), ('swim', 'drag', ('drag_coefficients',)),
+          ('swim', 'all', all_fields[:4]), ('swim', 'friction', ('geom_friction',)),
+          ('ground', 'none', ()), ('ground', 'sd', ('jnt_stiffness', 'dof_damping')),
+          ('ground', 'friction', ('geom_friction',)),
+          ('ground', 'all', ('geom_friction', 'jnt_stiffness', 'dof_damping'))]),
+        ({'centipede': ('centipede', args.centipede_envs)},
+         [('centipede', 'none', ()), ('centipede', 'friction', ('geom_friction',))]),
+    ]
     out = {'card': card(), 'rounds': args.rounds, 'launches_per_window': args.launches,
            'physics_steps_per_launch': args.inner, 'ring': args.ring, 'unit': 'env-steps/s', 'configs': {}}
-    for eng, cfg, fields in configs:
-        r = np.array(rates[f'{eng}/{cfg}'])
-        base = np.median(rates[f'{eng}/none'])
-        physics = engines[eng][0]
-        table_bytes = 4*sum(int(np.prod(tables[eng][f].shape[1:])) for f in fields)*physics.log_view.env_pad
-        out['configs'][f'{eng}/{cfg}'] = {
-            'n_envs': physics.n_envs, 'fields': list(fields), 'median': float(np.median(r)), 'min': float(r.min()),
-            'max': float(r.max()), 'runs': [float(x) for x in r],
-            'cost_vs_none_percent': float(100.0*(1.0 - np.median(r)/base)),
-            'table_bytes': int(table_bytes),
-            'table_bytes_per_env_step': 4*sum(int(np.prod(tables[eng][f].shape[1:])) for f in fields),
-            'log_bytes_per_env_step': physics.log_bytes_per_env_step,
-        }
+    for specs, configs in groups:
+        engines = {key: engine(name, n, args.ring) for key, (name, n) in specs.items()}
+        streams, tables = {}, {}
+        for key, (physics, model, _) in engines.items():
+            ptr = ctypes.c_void_p()
+            physics._check(physics.lib.fb_device_ptr_stream(physics._handle, ctypes.byref(ptr)))  # pylint: disable=protected-access
+            streams[key] = torch.cuda.ExternalStream(ptr.value, device=0)
+            tables[key] = table_values(model, physics.tables, physics.n_envs, all_fields)
+        rates = {f'{e}/{c}': [] for e, c, _ in configs}
+        for _ in range(args.rounds):
+            for eng, cfg, fields in configs:
+                physics, _, (qpos0, qvel0) = engines[eng]
+                physics.set_env_params(**{f: (tables[eng][f] if f in fields else None) for f in all_fields})
+                physics.reset(qpos0, qvel0)
+                rates[f'{eng}/{cfg}'].append(timed(physics, streams[eng], args.inner, args.launches, args.warmup))
+                assert not physics.flags.any(), f'{eng}/{cfg}: flags set'
+        for eng, cfg, fields in configs:
+            r = np.array(rates[f'{eng}/{cfg}'])
+            base = np.median(rates[f'{eng}/none'])
+            physics = engines[eng][0]
+            width = sum(table_width(physics.model, f, tables[eng][f]) for f in fields)
+            table_bytes = 4*width*physics.log_view.env_pad
+            out['configs'][f'{eng}/{cfg}'] = {
+                'n_envs': physics.n_envs, 'fields': list(fields), 'median': float(np.median(r)), 'min': float(r.min()),
+                'max': float(r.max()), 'runs': [float(x) for x in r],
+                'cost_vs_none_percent': float(100.0*(1.0 - np.median(r)/base)),
+                'table_bytes': int(table_bytes),
+                'table_bytes_per_env_step': 4*width,
+                'log_bytes_per_env_step': physics.log_bytes_per_env_step,
+            }
+        for physics, _, _ in engines.values():
+            physics.close()
     text = json.dumps(out, indent=1)
     print(text)
     if args.out:
         os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
         with open(args.out, 'w') as f:
             f.write(text + '\n')
-    for physics, _, _ in engines.values():
-        physics.close()
 
 
 if __name__ == '__main__':
