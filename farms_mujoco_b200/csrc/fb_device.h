@@ -1742,7 +1742,7 @@ enum { FB_MODE_STEP = 0, FB_MODE_RESET = 1 };
 struct FbParams {
   DevModel m;
   int n_envs, n_steps, ring, mode, want_derived;
-  long long it0;                  /* physics steps taken since reset */
+  long long it0;                  /* batch iteration: physics steps taken since fb_reset */
   float *qpos, *qvel, *ctrl, *xfrc_applied, *qpos_spring, *env_phase;
   int *flags;
   long long *iteration;
@@ -1790,10 +1790,14 @@ struct FbParams {
  * A launch argument of its own (not a member of FbParams), so that the parameter blocks of the
  * kernels that do not read it keep their layout: the team kernel tests the pointers at run time,
  * the per-thread kernels read them in their ENVP twins only (the unconstrained twins never read
- * `fric`: the member is last, so the members they read keep their offsets). */
+ * `fric`: the member is last, so the members they read keep their offsets).
+ * episode_start [n_envs] (fb_reset_envs): batch iteration of each environment's episode row 0; the
+ * travelling-wave controller reads the episode's time (it0 + k - episode_start).  Bound only while
+ * the wave controller is on and some episode began after iteration 0; NULL: it0 + k. */
 struct FbEnvTables {
   const float *stiffness, *damping, *coef, *wvel;
   const float *fric;
+  const long long *episode_start;
 };
 
 #define FB_NEVER_DIRTY (-(1LL << 60))
@@ -1834,7 +1838,8 @@ FB_DEV EnvPtrs fb_env_ptrs(const FbParams &P, const FbEnvTables &T, int env) {
   return g;
 }
 
-/* Reset: forward at the loaded state, log row 0.  Step k of a launch: control,
+/* Reset: forward at the loaded state, log row it0 % ring (0 after fb_reset; the episode's row 0 of
+ * an environment fb_reset_envs restarts at it0).  Step k of a launch: control,
  * forward (derived quantities of the pre-step state), Euler, log row
  * (it0+k+1) % ring = {derived of the pre-step state, qpos/qvel of the new
  * state} (SURVEY.md Appendix D-1), then the drag wrench for the next step. */
@@ -1851,7 +1856,7 @@ FB_DEV void fb_run_env(const FbParams &P, const FbEnvTables &T, int env, int k0,
     long long row;
     if (P.mode == FB_MODE_RESET) {
       st.forward(1);
-      row = 0;
+      row = P.it0 % P.ring;
     } else {
       if (P.ctrl_seq) {
         const float *seqk = P.ctrl_seq + ((size_t)(P.seq_pos + k)*P.seq_stride)*P.env_pad + e;
@@ -1859,7 +1864,7 @@ FB_DEV void fb_run_env(const FbParams &P, const FbEnvTables &T, int env, int k0,
         for (int i = lane; i < P.n_spring; i += TEAM) st.g.qpos_spring[P.spring_qadr[i]] = seqk[(long long)(m.nu + i)*P.env_pad];
         st.seq_control(seqk, P.env_pad);
       }
-      if (m.n_wc > 0) st.wave_control((float)(P.it0 + k)*m.timestep);
+      if (m.n_wc > 0) st.wave_control((float)(P.it0 + k - (T.episode_start ? T.episode_start[e] : 0))*m.timestep);
       int wd = P.want_derived && k == n - 1;
       st.forward(wd);
       if (wd) st.write_derived();
@@ -1875,8 +1880,8 @@ FB_DEV void fb_run_env(const FbParams &P, const FbEnvTables &T, int env, int k0,
   }
   st.store_state(P.ctrl_seq != 0 && P.mode != FB_MODE_RESET);
   if (lane == 0) {
-    P.iteration[env] = P.mode == FB_MODE_RESET ? 0 : P.it0 + P.n_steps;
-    if (k0 < n) P.con_dirty[env] = P.mode == FB_MODE_RESET ? 0 : P.it0 + P.n_steps;   /* full rows, constraint columns included */
+    P.iteration[env] = P.mode == FB_MODE_RESET ? P.it0 : P.it0 + P.n_steps;
+    if (k0 < n) P.con_dirty[env] = P.mode == FB_MODE_RESET ? P.it0 : P.it0 + P.n_steps;   /* full rows, constraint columns included */
   }
 }
 

@@ -64,11 +64,44 @@ static int dev_sync(fbStream st) { return cudaStreamSynchronize(st) == cudaSucce
 static const char *dev_error() { return cudaGetErrorString(cudaGetLastError()); }
 #endif
 
+/* fb_reset_envs: what a restart writes besides the reset's forward pass (the team kernel's) */
+struct FbResetArgs {
+  const uint8_t *mask;             /* [n_envs] non-zero: restart */
+  const float *qpos0, *qvel0;      /* given rows ([row][nq] / [row][nv]) or NULL: the keyframe */
+  const int *row_of;               /* [n_envs] row of qpos0 / qvel0 of a restarted environment; NULL: env */
+  const float *key_qpos, *key_qvel;
+  float *qpos, *qvel, *ctrl, *xfrc_applied;
+  int *flags;
+  long long *episode_start;
+  float *theta, *r, *rd;           /* on-device CPG state [n_osc][env_pad] (n_osc = 0: no CPG) */
+  const float *theta0, *r0;        /* ... as fb_set_cpg_state last set it */
+  int n_envs, nq, nv, nu, nbody, n_osc;
+  long long env_pad, it;
+};
+
+/* one environment: its state rows as fb_reset writes them, its CPG rows, its episode start */
+FB_DEV void fb_reset_env(const FbResetArgs &A, int env) {
+  if (!A.mask[env]) return;
+  const size_t e = (size_t)env, row = A.row_of ? (size_t)A.row_of[env] : e;
+  for (int i = 0; i < A.nq; i++) A.qpos[e*A.nq + i] = A.qpos0 ? A.qpos0[row*A.nq + i] : A.key_qpos[i];
+  for (int i = 0; i < A.nv; i++) A.qvel[e*A.nv + i] = A.qvel0 ? A.qvel0[row*A.nv + i] : A.key_qvel[i];
+  const int nu = A.nu > 0 ? A.nu : 1;
+  for (int i = 0; i < nu; i++) A.ctrl[e*nu + i] = 0.f;
+  for (int i = 0; i < 6*A.nbody; i++) A.xfrc_applied[e*6*A.nbody + i] = 0.f;
+  A.flags[env] = 0;
+  for (int o = 0; o < A.n_osc; o++) {
+    const size_t k = (size_t)o*A.env_pad + e;
+    A.theta[k] = A.theta0[k]; A.r[k] = A.r0[k]; A.rd[k] = 0.f;
+  }
+  A.episode_start[env] = A.it;
+}
+
 /* --------------------------------------------------------------- kernels */
 #ifndef FB_HOST_EMU
+/* only: FB_MODE_RESET of fb_reset_envs, the environments to restart ([n_envs], non-zero); NULL: all */
 template <int TEAM>
 __global__ void __launch_bounds__(128)
-fb_step_kernel(const __grid_constant__ FbParams P, const __grid_constant__ FbEnvTables T) {
+fb_step_kernel(const __grid_constant__ FbParams P, const __grid_constant__ FbEnvTables T, const uint8_t *only) {
   extern __shared__ __align__(16) float fb_smem[];
   const DevModel &m = P.m;
   const int tid = threadIdx.x, team = tid/TEAM, lane = tid % TEAM;
@@ -78,7 +111,7 @@ fb_step_kernel(const __grid_constant__ FbParams P, const __grid_constant__ FbEnv
     if (env >= P.pending_count[P.parity]) return;
     env = P.pending[env];
     k0 = P.steps_done[env];
-  } else if (env >= P.n_envs) {
+  } else if (env >= P.n_envs || (only && !only[env])) {
     return;
   }
   const int base = (tid & 31)/TEAM*TEAM;
@@ -98,9 +131,10 @@ struct FbFastParams {
 /* BLK environments per warp (32, or 16 in a half-filled warp).  MULTI: blocks of 2..8 warps
  * (blockDim.x/32) kept in step by a barrier per physics step (FbFast::run_t). */
 /* Every per-thread entry point has an ENVP twin (fb_*_envp_kernel, same template arguments) that reads
- * the per-environment parameter tables of fb_set_env_param; launch() takes the twin while a table the
- * kernel reads is set: any table for the constrained kernels, any but the candidate friction for the
- * unconstrained ones (they have no contacts).  An entry point and its twin expand the same body
+ * the per-environment parameter tables of fb_set_env_param and runs the episode clock of
+ * fb_reset_envs; launch() takes the twin while a table the kernel reads is set: any table for the
+ * constrained kernels, any but the candidate friction for the unconstrained ones (they have no
+ * contacts), and while the episode clock is bound.  An entry point and its twin expand the same body
  * (FB_*_BODY: ENVP is a template argument
  * of FbFast / FbFastCon, T the tables); written out in each kernel rather than called as an inlined
  * function, which ptxas was found to schedule differently.  A twin's parameters are the entry
@@ -376,6 +410,18 @@ __global__ void __launch_bounds__(128) fb_cpg_kernel(CpgDev c, int n_envs, long 
   if (env < n_envs) fb_cpg_env(c, env, env_pad, n_steps, nu, dt, ctrl, seq);
 }
 
+/* fb_reset_envs_where: one thread per environment */
+__global__ void __launch_bounds__(128) fb_reset_envs_kernel(const FbResetArgs A) {
+  const int env = blockIdx.x*blockDim.x + threadIdx.x;
+  if (env < A.n_envs) fb_reset_env(A, env);
+}
+
+/* fb_reset_envs: the host list envs[n] -> mask (zeroed before) and the row of each listed environment */
+__global__ void fb_reset_list_kernel(const int *__restrict__ envs, int n, uint8_t *mask, int *row_of) {
+  const int i = blockIdx.x*blockDim.x + threadIdx.x;
+  if (i < n) { mask[envs[i]] = 1; row_of[envs[i]] = i; }
+}
+
 /* the whole ring of one environment -> dense [ring][row_floats] */
 __global__ void fb_gather_env_kernel(const float *__restrict__ log, int ring, int row_floats, int vec,
                                      long long env_pad, int env, float *__restrict__ out) {
@@ -427,8 +473,15 @@ struct FbHandle {
   float *ep_dev[FB_N_ENV_PARAM];
   std::vector<double> ep_host[FB_N_ENV_PARAM];
   FbEnvTables ep;                   /* ep_dev as the kernels take it */
+  /* per-environment episodes (fb_reset_envs): device [n_envs] batch iteration of each episode's row 0,
+   * and whether one may be non-zero (a restart after iteration 0 since fb_reset) */
+  long long *episode_start;
+  bool episode_late;
+  uint8_t *reset_mask;              /* fb_reset_envs staging (allocated at the first call): the mask ... */
+  int *reset_list, *reset_row;      /* ... the uploaded list and each listed environment's row in it ... */
+  float *reset_q, *reset_v;         /* ... and the uploaded rows [n][nq] / [n][nv] */
   long long launches;
-  long long it;            /* physics steps since reset */
+  long long it;            /* batch iteration: physics steps since fb_reset */
   float last_ms;
   float *gather_links, *gather_joints;   /* fb_step_host staging */
   int joint_sel_n, joint_sel[32];        /* fb_set_host_joint_columns: columns of the joints row fb_step_host returns (0 = all) */
@@ -444,6 +497,7 @@ struct FbHandle {
   bool cpg_on;
   CpgDev cpg;
   std::vector<void *> cpg_allocs;
+  float *cpg_theta0, *cpg_r0;          /* the state fb_set_cpg_state last set ([n_osc][env_pad]), for fb_reset_envs */
   std::vector<int> spring_qadr_host;   /* qpos addresses of the CPG's spring-reference outputs */
   const int *cpg_spring_qadr;          /* the same on the device */
   /* wave-controller copies (owned) */
@@ -694,7 +748,8 @@ template <int ENVP, int CENVP> static void emu_per_thread(FbHandle *h, FbParams 
 }
 #endif
 
-static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
+/* only (FB_MODE_RESET): the environments fb_reset_envs restarts, at the current iteration; NULL: all */
+static int launch(FbHandle *h, int mode, int n_steps, int want_derived, const uint8_t *only = nullptr) {
   FbParams &P = h->P;
   P.mode = mode; P.n_steps = n_steps; P.want_derived = want_derived; P.it0 = h->it;
   /* The per-thread kernel advances every environment while it is unconstrained; the
@@ -723,9 +778,12 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
     if (h->seq_pos == h->seq_len) h->seq_len = h->seq_pos = 0;     /* consumed: ctrl is held again */
   }
   const int use_fast = h->fast_enabled && P.m.X.ok && mode == FB_MODE_STEP && !want_derived;
-  /* the per-thread kernels' ENVP twins while a per-environment parameter table they read is set: the
-   * unconstrained kernels never read the candidate friction */
-  const bool envp = h->ep.stiffness || h->ep.damping || h->ep.coef || h->ep.wvel;
+  /* the per-thread kernels' ENVP twins while a per-environment parameter table they read is set (the
+   * unconstrained kernels never read the candidate friction), or the episode clock is bound: only
+   * while the wave controller, the one step code that reads time, is on and some episode began
+   * after iteration 0 */
+  h->ep.episode_start = P.m.n_wc > 0 && h->episode_late ? h->episode_start : nullptr;
+  const bool envp = h->ep.stiffness || h->ep.damping || h->ep.coef || h->ep.wvel || h->ep.episode_start;
   const bool cenvp = envp || h->ep.fric;
   const int con_thread = use_fast && h->con_thread && P.m.X.con_ok;
   P.use_pending = use_fast;
@@ -743,6 +801,7 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
   const int count = use_fast ? (con_thread ? 0 : P.pending_count[P.parity]) : P.n_envs;
   for (int i = 0; i < count; i++) {
     int env = use_fast ? P.pending[i] : i;
+    if (only && !only[env]) continue;
     fb_run_env<1>(P, h->ep, env, use_fast ? P.steps_done[env] : 0, s.data(), si.data(), 0, 0, 1u);
   }
   h->last_ms = 0.f;
@@ -825,9 +884,9 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
     }
   }
   if (!con_thread) switch (h->team) {
-    case 8: fb_step_kernel<8><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep); break;
-    case 16: fb_step_kernel<16><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep); break;
-    default: fb_step_kernel<32><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep); break;
+    case 8: fb_step_kernel<8><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep, only); break;
+    case 16: fb_step_kernel<16><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep, only); break;
+    default: fb_step_kernel<32><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep, only); break;
   }
   cudaEventRecord(h->ev1, h->stream);
   {
@@ -836,7 +895,7 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived) {
   }
 #endif
   h->launches++;
-  if (mode == FB_MODE_RESET) h->it = 0; else h->it += n_steps;
+  if (mode == FB_MODE_STEP) h->it += n_steps;       /* fb_reset set it to 0 before, fb_reset_envs keeps it */
 #ifndef FB_HOST_EMU
   /* Half-filled warps (16 environments each) pay for candidate-rich models only through the
    * constrained step: a warp visits the union of its lanes' contacts.  Whether an episode is of
@@ -1066,7 +1125,9 @@ int fb_create(const FbModel *model, const FbFarms *farms, int n_envs, int device
   memset(&h->ep, 0, sizeof(h->ep));
   h->last_ms = 0.f; h->has_wc = false; h->gather_links = h->gather_joints = h->gather_env = nullptr;
   h->seq_dev = h->seq_stage = nullptr; h->seq_len = h->seq_pos = h->seq_cap = h->seq_rows = 0;
-  h->cpg_on = false; memset(&h->cpg, 0, sizeof(h->cpg));
+  h->cpg_on = false; memset(&h->cpg, 0, sizeof(h->cpg)); h->cpg_theta0 = h->cpg_r0 = nullptr;
+  h->episode_start = nullptr; h->episode_late = false;
+  h->reset_mask = nullptr; h->reset_list = h->reset_row = nullptr; h->reset_q = h->reset_v = nullptr;
   h->joint_sel_n = 0; h->link_sel_n = 0; h->link_items_n = 0; h->ctrl_sel_n = 0;
   h->export_stage[0] = h->export_stage[1] = nullptr; h->export_stage_floats = 0;
   h->fast_enabled = 1; h->fast_block = 1; h->fast_smem_bytes = 0; h->launch_parity = 0;
@@ -1213,6 +1274,7 @@ int fb_create(const FbModel *model, const FbFarms *farms, int n_envs, int device
   bad |= alloc_arr(h, &P.flags, n); bad |= alloc_arr(h, &P.iteration, n);
   bad |= alloc_arr(h, &P.pending, n); bad |= alloc_arr(h, &P.pending_count, 2); bad |= alloc_arr(h, &P.steps_done, n);
   bad |= alloc_arr(h, &P.con_dirty, n);
+  bad |= alloc_arr(h, &h->episode_start, n);
   bad |= alloc_arr(h, &h->con_split_done, (n + 15)/16);
   P.fast_scratch_stride = (long long)((n + 31) & ~(size_t)31);
   P.fast_scratch = nullptr;
@@ -1286,9 +1348,11 @@ int fb_reset(FbHandle *h, const double *qpos0, const double *qvel0) {
   bad |= dev_zero(P.ctrl, n*(m.nu > 0 ? m.nu : 1)*sizeof(float), h->stream);
   bad |= dev_zero(P.xfrc_applied, n*6*m.nbody*sizeof(float), h->stream);
   bad |= dev_zero(P.flags, n*sizeof(int), h->stream);
+  bad |= dev_zero(h->episode_start, n*sizeof(long long), h->stream);
   bad |= dev_sync(h->stream);   /* q, v are stack-owned */
   if (bad) return fail(std::string("fb_reset: ") + dev_error());
   h->it = 0;
+  h->episode_late = false;
   h->seq_len = h->seq_pos = 0;
 #ifndef FB_HOST_EMU
   if (h->fast_enabled && h->fast_block_auto) {
@@ -1298,6 +1362,93 @@ int fb_reset(FbHandle *h, const double *qpos0, const double *qvel0) {
 #endif
   if (launch(h, FB_MODE_RESET, 1, 1)) return -1;
   return dev_sync(h->stream) ? fail(std::string("fb_reset: ") + dev_error()) : 0;
+}
+
+/* fb_reset_envs / fb_reset_envs_where: the state rows, CPG rows and episode start of the masked
+ * environments, then the reset's forward pass for them alone (log row it % ring, derived view), all
+ * on the handle's stream and without a host synchronisation */
+static int reset_envs_enqueue(FbHandle *h, const uint8_t *mask, const int *row_of, const float *qpos0, const float *qvel0) {
+  FbParams &P = h->P;
+  const DevModel &m = h->hm.m;
+  FbResetArgs A;
+  A.mask = mask; A.qpos0 = qpos0; A.qvel0 = qvel0; A.row_of = row_of;
+  A.key_qpos = h->F_dev + m.o.key_qpos; A.key_qvel = h->F_dev + m.o.key_qvel;
+  A.qpos = P.qpos; A.qvel = P.qvel; A.ctrl = P.ctrl; A.xfrc_applied = P.xfrc_applied; A.flags = P.flags;
+  A.episode_start = h->episode_start;
+  A.n_osc = h->cpg_on ? h->cpg.n_osc : 0;
+  A.theta = h->cpg.theta; A.r = h->cpg.r; A.rd = h->cpg.rd; A.theta0 = h->cpg_theta0; A.r0 = h->cpg_r0;
+  A.n_envs = P.n_envs; A.nq = m.nq; A.nv = m.nv; A.nu = m.nu; A.nbody = m.nbody;
+  A.env_pad = P.env_pad; A.it = h->it;
+#ifdef FB_HOST_EMU
+  for (int env = 0; env < P.n_envs; env++) fb_reset_env(A, env);
+#else
+  fb_reset_envs_kernel<<<(P.n_envs + 127)/128, 128, 0, h->stream>>>(A);
+  h->launches++;
+#endif
+  if (h->it > 0) h->episode_late = true;
+  return launch(h, FB_MODE_RESET, 1, 1, mask);
+}
+
+int fb_reset_envs(FbHandle *h, int n, const int32_t *envs, const double *qpos0, const double *qvel0) {
+  if (!h) return fail("null handle");
+  if (n < 0 || (n > 0 && !envs)) return fail("fb_reset_envs: n must be >= 0, with envs[n]");
+  if (n == 0) return 0;
+  const DevModel &m = h->hm.m;
+  const int N = h->P.n_envs;
+  std::vector<int> seen((size_t)N, -1);
+  for (int i = 0; i < n; i++) {
+    const int e = envs[i];
+    if (e < 0 || e >= N)
+      return fail("fb_reset_envs: envs[" + std::to_string(i) + "] = " + std::to_string(e) + " is out of range [0, " +
+                  std::to_string(N) + ")");
+    if (seen[e] >= 0)
+      return fail("fb_reset_envs: environment " + std::to_string(e) + " is given twice (envs[" + std::to_string(seen[e]) +
+                  "] and envs[" + std::to_string(i) + "])");
+    seen[e] = i;
+  }
+  std::vector<float> q(qpos0 ? (size_t)n*m.nq : 0), v(qvel0 ? (size_t)n*m.nv : 0);
+  const struct { const double *src; std::vector<float> &dst; int w; const char *name; } rows[2] = {
+    {qpos0, q, m.nq, "qpos0"}, {qvel0, v, m.nv, "qvel0"}};
+  for (const auto &r : rows)
+    for (size_t k = 0; k < r.dst.size(); k++) {
+      if (!std::isfinite(r.src[k]))
+        return fail(std::string("fb_reset_envs: non-finite ") + r.name + " at row " + std::to_string(k/r.w) +
+                    " (environment " + std::to_string(envs[k/r.w]) + "), index " + std::to_string(k % r.w));
+      r.dst[k] = (float)r.src[k];
+    }
+  if (!h->reset_mask) {
+    int bad = alloc_arr(h, &h->reset_mask, (size_t)N);
+    bad |= alloc_arr(h, &h->reset_list, (size_t)N); bad |= alloc_arr(h, &h->reset_row, (size_t)N);
+    bad |= alloc_arr(h, &h->reset_q, (size_t)N*m.nq); bad |= alloc_arr(h, &h->reset_v, (size_t)N*m.nv);
+    if (bad) return fail("fb_reset_envs: device allocation failed");
+  }
+  int bad = dev_zero(h->reset_mask, (size_t)N, h->stream);
+  bad |= h2d(h->reset_list, envs, (size_t)n*sizeof(int32_t), h->stream);
+  if (qpos0) bad |= h2d(h->reset_q, q.data(), q.size()*sizeof(float), h->stream);
+  if (qvel0) bad |= h2d(h->reset_v, v.data(), v.size()*sizeof(float), h->stream);
+  if (bad) return fail(std::string("fb_reset_envs: ") + dev_error());
+#ifdef FB_HOST_EMU
+  for (int i = 0; i < n; i++) { h->reset_mask[envs[i]] = 1; h->reset_row[envs[i]] = i; }
+#else
+  fb_reset_list_kernel<<<(n + 127)/128, 128, 0, h->stream>>>(h->reset_list, n, h->reset_mask, h->reset_row);
+  h->launches++;
+#endif
+  if (reset_envs_enqueue(h, h->reset_mask, h->reset_row, qpos0 ? h->reset_q : nullptr, qvel0 ? h->reset_v : nullptr))
+    return -1;
+  return dev_sync(h->stream) ? fail(std::string("fb_reset_envs: ") + dev_error()) : 0;   /* q, v are stack-owned */
+}
+
+int fb_reset_envs_where(FbHandle *h, const uint8_t *mask, const float *qpos0, const float *qvel0) {
+  if (!h) return fail("null handle");
+  if (!mask) return fail("fb_reset_envs_where: null mask");
+  return reset_envs_enqueue(h, mask, nullptr, qpos0, qvel0);
+}
+
+int fb_get_episode_start(FbHandle *h, int64_t *out) {
+  if (!h || !out) return fail("null argument");
+  if (d2h(out, h->episode_start, (size_t)h->P.n_envs*sizeof(long long), h->stream) || dev_sync(h->stream))
+    return fail(std::string("fb_get_episode_start: ") + dev_error());
+  return 0;
 }
 
 static int upload_doubles(FbHandle *h, float *dst, const double *src, size_t count, const char *what) {
@@ -1367,6 +1518,7 @@ int fb_set_cpg(FbHandle *h, const FbCpgNetwork *net) {
   h->cpg_allocs.clear();
   h->cpg_on = false;
   memset(&h->cpg, 0, sizeof(h->cpg));
+  h->cpg_theta0 = h->cpg_r0 = nullptr;
   h->cpg_spring_qadr = nullptr;
   if (!h->spring_qadr_host.empty()) {
     h->spring_qadr_host.clear();
@@ -1399,11 +1551,13 @@ int fb_set_cpg(FbHandle *h, const FbCpgNetwork *net) {
   bad |= cpg_upload(h, net->out_gain, net->n_out, &c.o_gain);
   bad |= cpg_upload(h, net->out_offset, net->n_out, &c.o_off);
   const size_t st = (size_t)net->n_osc*h->P.env_pad;
-  void *pt = nullptr, *pr = nullptr, *pd = nullptr;
+  void *pt = nullptr, *pr = nullptr, *pd = nullptr, *pt0 = nullptr, *pr0 = nullptr;
   bad |= dev_alloc(&pt, st*sizeof(float)); bad |= dev_alloc(&pr, st*sizeof(float)); bad |= dev_alloc(&pd, st*sizeof(float));
+  bad |= dev_alloc(&pt0, st*sizeof(float)); bad |= dev_alloc(&pr0, st*sizeof(float));
   if (bad) return fail("fb_set_cpg: device allocation / upload failed");
-  h->cpg_allocs.push_back(pt); h->cpg_allocs.push_back(pr); h->cpg_allocs.push_back(pd);
+  for (void *p : {pt, pr, pd, pt0, pr0}) h->cpg_allocs.push_back(p);
   c.theta = static_cast<float *>(pt); c.r = static_cast<float *>(pr); c.rd = static_cast<float *>(pd);
+  h->cpg_theta0 = static_cast<float *>(pt0); h->cpg_r0 = static_cast<float *>(pr0);
   h->cpg_on = true;
   h->seq_len = h->seq_pos = 0;
   return 0;
@@ -1453,9 +1607,12 @@ int fb_set_cpg_state(FbHandle *h, const double *phase, const double *amplitude) 
       th[i*pad + e] = (float)phase[e*no + i];
       if (amplitude) r[i*pad + e] = (float)amplitude[e*no + i];
     }
+  /* the device copy in cpg_theta0 / cpg_r0 is what fb_reset_envs restores */
   if (h2d(h->cpg.theta, th.data(), th.size()*sizeof(float), h->stream) ||
       h2d(h->cpg.r, r.data(), r.size()*sizeof(float), h->stream) ||
-      h2d(h->cpg.rd, rd.data(), rd.size()*sizeof(float), h->stream) || dev_sync(h->stream))
+      h2d(h->cpg.rd, rd.data(), rd.size()*sizeof(float), h->stream) ||
+      h2d(h->cpg_theta0, th.data(), th.size()*sizeof(float), h->stream) ||
+      h2d(h->cpg_r0, r.data(), r.size()*sizeof(float), h->stream) || dev_sync(h->stream))
     return fail(std::string("fb_set_cpg_state: ") + dev_error());
   return 0;
 }
@@ -1697,6 +1854,12 @@ int fb_export_farms(FbHandle *h, int env, double *links, double *joints, double 
   const FbParams &P = h->P;
   if (env < 0 || env >= P.n_envs) return fail("fb_export_farms: env out of range");
   const DevModel &dm = h->hm.m;
+  /* the environment's current episode: exported row r is ring row (s + r) % ring; when s > 0, rows
+   * the episode has not reached (r > it - s) are zero */
+  long long s = 0;
+  if (d2h(&s, h->episode_start + env, sizeof(s), h->stream) || dev_sync(h->stream))
+    return fail(std::string("fb_export_farms: ") + dev_error());
+  const long long reached = h->it - s;
   struct Item { double *dst; const float *src; int row_floats, vec; } items[4] = {
     {links, P.log_links, dm.n_links*20, FB_VEC_LINKS},
     {joints, P.log_joints, dm.n_joints*dm.joint_cols, FB_VEC_JOINTS},
@@ -1718,7 +1881,11 @@ int fb_export_farms(FbHandle *h, int env, double *links, double *joints, double 
     if (d2h(tmp.data(), h->gather_env, count*sizeof(float), h->stream) || dev_sync(h->stream))
       return fail(std::string("fb_export_farms: ") + dev_error());
 #endif
-    for (size_t i = 0; i < count; i++) it.dst[i] = (double)tmp[i];
+    for (long long r = 0; r < P.ring; r++) {
+      double *dst = it.dst + (size_t)r*it.row_floats;
+      const float *src = tmp.data() + (size_t)((s + r) % P.ring)*it.row_floats;
+      for (int i = 0; i < it.row_floats; i++) dst[i] = s > 0 && r > reached ? 0.0 : (double)src[i];
+    }
   }
   return 0;
 }

@@ -215,13 +215,19 @@ template <int SYNC> FB_DEV void fb_block_sync() {
  * come from the per-environment tables (FbEnvTables, `ept`) where one is set (a uniform null test
  * per table), else from the records / the model as with ENVP = 0.  Same arithmetic on the values. */
 /* the tables' pointer is a member of the ENVP variants only: a member that the other variants never
- * read still changed how ptxas scheduled the SLIM kernels */
+ * read still changed how ptxas scheduled the SLIM kernels.  The ENVP variants also run the episode
+ * clock (fb_reset_envs): the wave controller's time is formed from episode_it(it0 + k), with the
+ * environment's episode start loaded once per launch (0 while FbEnvTables::episode_start is not
+ * bound, which gives the same value as it0 + k). */
 template <int ENVP> struct FbEnvRef {
   const FbEnvTables *ept;   /* the per-environment parameter tables (kernel parameters) */
-  FB_MEM FbEnvRef(const FbEnvTables *ept_) : ept(ept_) {}
+  long long ep0;            /* batch iteration of this environment's episode row 0 */
+  FB_MEM FbEnvRef(const FbEnvTables *ept_, int env) : ept(ept_), ep0(ept_->episode_start ? ept_->episode_start[env] : 0) {}
+  FB_MEM long long episode_it(long long it) const { return it - ep0; }
 };
 template <> struct FbEnvRef<0> {
-  FB_MEM FbEnvRef(const FbEnvTables *) {}
+  FB_MEM FbEnvRef(const FbEnvTables *, int) {}
+  FB_MEM long long episode_it(long long it) const { return it; }
 };
 template <int BLK, int SLIM = 0, int LEAN = 0, int SPLIT = 0, int ENVP = 0> struct FbFast : FbEnvRef<ENVP> {
   /* SLIM scratch block: W[6] U 1/d trq q qd V[6] tc tu -- the first 17 are one contiguous run */
@@ -258,7 +264,7 @@ template <int BLK, int SLIM = 0, int LEAN = 0, int SPLIT = 0, int ENVP = 0> stru
   int *sflag;
 
   FB_MEM FbFast(const FbParams &P_, const FastRec *rec_, float *s_, float *gs_, int env_, const FbEnvTables *ept_ = 0)
-      : FbEnvRef<ENVP>(ept_), P(P_), m(P_.m), rec(rec_), s(s_), env(env_), gs(gs_), cs(0), csc(0), crec(0) {
+      : FbEnvRef<ENVP>(ept_, env_), P(P_), m(P_.m), rec(rec_), s(s_), env(env_), gs(gs_), cs(0), csc(0), crec(0) {
     env_phase = P.env_phase[env];
     dirty_c = P.con_dirty[env];
     zfill = 1;
@@ -1260,7 +1266,7 @@ FB_UNROLL
       float *row_joints = fb_log_row(P.log_joints, row, m.n_joints*m.joint_cols, P.env_pad, FB_VEC_JOINTS, e);
       float *row_contacts = fb_log_row(P.log_contacts, row, m.n_contacts*12, P.env_pad, FB_VEC_CONTACTS, e);
       float *row_xfrc = fb_log_row(P.log_xfrc, row, m.n_xfrc*6, P.env_pad, FB_VEC_XFRC, e);
-      const float time = (float)(P.it0 + k)*m.timestep;
+      const float time = (float)this->episode_it(P.it0 + k)*m.timestep;
       zfill = log_row_dirty(P.it0 + k + 1);
       fb_block_sync<SYNC>();
       if (!dead && pass_poses(row_links)) { kdone = k; dead = 1; }
@@ -1301,7 +1307,7 @@ FB_UNROLL
       float *row_joints = fb_log_row(P.log_joints, row, m.n_joints*m.joint_cols, P.env_pad, FB_VEC_JOINTS, e);
       float *row_contacts = fb_log_row(P.log_contacts, row, m.n_contacts*12, P.env_pad, FB_VEC_CONTACTS, e);
       float *row_xfrc = fb_log_row(P.log_xfrc, row, m.n_xfrc*6, P.env_pad, FB_VEC_XFRC, e);
-      const float time = (float)(P.it0 + k)*m.timestep;
+      const float time = (float)this->episode_it(P.it0 + k)*m.timestep;
       zfill = log_row_dirty(P.it0 + k + 1);
       if (role == 0) sflag[0] = 0;
       FB_BLOCK_BARRIER();

@@ -1262,7 +1262,7 @@ FB_UNROLL
       float *row_joints = fb_log_row(P.log_joints, row, m.n_joints*m.joint_cols, P.env_pad, FB_VEC_JOINTS, e);
       float *row_contacts = fb_log_row(P.log_contacts, row, m.n_contacts*12, P.env_pad, FB_VEC_CONTACTS, e);
       float *row_xfrc = fb_log_row(P.log_xfrc, row, m.n_xfrc*6, P.env_pad, FB_VEC_XFRC, e);
-      const float time = (float)(P.it0 + k)*m.timestep;
+      const float time = (float)this->episode_it(P.it0 + k)*m.timestep;
       const int maybe = this->pass_poses(row_links);
       if (rec[1].jtype == FB_JNT_FREE) { rt[3] = rqn[0]; rt[4] = rqn[1]; rt[5] = rqn[2]; rt[6] = rqn[3]; }
       float aroot[6] = {0.f, 0.f, 0.f, -m.grav[0], -m.grav[1], -m.grav[2]};
@@ -1310,7 +1310,7 @@ FB_UNROLL
       float *row_joints = fb_log_row(P.log_joints, row, m.n_joints*m.joint_cols, P.env_pad, FB_VEC_JOINTS, e);
       float *row_contacts = fb_log_row(P.log_contacts, row, m.n_contacts*12, P.env_pad, FB_VEC_CONTACTS, e);
       float *row_xfrc = fb_log_row(P.log_xfrc, row, m.n_xfrc*6, P.env_pad, FB_VEC_XFRC, e);
-      const float time = (float)(P.it0 + k)*m.timestep;
+      const float time = (float)this->episode_it(P.it0 + k)*m.timestep;
       const int maybe = rany(this->pass_poses(row_links));
       if (role == 0 && rec[1].jtype == FB_JNT_FREE) { rt[3] = rqn[0]; rt[4] = rqn[1]; rt[5] = rqn[2]; rt[6] = rqn[3]; }
       float aroot[6] = {0.f, 0.f, 0.f, -m.grav[0], -m.grav[1], -m.grav[2]};

@@ -32,6 +32,9 @@ ABI_SYMBOLS = {
                              ct.c_int, ct.c_int, ct.c_int, ct.POINTER(_H)]),
     'fb_destroy': (None, [_H]),
     'fb_reset': (ct.c_int, [_H, cabi.c_double_p, cabi.c_double_p]),
+    'fb_reset_envs': (ct.c_int, [_H, ct.c_int, ct.POINTER(ct.c_int32), cabi.c_double_p, cabi.c_double_p]),
+    'fb_reset_envs_where': (ct.c_int, [_H, ct.c_void_p, ct.c_void_p, ct.c_void_p]),
+    'fb_get_episode_start': (ct.c_int, [_H, cabi.c_int64_p]),
     'fb_set_ctrl': (ct.c_int, [_H, cabi.c_double_p]),
     'fb_set_qpos_spring': (ct.c_int, [_H, cabi.c_double_p]),
     'fb_set_ctrl_sequence': (ct.c_int, [_H, ct.c_void_p, ct.c_int]),
@@ -173,6 +176,31 @@ def _ptr(p):
     return ct.cast(p, ct.c_void_p).value or 0
 
 
+def _device_address(arr):
+    """Device address of a CUDA array (``__cuda_array_interface__``, or a torch CUDA tensor's
+    ``data_ptr()``); None for host data."""
+    if hasattr(arr, 'data_ptr') and getattr(arr, 'is_cuda', False):
+        return int(arr.data_ptr())
+    cai = getattr(arr, '__cuda_array_interface__', None)
+    return None if cai is None else int(cai['data'][0])
+
+
+def _device_shape(arr):
+    """(shape, typestr) of a CUDA array; it must be C-contiguous."""
+    cai = arr.__cuda_array_interface__
+    shape = tuple(int(d) for d in cai['shape'])
+    strides = cai.get('strides')
+    if strides is not None:
+        item = int(cai['typestr'][2:])
+        expect, acc = [], item
+        for d in reversed(shape):
+            expect.insert(0, acc)
+            acc *= d
+        if tuple(strides) != tuple(expect):
+            raise ValueError('reset_envs: device arrays must be C-contiguous')
+    return shape, cai['typestr']
+
+
 class BatchedPhysics:
     """``n_envs`` copies of one compiled FARMS model stepping in lockstep."""
     # pylint: disable=too-many-instance-attributes,too-many-public-methods
@@ -271,6 +299,79 @@ class BatchedPhysics:
             None if qp is None else qp.ctypes.data_as(cabi.c_double_p),
             None if qv is None else qv.ctypes.data_as(cabi.c_double_p)))
         self.iteration = 0
+
+    def reset_envs(self, envs, qpos=None, qvel=None):
+        """Restart some environments while the others keep running (fb_reset_envs): each one takes
+        its row of ``qpos`` / ``qvel`` (``None``: the keyframe), ctrl 0, and from here on steps as the
+        same environment of a freshly reset batch; its episode starts at the current ``iteration``
+        (``episode_start``), and its log accessors (``export_farms``, ``log_arrays(env=)``) return
+        that episode.  ``self.iteration`` stays the batch counter.
+
+        ``envs``: host int indices (``qpos [len(envs), nq]``, ``qvel [len(envs), nv]``) or a bool
+        ``[n_envs]`` host array (rows ``[n_envs, ...]``, those of unmasked environments ignored); or a
+        bool / uint8 ``[n_envs]`` CUDA array (``__cuda_array_interface__`` or ``data_ptr()``) with
+        float32 CUDA ``qpos [n_envs, nq]`` / ``qvel [n_envs, nv]``: stream-ordered on the engine's
+        stream (``fb_device_ptr_stream``), no host synchronisation, and not validated (a non-finite
+        row shows as ``flags`` bit 0 after the next step).  Refused between the sub-steps of a
+        logged iteration (``iteration % log_stride != 0``)."""
+        if self.iteration % self.log_stride:
+            raise ValueError(f'reset_envs: iteration {self.iteration} is not a full step (log_stride '
+                             f'{self.log_stride}); restart environments between logged iterations')
+        if _device_address(envs) is not None:
+            self._reset_envs_where(envs, qpos, qvel)
+            return
+        arr = np.asarray(envs)
+        if arr.dtype == np.bool_:
+            if arr.shape != (self.n_envs,):
+                raise ValueError(f'reset_envs: a bool mask must be [{self.n_envs}], got {list(arr.shape)}')
+            idx = np.flatnonzero(arr)
+            pick = lambda rows: None if rows is None else np.asarray(rows, dtype=np.float64)[idx]
+            qpos, qvel = pick(qpos), pick(qvel)
+        else:
+            if arr.size and not np.issubdtype(arr.dtype, np.integer):
+                raise TypeError(f'reset_envs: envs must be integer indices or a bool mask, got {arr.dtype}')
+            idx = arr.reshape(-1)
+        idx = np.ascontiguousarray(idx, dtype=np.int32)
+        rows = []
+        for name, values, width in (('qpos', qpos, self.model.nq), ('qvel', qvel, self.model.nv)):
+            if values is None:
+                rows.append(None)
+                continue
+            values = np.ascontiguousarray(values, dtype=np.float64)
+            if values.shape != (len(idx), width):
+                raise ValueError(f'reset_envs: {name} must be [{len(idx)}, {width}], got {list(values.shape)}')
+            rows.append(values)
+        self._check(self.lib.fb_reset_envs(
+            self._handle, len(idx), idx.ctypes.data_as(ct.POINTER(ct.c_int32)),
+            *[None if r is None else r.ctypes.data_as(cabi.c_double_p) for r in rows]))
+
+    def _reset_envs_where(self, mask, qpos, qvel):
+        """fb_reset_envs_where on device arrays (no host synchronisation)."""
+        shape, typestr = _device_shape(mask)
+        if shape != (self.n_envs,) or typestr not in ('|b1', '|u1'):
+            raise ValueError(f'reset_envs: a device mask must be bool / uint8 [{self.n_envs}], got {typestr} {list(shape)}')
+        ptrs = []
+        for name, values, width in (('qpos', qpos, self.model.nq), ('qvel', qvel, self.model.nv)):
+            if values is None:
+                ptrs.append(None)
+                continue
+            ptr = _device_address(values)
+            if ptr is None:
+                raise TypeError(f'reset_envs: with a device mask, {name} must be a CUDA array')
+            vshape, vtype = _device_shape(values)
+            if vshape != (self.n_envs, width) or vtype != '<f4':
+                raise ValueError(f'reset_envs: {name} must be float32 [{self.n_envs}, {width}] on the device, '
+                                 f'got {vtype} {list(vshape)}')
+            ptrs.append(ptr)
+        self._check(self.lib.fb_reset_envs_where(self._handle, _device_address(mask), *ptrs))
+
+    def episode_start(self):
+        """int64 ``[n_envs]``: the batch iteration (physics steps since ``reset``) at which each
+        environment's current episode began; 0 after ``reset``.  Episode iteration = ``iteration -
+        episode_start()``."""
+        out = np.zeros(self.n_envs, dtype=np.int64)
+        self._check(self.lib.fb_get_episode_start(self._handle, out.ctypes.data_as(cabi.c_int64_p)))
+        return out
 
     def step(self, n_steps=1, want_derived=False, sync=True):
         """``n_steps`` x (control -> mj_step -> log row -> drag) for every environment."""
@@ -532,8 +633,11 @@ class BatchedPhysics:
     def log_arrays(self, env=None):
         """Host copy of the device log: dict of ``[n_envs, ring, n_items, n_cols]`` float32
         (or ``[ring, n_items, n_cols]`` for one ``env``: exactly the reference's
-        ``data.sensors.<kind>.array`` shape, task.py:158)."""
+        ``data.sensors.<kind>.array`` shape, task.py:158).  The whole batch comes in batch rows; one
+        ``env`` comes as its current episode (``reset_envs``): row ``i`` of the episode's latest pass
+        over the ring, rows the episode has not reached zero."""
         log, names = self._log, self.names
+        start = 0 if env is None else int(self.episode_start()[int(env)])
         shapes = dict(
             links=(log.links_dev, len(names.links.names), sc.link_size, log.links_vec),
             joints=(log.joints_dev, len(names.joints.names), sc.joint_size, log.joints_vec),
@@ -554,6 +658,13 @@ class BatchedPhysics:
                 out[kind] = np.ascontiguousarray(arr).reshape(self.n_envs, ring, n_items, cols)
             else:
                 arr = raw[:, :, :, int(env), :]
+                if start > 0:
+                    # episode row r is device row (start + r*stride) % (ring*stride), a multiple of the
+                    # stride (reset_envs runs at full steps); rows past the episode's latest
+                    # iteration were not written in this episode
+                    r = np.arange(ring)
+                    arr = arr[(start//stride + r) % ring]
+                    arr[r*stride > self.iteration - start] = 0.0
                 out[kind] = np.ascontiguousarray(arr).reshape(ring, n_items, cols)
         return out
 

@@ -157,7 +157,7 @@ typedef struct FbStateView {
   float *qpos_spring_dev;  /* [n_envs][nq] */
   float *env_phase_dev;    /* [n_envs] */
   int32_t *flags_dev;      /* [n_envs] bit0: non-finite state (PhysicsError analogue, simulation.py:157-161); bit1: contact overflow; bit2: solver not converged */
-  int64_t *iteration_dev;  /* [n_envs] physics steps taken since reset */
+  int64_t *iteration_dev;  /* [n_envs] batch iteration: physics steps since fb_reset, the same for every environment after each step (fb_get_episode_start maps it to an environment's episode) */
 } FbStateView;
 
 /* mjData-like derived quantities of the state at the START of the last step
@@ -192,6 +192,32 @@ void fb_destroy(FbHandle *h);
  * qpos0/qvel0 ([n_envs,nq]/[n_envs,nv] host float64, NULL -> keyframe 0),
  * ctrl <- 0, iteration <- 0; runs the forward pass and writes log row 0. */
 int fb_reset(FbHandle *h, const double *qpos0, const double *qvel0);
+
+/* Per-environment episodes: restart some environments while the others keep running.  At batch
+ * iteration it, a restarted environment e takes the given state (or the keyframe), ctrl, xfrc_applied
+ * and flags <- 0, its on-device CPG rows <- the state last set by fb_set_cpg_state (rates 0), and
+ * runs the reset's forward pass, which writes its log row it % ring (the episode's row 0; the
+ * previous episode's terminal row there is overwritten) and its derived view.  From then on it steps
+ * bit for bit as environment e of a fresh batch (fb_reset, fb_set_cpg_state) would: the
+ * travelling-wave controller reads the episode's time.  qpos_spring, env_phase and the
+ * per-environment parameter tables are kept, as fb_reset keeps them.  Batch-wide nothing changes:
+ * the batch iteration, the control sequence and its position, the kernel selection.
+ *
+ * Restart the environments in envs[n] (host, no duplicates); qpos0 [n][nq] / qvel0 [n][nv] host
+ * float64 rows in the order of envs, NULL -> keyframe.  Uploads O(n) rows, not O(n_envs); n = 0
+ * enqueues nothing.  Refused, naming the first bad entry: an index out of range or given twice,
+ * a non-finite qpos0 / qvel0 value. */
+int fb_reset_envs(FbHandle *h, int n, const int32_t *envs, const double *qpos0, const double *qvel0);
+/* Same from device memory, stream-ordered, no host synchronisation: mask [n_envs] uint8 (non-zero
+ * = restart), qpos0 [n_envs][nq] / qvel0 [n_envs][nv] float32 (rows of unmasked environments are
+ * not read; NULL -> keyframe).  Write them on the handle's stream (fb_device_ptr_stream) or
+ * synchronise first.  Device data cannot be validated here: a non-finite row shows as flags bit 0
+ * after the next step. */
+int fb_reset_envs_where(FbHandle *h, const uint8_t *mask, const float *qpos0, const float *qvel0);
+/* [n_envs] batch iteration of each environment's episode row 0 (0 after fb_reset).  Accessors of
+ * one environment (fb_export_farms) return its current episode; whole-batch ones (fb_export_rows,
+ * fb_step_host, FbLogView) keep batch rows. */
+int fb_get_episode_start(FbHandle *h, int64_t *out);
 
 /* Control inputs (task.py:307,317,332,343-346). */
 int fb_set_ctrl(FbHandle *h, const double *ctrl);                 /* [n_envs][nu] */
@@ -270,7 +296,9 @@ int fb_state_view(FbHandle *h, FbStateView *out);
 int fb_derived_view(FbHandle *h, FbDerivedView *out);
 
 /* Copy one environment's log to host float64 arrays shaped like the
- * reference's data.sensors.<kind>.array (NULL pointers are skipped). */
+ * reference's data.sensors.<kind>.array (NULL pointers are skipped).  Rows are those of the
+ * environment's current episode: row r is device row (s + r) % ring, s = its episode start; when
+ * s > 0, rows the episode has not reached yet are zero (as in a fresh log). */
 int fb_export_farms(FbHandle *h, int env, double *links, double *joints,
                     double *contacts, double *xfrc);
 /* End-to-end call on HOST buffers (pinned recommended), the batched analogue of
