@@ -21,6 +21,7 @@
 #include <ctime>
 #include <new>
 #include <string>
+#include <type_traits>
 #include <vector>
 #ifdef FB_HOST_EMU
 #include <thread>
@@ -97,6 +98,10 @@ FB_DEV void fb_reset_env(const FbResetArgs &A, int env) {
 }
 
 /* --------------------------------------------------------------- kernels */
+/* behind the body blocks of a SPLIT block: root position [3][32] + hand-over flags [32] ... */
+#define FB_SPLIT_EXTRA_BYTES 512
+/* ... and of a constrained SPLIT block, floats per lane: root position [3], hand-over flag, reduction buffers */
+#define FB_CSPLIT_EXTRA (4 + 2*FB_SPLIT_MAXW*FB_RED_MAX)
 #ifndef FB_HOST_EMU
 /* only: FB_MODE_RESET of fb_reset_envs, the environments to restart ([n_envs], non-zero); NULL: all */
 template <int TEAM>
@@ -128,48 +133,46 @@ struct FbFastParams {
   FastRec rec[FB_FAST_MAXBODY];   /* per-body records, read from the constant bank */
 };
 
+/* Every per-thread kernel takes ENVP as its last template argument.  ENVP = 1 reads the
+ * per-environment parameter tables of fb_set_env_param and runs the episode clock of fb_reset_envs;
+ * its parameters are the ENVP = 0 struct with the tables appended (Fb*EnvParams), so the ENVP = 0
+ * layouts stay as they are.  fb_plan picks ENVP = 1 while a table the kernel reads is set or the
+ * episode clock is bound.  Each body is written out inside its __global__ function rather than
+ * called as an inlined function, which ptxas was found to schedule differently. */
+template <int ENVP, class Q> FB_DEV const FbEnvTables *fb_env_tables(const Q &q) {
+  if constexpr (ENVP != 0) return &q.T; else return nullptr;
+}
+struct FbFastEnvParams : FbFastParams { FbEnvTables T; };
+
 /* BLK environments per warp (32, or 16 in a half-filled warp).  MULTI: blocks of 2..8 warps
  * (blockDim.x/32) kept in step by a barrier per physics step (FbFast::run_t). */
-/* Every per-thread entry point has an ENVP twin (fb_*_envp_kernel, same template arguments) that reads
- * the per-environment parameter tables of fb_set_env_param and runs the episode clock of
- * fb_reset_envs; launch() takes the twin while a table the kernel reads is set: any table for the
- * constrained kernels, any but the candidate friction for the unconstrained ones (they have no
- * contacts), and while the episode clock is bound.  An entry point and its twin expand the same body
- * (FB_*_BODY: ENVP is a template argument
- * of FbFast / FbFastCon, T the tables); written out in each kernel rather than called as an inlined
- * function, which ptxas was found to schedule differently.  A twin's parameters are the entry
- * point's with the tables appended; the entry point's keep their layout. */
-struct FbFastEnvParams : FbFastParams { FbEnvTables T; };
-#define FB_FAST_BODY(ENVP, T) \
-  extern __shared__ __align__(16) float fb_smem[];                                                                    \
-  const FbParams &P = Q.P;                                                                                            \
-  const int warp = MULTI ? threadIdx.x >> 5 : 0, lane = MULTI ? threadIdx.x & 31 : threadIdx.x;                       \
-  const int wid = MULTI ? blockIdx.x*(blockDim.x >> 5) + warp : blockIdx.x;   /* warp index of the launch */          \
-  const int env = wid*BLK + lane;                                                                                     \
-  if (blockIdx.x == 0 && threadIdx.x == 0) P.pending_count[P.parity ^ 1] = 0;   /* for the next launch */             \
-  const int valid = env < P.n_envs;                                                                                   \
-  if (!MULTI && !valid) return;                                                                                       \
-  const int n_float = SLIM ? P.m.X.n_float_slim : P.m.X.n_float;                                                      \
-  const size_t warp_floats = (size_t)n_float*BLK;                                                                     \
-  /* L2-resident scratch [warp][field][lane]: compile-time strides, coalesced */                                      \
-  FbFast<BLK, SLIM, LEAN, 0, ENVP> st(P, Q.rec, fb_smem + warp*warp_floats + lane,                                    \
-                             P.fast_scratch + (size_t)wid*(SLIM ? P.m.X.n_scratch_slim : P.m.X.n_scratch)*BLK + lane, \
-                             valid ? env : 0, T);                                                                     \
-  /* full warps move their state through a shared-memory tile (coalesced); a partial last                             \
-   * warp, or a model whose state rows do not fit the tile, uses per-thread accesses (the SLIM                        \
-   * layout's smaller blocks take the rows in two phases) */                                                          \
-  const int coop = BLK == 32 && (wid + 1)*BLK <= P.n_envs ? (SLIM ? 2*P.m.X.coop_io2 : P.m.X.coop_io) : 0;            \
-  const int done = st.template run_t<MULTI>(coop, lane, valid);                                                       \
-  if (valid && done < P.n_steps) {                                                                                    \
-    P.steps_done[env] = done;                                                                                         \
-    P.pending[atomicAdd(P.pending_count + P.parity, 1)] = env;                                                        \
+template <int BLK, int SLIM, int MULTI, int LEAN, int ENVP>
+__global__ void __launch_bounds__(MULTI ? 256 : 32)
+fb_fast_kernel(const __grid_constant__ std::conditional_t<ENVP != 0, FbFastEnvParams, FbFastParams> Q) {
+  extern __shared__ __align__(16) float fb_smem[];
+  const FbParams &P = Q.P;
+  const int warp = MULTI ? threadIdx.x >> 5 : 0, lane = MULTI ? threadIdx.x & 31 : threadIdx.x;
+  const int wid = MULTI ? blockIdx.x*(blockDim.x >> 5) + warp : blockIdx.x;   /* warp index of the launch */
+  const int env = wid*BLK + lane;
+  if (blockIdx.x == 0 && threadIdx.x == 0) P.pending_count[P.parity ^ 1] = 0;   /* for the next launch */
+  const int valid = env < P.n_envs;
+  if (!MULTI && !valid) return;
+  const int n_float = SLIM ? P.m.X.n_float_slim : P.m.X.n_float;
+  const size_t warp_floats = (size_t)n_float*BLK;
+  /* L2-resident scratch [warp][field][lane]: compile-time strides, coalesced */
+  FbFast<BLK, SLIM, LEAN, 0, ENVP> st(P, Q.rec, fb_smem + warp*warp_floats + lane,
+                             P.fast_scratch + (size_t)wid*(SLIM ? P.m.X.n_scratch_slim : P.m.X.n_scratch)*BLK + lane,
+                             valid ? env : 0, fb_env_tables<ENVP>(Q));
+  /* full warps move their state through a shared-memory tile (coalesced); a partial last
+   * warp, or a model whose state rows do not fit the tile, uses per-thread accesses (the SLIM
+   * layout's smaller blocks take the rows in two phases) */
+  const int coop = BLK == 32 && (wid + 1)*BLK <= P.n_envs ? (SLIM ? 2*P.m.X.coop_io2 : P.m.X.coop_io) : 0;
+  const int done = st.template run_t<MULTI>(coop, lane, valid);
+  if (valid && done < P.n_steps) {
+    P.steps_done[env] = done;
+    P.pending[atomicAdd(P.pending_count + P.parity, 1)] = env;
   }
-template <int BLK, int SLIM, int MULTI, int LEAN = 0>
-__global__ void __launch_bounds__(MULTI ? 256 : 32)
-fb_fast_kernel(const __grid_constant__ FbFastParams Q) { FB_FAST_BODY(0, 0) }
-template <int BLK, int SLIM, int MULTI, int LEAN = 0>
-__global__ void __launch_bounds__(MULTI ? 256 : 32)
-fb_fast_envp_kernel(const __grid_constant__ FbFastEnvParams Q) { FB_FAST_BODY(1, &Q.T) }
+}
 
 /* SPLIT variant (small batches): one block = 32 environments stepped by split.nwarps warps */
 struct FbFastSplitParams {
@@ -177,7 +180,6 @@ struct FbFastSplitParams {
   FastRec rec[FB_FAST_MAXBODY];
   FastSplit split;
 };
-#define FB_SPLIT_EXTRA_BYTES 512       /* root position [3][32] + hand-over flags [32] behind the body blocks */
 
 /* registers capped for 3 blocks of 128 threads per SM (168): with the 96-thread blocks of a
  * three-way split four blocks are then resident (shared memory allows four), i.e. 592 blocks =
@@ -188,30 +190,27 @@ struct FbFastSplitParams {
 #define FB_SPLIT_MINBLOCKS 3
 #endif
 struct FbFastSplitEnvParams : FbFastSplitParams { FbEnvTables T; };
-#define FB_FAST_SPLIT_BODY(ENVP, T) \
-  extern __shared__ __align__(16) float fb_smem[];                                                                  \
-  const FbParams &P = Q.P;                                                                                          \
-  const int role = threadIdx.x >> 5, lane = threadIdx.x & 31, wid = blockIdx.x;                                     \
-  const int env = wid*32 + lane;                                                                                    \
-  if (blockIdx.x == 0 && threadIdx.x == 0) P.pending_count[P.parity ^ 1] = 0;   /* for the next launch */           \
-  const int valid = env < P.n_envs;                                                                                 \
-  const int n_float = P.m.X.n_float;                                                                                \
-  FbFast<32, 0, LEAN, 1, ENVP> st(P, Q.rec, fb_smem + lane, P.fast_scratch + (size_t)wid*P.m.X.n_scratch*32 + lane, \
-                            valid ? env : 0, T);                                                                    \
-  float *extra = fb_smem + (size_t)n_float*32;                                                                      \
-  st.split_setup(Q.split, role, extra + lane, reinterpret_cast<int *>(extra + 3*32) + lane);                        \
-  const int coop = (wid + 1)*32 <= P.n_envs ? P.m.X.coop_io : 0;                                                    \
-  const int done = st.run_split(coop, lane, valid);                                                                 \
-  if (role == 0 && valid && done < P.n_steps) {                                                                     \
-    P.steps_done[env] = done;                                                                                       \
-    P.pending[atomicAdd(P.pending_count + P.parity, 1)] = env;                                                      \
+template <int LEAN, int ENVP>
+__global__ void __launch_bounds__(32*FB_SPLIT_MAXW, FB_SPLIT_MINBLOCKS)
+fb_fast_split_kernel(const __grid_constant__ std::conditional_t<ENVP != 0, FbFastSplitEnvParams, FbFastSplitParams> Q) {
+  extern __shared__ __align__(16) float fb_smem[];
+  const FbParams &P = Q.P;
+  const int role = threadIdx.x >> 5, lane = threadIdx.x & 31, wid = blockIdx.x;
+  const int env = wid*32 + lane;
+  if (blockIdx.x == 0 && threadIdx.x == 0) P.pending_count[P.parity ^ 1] = 0;   /* for the next launch */
+  const int valid = env < P.n_envs;
+  const int n_float = P.m.X.n_float;
+  FbFast<32, 0, LEAN, 1, ENVP> st(P, Q.rec, fb_smem + lane, P.fast_scratch + (size_t)wid*P.m.X.n_scratch*32 + lane,
+                            valid ? env : 0, fb_env_tables<ENVP>(Q));
+  float *extra = fb_smem + (size_t)n_float*32;
+  st.split_setup(Q.split, role, extra + lane, reinterpret_cast<int *>(extra + 3*32) + lane);
+  const int coop = (wid + 1)*32 <= P.n_envs ? P.m.X.coop_io : 0;
+  const int done = st.run_split(coop, lane, valid);
+  if (role == 0 && valid && done < P.n_steps) {
+    P.steps_done[env] = done;
+    P.pending[atomicAdd(P.pending_count + P.parity, 1)] = env;
   }
-template <int LEAN>
-__global__ void __launch_bounds__(32*FB_SPLIT_MAXW, FB_SPLIT_MINBLOCKS)
-fb_fast_split_kernel(const __grid_constant__ FbFastSplitParams Q) { FB_FAST_SPLIT_BODY(0, 0) }
-template <int LEAN>
-__global__ void __launch_bounds__(32*FB_SPLIT_MAXW, FB_SPLIT_MINBLOCKS)
-fb_fast_split_envp_kernel(const __grid_constant__ FbFastSplitEnvParams Q) { FB_FAST_SPLIT_BODY(1, &Q.T) }
+}
 
 struct FbFastConParams {
   FbParams P;
@@ -221,28 +220,25 @@ struct FbFastConParams {
 static_assert(sizeof(FbFastConParams) <= 32764, "kernel parameters of fb_fastc_kernel exceed 32 KB");
 
 struct FbFastConEnvParams : FbFastConParams { FbEnvTables T; };
-static_assert(sizeof(FbFastConEnvParams) <= 32764, "kernel parameters of fb_fastc_envp_kernel exceed 32 KB");
-#define FB_FASTC_BODY(ENVP, T) \
-  extern __shared__ __align__(16) float fb_smem[];                                                                             \
-  const FbParams &P = Q.P;                                                                                                     \
-  const int i = blockIdx.x*BLK + threadIdx.x;                                                                                  \
-  const int count = P.use_pending ? P.pending_count[P.parity] : P.n_envs;                                                      \
-  if (i >= count) return;                                                                                                      \
-  if (P.con_split_done && P.con_split_done[blockIdx.x]) return;      /* stepped by the SPLIT variant */                        \
-  const int identity = !P.use_pending || count == P.n_envs;                                                                    \
-  const int env = identity ? i : P.pending[i];                                                                                 \
-  const int k0 = P.use_pending ? P.steps_done[env] : 0;                                                                        \
-  const size_t t0 = (size_t)blockIdx.x*BLK;                                                                                    \
-  FbFastCon<BLK, LEAN, 0, ENVP> st(P, Q.rec, Q.cand, fb_smem + threadIdx.x, P.fast_scratch + t0*P.m.X.n_scratch + threadIdx.x, \
-                    P.con_scratch + t0*P.m.X.n_con + threadIdx.x, env, T);                                                     \
-  const int coop = BLK == 32 && identity && P.m.X.coop_io && (blockIdx.x + 1)*BLK <= count;                                    \
-  st.run_con(k0, coop, threadIdx.x);                                                                                           
-template <int BLK, int LEAN = 0>
+static_assert(sizeof(FbFastConEnvParams) <= 32764, "kernel parameters of fb_fastc_kernel<..., 1> exceed 32 KB");
+template <int BLK, int LEAN, int ENVP>
 __global__ void __launch_bounds__(BLK)
-fb_fastc_kernel(const __grid_constant__ FbFastConParams Q) { FB_FASTC_BODY(0, 0) }
-template <int BLK, int LEAN = 0>
-__global__ void __launch_bounds__(BLK)
-fb_fastc_envp_kernel(const __grid_constant__ FbFastConEnvParams Q) { FB_FASTC_BODY(1, &Q.T) }
+fb_fastc_kernel(const __grid_constant__ std::conditional_t<ENVP != 0, FbFastConEnvParams, FbFastConParams> Q) {
+  extern __shared__ __align__(16) float fb_smem[];
+  const FbParams &P = Q.P;
+  const int i = blockIdx.x*BLK + threadIdx.x;
+  const int count = P.use_pending ? P.pending_count[P.parity] : P.n_envs;
+  if (i >= count) return;
+  if (P.con_split_done && P.con_split_done[blockIdx.x]) return;      /* stepped by the SPLIT variant */
+  const int identity = !P.use_pending || count == P.n_envs;
+  const int env = identity ? i : P.pending[i];
+  const int k0 = P.use_pending ? P.steps_done[env] : 0;
+  const size_t t0 = (size_t)blockIdx.x*BLK;
+  FbFastCon<BLK, LEAN, 0, ENVP> st(P, Q.rec, Q.cand, fb_smem + threadIdx.x, P.fast_scratch + t0*P.m.X.n_scratch + threadIdx.x,
+                    P.con_scratch + t0*P.m.X.n_con + threadIdx.x, env, fb_env_tables<ENVP>(Q));
+  const int coop = BLK == 32 && identity && P.m.X.coop_io && (blockIdx.x + 1)*BLK <= count;
+  st.run_con(k0, coop, threadIdx.x);
+}
 
 /* SPLIT variant of the constrained kernel: one block = the BLK environments of one group (the
  * lanes of a warp; the upper half-warp leaves at once when BLK = 16) stepped by split.nwarps
@@ -256,58 +252,31 @@ struct FbFastConSplitParams {
   FastSplit split;
 };
 static_assert(sizeof(FbFastConSplitParams) <= 32764, "kernel parameters of fb_fastc_split_kernel exceed 32 KB");
-/* floats per lane behind the body blocks: root position [3], hand-over flag, reduction buffers */
-#define FB_CSPLIT_EXTRA (4 + 2*FB_SPLIT_MAXW*FB_RED_MAX)
 #ifndef FB_CSPLIT_MINBLOCKS
 #define FB_CSPLIT_MINBLOCKS 2
 #endif
 struct FbFastConSplitEnvParams : FbFastConSplitParams { FbEnvTables T; };
-static_assert(sizeof(FbFastConSplitEnvParams) <= 32764, "kernel parameters of fb_fastc_split_envp_kernel exceed 32 KB");
-#define FB_FASTC_SPLIT_BODY(ENVP, T) \
-  extern __shared__ __align__(16) float fb_smem[];                                                                       \
-  const FbParams &P = Q.P;                                                                                               \
-  const int role = threadIdx.x >> 5, lane = threadIdx.x & 31, grp = blockIdx.x;                                          \
-  const int env = grp*BLK + lane;                                                                                        \
-  if (lane >= BLK || env >= P.n_envs) return;                                                                            \
-  /* block-uniform: every warp sees the same lanes */                                                                    \
-  const int all0 = P.pending_count[P.parity] == P.n_envs && __ballot_sync(__activemask(), P.steps_done[env] != 0) == 0u; \
-  if (threadIdx.x == 0) P.con_split_done[grp] = all0;                                                                    \
-  if (!all0) return;                                                                                                     \
-  const size_t t0 = (size_t)grp*BLK;                                                                                     \
-  FbFastCon<BLK, LEAN, 1, ENVP> st(P, Q.rec, Q.cand, fb_smem + lane, P.fast_scratch + t0*P.m.X.n_scratch + lane,         \
-                             P.con_scratch + t0*P.m.X.n_con + lane, env, T);                                             \
-  float *extra = fb_smem + (size_t)P.m.X.n_float*BLK;                                                                    \
-  st.split_setup(Q.split, role, extra + lane, reinterpret_cast<int *>(extra + 3*BLK) + lane);                            \
-  st.con_split_setup(Q.split, extra + 4*BLK + lane);                                                                     \
-  const int coop = BLK == 32 && P.m.X.coop_io && (grp + 1)*BLK <= P.n_envs;                                              \
-  st.run_con_split(coop, lane);                                                                                          
-template <int BLK, int LEAN>
+static_assert(sizeof(FbFastConSplitEnvParams) <= 32764, "kernel parameters of fb_fastc_split_kernel<..., 1> exceed 32 KB");
+template <int BLK, int LEAN, int ENVP>
 __global__ void __launch_bounds__(32*FB_SPLIT_MAXW, FB_CSPLIT_MINBLOCKS)
-fb_fastc_split_kernel(const __grid_constant__ FbFastConSplitParams Q) { FB_FASTC_SPLIT_BODY(0, 0) }
-template <int BLK, int LEAN>
-__global__ void __launch_bounds__(32*FB_SPLIT_MAXW, FB_CSPLIT_MINBLOCKS)
-fb_fastc_split_envp_kernel(const __grid_constant__ FbFastConSplitEnvParams Q) { FB_FASTC_SPLIT_BODY(1, &Q.T) }
-
-/* launch an entry point or its ENVP twin */
-template <int BLK, int SLIM, int MULTI, int LEAN>
-static void fb_launch_fast(bool envp, int grid, int threads, size_t bytes, cudaStream_t st, const FbFastEnvParams &Q) {
-  if (envp) fb_fast_envp_kernel<BLK, SLIM, MULTI, LEAN><<<grid, threads, bytes, st>>>(Q);
-  else fb_fast_kernel<BLK, SLIM, MULTI, LEAN><<<grid, threads, bytes, st>>>(static_cast<const FbFastParams &>(Q));
-}
-template <int LEAN>
-static void fb_launch_fast_split(bool envp, int grid, int threads, size_t bytes, cudaStream_t st, const FbFastSplitEnvParams &Q) {
-  if (envp) fb_fast_split_envp_kernel<LEAN><<<grid, threads, bytes, st>>>(Q);
-  else fb_fast_split_kernel<LEAN><<<grid, threads, bytes, st>>>(static_cast<const FbFastSplitParams &>(Q));
-}
-template <int BLK, int LEAN>
-static void fb_launch_fastc(bool envp, int grid, size_t bytes, cudaStream_t st, const FbFastConEnvParams &Q) {
-  if (envp) fb_fastc_envp_kernel<BLK, LEAN><<<grid, BLK, bytes, st>>>(Q);
-  else fb_fastc_kernel<BLK, LEAN><<<grid, BLK, bytes, st>>>(static_cast<const FbFastConParams &>(Q));
-}
-template <int BLK, int LEAN>
-static void fb_launch_fastc_split(bool envp, int grid, int threads, size_t bytes, cudaStream_t st, const FbFastConSplitEnvParams &Q) {
-  if (envp) fb_fastc_split_envp_kernel<BLK, LEAN><<<grid, threads, bytes, st>>>(Q);
-  else fb_fastc_split_kernel<BLK, LEAN><<<grid, threads, bytes, st>>>(static_cast<const FbFastConSplitParams &>(Q));
+fb_fastc_split_kernel(const __grid_constant__ std::conditional_t<ENVP != 0, FbFastConSplitEnvParams, FbFastConSplitParams> Q) {
+  extern __shared__ __align__(16) float fb_smem[];
+  const FbParams &P = Q.P;
+  const int role = threadIdx.x >> 5, lane = threadIdx.x & 31, grp = blockIdx.x;
+  const int env = grp*BLK + lane;
+  if (lane >= BLK || env >= P.n_envs) return;
+  /* block-uniform: every warp sees the same lanes */
+  const int all0 = P.pending_count[P.parity] == P.n_envs && __ballot_sync(__activemask(), P.steps_done[env] != 0) == 0u;
+  if (threadIdx.x == 0) P.con_split_done[grp] = all0;
+  if (!all0) return;
+  const size_t t0 = (size_t)grp*BLK;
+  FbFastCon<BLK, LEAN, 1, ENVP> st(P, Q.rec, Q.cand, fb_smem + lane, P.fast_scratch + t0*P.m.X.n_scratch + lane,
+                             P.con_scratch + t0*P.m.X.n_con + lane, env, fb_env_tables<ENVP>(Q));
+  float *extra = fb_smem + (size_t)P.m.X.n_float*BLK;
+  st.split_setup(Q.split, role, extra + lane, reinterpret_cast<int *>(extra + 3*BLK) + lane);
+  st.con_split_setup(Q.split, extra + 4*BLK + lane);
+  const int coop = BLK == 32 && P.m.X.coop_io && (grp + 1)*BLK <= P.n_envs;
+  st.run_con_split(coop, lane);
 }
 
 /* Stand-alone drag operator (fb_drag_forces, fb_drag.h): one thread = one link row */
@@ -432,6 +401,87 @@ __global__ void fb_gather_env_kernel(const float *__restrict__ log, int ring, in
 }
 #endif
 
+/* ------------------------------------------------------ per-thread kernel variants */
+enum { FB_FAST, FB_FAST_SPLIT, FB_FASTC, FB_FASTC_SPLIT };      /* FbKernelSel::kind */
+
+/* One per-thread kernel launch: the instantiation and its shape.  FB_FAST covers the regular
+ * layout (BLK = 32 or 16), SLIM (BLK = 32) and SLIM in blocks of threads/32 warps (MULTI);
+ * BLK of the constrained kernels is the environments per group. */
+struct FbKernelSel {
+  int kind, blk, slim, multi, lean, envp;
+  int grid, threads;
+  size_t bytes;
+};
+
+template <int KIND, int BLK, int SLIM, int MULTI, int LEAN, int ENVP> struct FbVariant {
+  static constexpr int kind = KIND, blk = BLK, slim = SLIM, multi = MULTI, lean = LEAN, envp = ENVP;
+};
+template <int KIND, int BLK, int SLIM, int MULTI, class F> static void fb_dispatch_le(const FbKernelSel &k, F &f) {
+  if (k.lean) {
+    if (k.envp) f(FbVariant<KIND, BLK, SLIM, MULTI, 1, 1>()); else f(FbVariant<KIND, BLK, SLIM, MULTI, 1, 0>());
+  } else {
+    if (k.envp) f(FbVariant<KIND, BLK, SLIM, MULTI, 0, 1>()); else f(FbVariant<KIND, BLK, SLIM, MULTI, 0, 0>());
+  }
+}
+/* The per-thread kernels built, each with LEAN x ENVP: calls f(FbVariant<...>()) for the one `k`
+ * selects.  Every launch, attribute and occupancy query of a per-thread kernel, and the emulation
+ * (which runs each variant with BLK = 1), goes through here. */
+template <class F> static void fb_dispatch(const FbKernelSel &k, F &&f) {
+  switch (k.kind) {
+    case FB_FAST:
+      if (k.blk == 16) fb_dispatch_le<FB_FAST, 16, 0, 0>(k, f);
+      else if (!k.slim) fb_dispatch_le<FB_FAST, 32, 0, 0>(k, f);
+      else if (!k.multi) fb_dispatch_le<FB_FAST, 32, 1, 0>(k, f);
+      else fb_dispatch_le<FB_FAST, 32, 1, 1>(k, f);
+      break;
+    case FB_FAST_SPLIT: fb_dispatch_le<FB_FAST_SPLIT, 32, 0, 0>(k, f); break;
+    case FB_FASTC:
+      if (k.blk == 16) fb_dispatch_le<FB_FASTC, 16, 0, 0>(k, f); else fb_dispatch_le<FB_FASTC, 32, 0, 0>(k, f);
+      break;
+    default:
+      if (k.blk == 16) fb_dispatch_le<FB_FASTC_SPLIT, 16, 0, 0>(k, f); else fb_dispatch_le<FB_FASTC_SPLIT, 32, 0, 0>(k, f);
+      break;
+  }
+}
+
+#ifndef FB_HOST_EMU
+template <class V> static auto fb_kernel_of(V) {
+  if constexpr (V::kind == FB_FAST) return fb_fast_kernel<V::blk, V::slim, V::multi, V::lean, V::envp>;
+  else if constexpr (V::kind == FB_FAST_SPLIT) return fb_fast_split_kernel<V::lean, V::envp>;
+  else if constexpr (V::kind == FB_FASTC) return fb_fastc_kernel<V::blk, V::lean, V::envp>;
+  else return fb_fastc_split_kernel<V::blk, V::lean, V::envp>;
+}
+
+/* The shared-memory attributes of the four LEAN x ENVP instantiations of `k` for k.bytes and, with
+ * per_sm, the fewest blocks of k.threads of them an SM holds */
+static cudaError_t fb_kernel_attributes(FbKernelSel k, int *per_sm = nullptr) {
+  cudaError_t ce = cudaSuccess;
+  if (per_sm) *per_sm = 1 << 30;
+  for (int v = 0; v < 4 && ce == cudaSuccess; v++) {
+    k.lean = v & 1; k.envp = v >> 1;
+    fb_dispatch(k, [&](auto var) {
+      const void *f = (const void *)fb_kernel_of(var);
+      ce = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.bytes);
+      if (ce == cudaSuccess) ce = cudaFuncSetAttribute(f, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+      int nb = 0;
+      if (ce == cudaSuccess && per_sm) ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, f, k.threads, k.bytes);
+      if (per_sm && nb < *per_sm) *per_sm = nb;
+    });
+  }
+  return ce;
+}
+
+/* the team kernel of `team` lanes per environment */
+typedef void (*FbTeamKernel)(FbParams, FbEnvTables, const uint8_t *);
+static FbTeamKernel fb_team_kernel(int team) {
+  switch (team) {
+    case 8: return fb_step_kernel<8>;
+    case 16: return fb_step_kernel<16>;
+    default: return fb_step_kernel<32>;
+  }
+}
+#endif
+
 /* ---------------------------------------------------------------- handle */
 enum { FB_N_ENV_PARAM = FB_ENV_CAND_FRICTION + 1 };     /* fields of fb_set_env_param */
 
@@ -454,8 +504,6 @@ struct FbHandle {
   bool fast_block_auto;             /* 16 environments per warp chosen by the heuristic ... */
   int block_review;                 /* ... and reviewed after the first launch of an episode */
   int max_smem;
-  size_t fast_slim_smem_bytes;
-  size_t fast_smem_bytes;
   long long launch_parity;
   int log_used;                     /* 0 until the first reset: the log is as fb_create zeroed it */
 #ifndef FB_HOST_EMU
@@ -635,14 +683,6 @@ static int upload_model(FbHandle *h) {
   return 0;
 }
 
-#ifndef FB_HOST_EMU
-static int fb_set_fast_block(FbHandle *h, int blk);
-static long long fb_con_split_blocks(FbHandle *h, int blk, cudaError_t *ce);
-
-static long long fb_con_cost(long long n_envs, int blk, long long capacity, int split);
-static bool fb_con_split_pays(FbHandle *h);
-#endif
-
 /* capacity of the device control sequence ([n_steps][nu][env_pad] + the upload staging) */
 static int ensure_sequence(FbHandle *h, int n_steps) {
   const DevModel &m = h->hm.m;
@@ -660,6 +700,155 @@ static int ensure_sequence(FbHandle *h, int n_steps) {
   return 0;
 }
 
+/* A per-thread kernel over the handle's batch with its launch shape: `blk` environments per warp
+ * (per group for the constrained kernels), SLIM in blocks of `wpb` warps; LEAN and ENVP are 0. */
+static FbKernelSel fb_kernel_sel(const FbHandle *h, int kind, int blk, int slim = 0, int wpb = 1) {
+  const size_t per_env = (size_t)(slim ? h->hm.m.X.n_float_slim : h->hm.m.X.n_float)*sizeof(float);
+  const int n = h->P.n_envs, warps = (n + 31)/32, split_threads = 32*h->hm.split.nwarps;
+  FbKernelSel k = {kind, blk, slim, wpb > 1, 0, 0, (n + blk - 1)/blk, blk, per_env*blk};
+  if (kind == FB_FAST_SPLIT) {
+    k.grid = warps; k.threads = split_threads; k.bytes += FB_SPLIT_EXTRA_BYTES;
+  } else if (kind == FB_FASTC_SPLIT) {
+    k.threads = split_threads; k.bytes += (size_t)FB_CSPLIT_EXTRA*blk*sizeof(float);
+  } else if (slim) {
+    k.grid = (warps + wpb - 1)/wpb; k.threads = 32*wpb; k.bytes *= wpb;
+  }
+  return k;
+}
+
+#ifndef FB_HOST_EMU
+/* blocks of `k` (any LEAN x ENVP) the device holds at once, its attributes set on the way; 0 on an error */
+static long long fb_capacity(FbHandle *h, const FbKernelSel &k, cudaError_t *ce) {
+  int per_sm = 0;
+  if (*ce == cudaSuccess) *ce = fb_kernel_attributes(k, &per_sm);
+  return *ce == cudaSuccess ? (long long)per_sm*h->sms : 0;
+}
+
+/* blocks of the constrained SPLIT variant the device holds at once with `blk` environments per group
+ * (0: not applicable) */
+static long long fb_con_split_blocks(FbHandle *h, int blk, cudaError_t *ce) {
+  const FbKernelSel k = fb_kernel_sel(h, FB_FASTC_SPLIT, blk);
+  if (!h->hm.m.X.con_ok || h->hm.split.nwarps < 2 || k.bytes > (size_t)h->max_smem) return 0;
+  return fb_capacity(h, k, ce);
+}
+
+/* A ground-contact launch is as long as one group's step sequence times the number of waves its
+ * blocks take: the SPLIT variant shortens the sequence (x FB_CSPLIT_GAIN, measured r2y: 1.7 .. 2.0
+ * faster per wave) and holds fewer groups per wave.  Cost of stepping n_envs environments in
+ * groups of blk, in units of a single-warp wave x 100; 0 = not available. */
+#define FB_CSPLIT_GAIN 55
+static long long fb_con_cost(long long n_envs, int blk, long long capacity, int split) {
+  if (capacity <= 0) return 0;
+  const long long groups = (n_envs + blk - 1)/blk, waves = (groups + capacity - 1)/capacity;
+  return waves*(split ? FB_CSPLIT_GAIN : 100);
+}
+static bool fb_con_split_pays(const FbHandle *h) {
+  const long long cs = fb_con_cost(h->P.n_envs, h->fast_block, h->con_split_capacity, 1);
+  const long long c1 = fb_con_cost(h->P.n_envs, h->fast_block, h->con_single_capacity, 0);
+  return cs > 0 && (c1 == 0 || cs < c1);
+}
+
+/* environments per warp of the per-thread kernels (regular layout): shared-memory attributes and
+ * the capacities of the SPLIT variants and the single-warp constrained kernel */
+static int fb_set_fast_block(FbHandle *h, int blk) {
+  h->fast_block = blk;
+  cudaError_t ce = fb_kernel_attributes(fb_kernel_sel(h, FB_FAST, blk));
+  if (ce == cudaSuccess) ce = fb_kernel_attributes(fb_kernel_sel(h, FB_FASTC, blk));
+  const FbKernelSel split = fb_kernel_sel(h, FB_FAST_SPLIT, 32), single = fb_kernel_sel(h, FB_FASTC, blk);
+  /* the SPLIT variant pays while ALL its blocks are resident at once (one wave) */
+  h->split_capacity = 0;
+  if (blk == 32 && h->hm.split.nwarps > 1 && split.bytes <= (size_t)h->max_smem) h->split_capacity = fb_capacity(h, split, &ce);
+  h->con_split_capacity = fb_con_split_blocks(h, blk, &ce);
+  h->con_single_capacity = 0;
+  if (h->hm.m.X.con_ok && single.bytes <= (size_t)h->max_smem) h->con_single_capacity = fb_capacity(h, single, &ce);
+  return ce == cudaSuccess ? 0 : fail(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ce));
+}
+
+/* shared-memory attributes of the SLIM variants (one warp per block, or 2..8 kept in step) */
+static int fb_slim_attributes(FbHandle *h) {
+  const FbKernelSel one = fb_kernel_sel(h, FB_FAST, 32, 1);
+  int fit = h->max_smem/(int)one.bytes;     /* warps of one block that fit an SM's shared memory */
+  if (fit > 8) fit = 8;
+  FbKernelSel multi = fb_kernel_sel(h, FB_FAST, 32, 1, 2);
+  multi.bytes = (fit >= 2 ? fit : 1)*one.bytes;
+  cudaError_t ce = fb_kernel_attributes(one);
+  if (ce == cudaSuccess) ce = fb_kernel_attributes(multi);
+  if (ce != cudaSuccess) return fail(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ce));
+  if (h->fast_wpb > fit) h->fast_wpb = fit;
+  if (h->fast_wpb < 2) h->fast_wpb = 1;
+  return 0;
+}
+#endif
+
+/* What one launch runs */
+struct FbPlan {
+  bool fast;            /* the unconstrained per-thread kernel `uncon` runs first; else the team kernel alone */
+  FbKernelSel uncon;
+  bool con_thread;      /* its hand-overs go to the per-thread constrained kernel `con`; else to the team kernel */
+  bool con_split;       /* ... with the constrained SPLIT variant `csplit` launched in front */
+  FbKernelSel con, csplit;
+  int team_grid;        /* blocks of the team kernel (FbHandle::threads threads, smem_bytes bytes) */
+};
+
+/* The kernels a launch of `mode` runs.  The per-thread kernel advances every environment while it
+ * is unconstrained; the constrained kernel or the team kernel finishes the ones it handed over.
+ * Reset and derived-view requests go to the team kernel alone (it is the one that produces
+ * mjData-like quantities).  The fb_* queries of the kernel selection read the plan of the next
+ * fb_step. */
+static FbPlan fb_plan(const FbHandle *h, int mode, int want_derived, bool ctrl_seq) {
+  const DevModel &m = h->hm.m;
+  const FbEnvTables &ep = h->ep;
+  const int nw = h->hm.split.nwarps;
+  FbPlan p = {};
+  p.team_grid = (h->P.n_envs + h->envs_per_block - 1)/h->envs_per_block;
+  p.fast = h->fast_enabled && m.X.ok && mode == FB_MODE_STEP && !want_derived;
+  if (!p.fast) return p;
+  /* LEAN: the same arithmetic with the model's unused paths compiled out; a control sequence needs
+   * the general variant */
+  const int lean = h->fast_lean && m.X.lean && !ctrl_seq;
+  /* ENVP while a per-environment parameter table the kernel reads is set (the unconstrained kernels
+   * never read the candidate friction), or the episode clock is bound: only while the wave
+   * controller, the one step code that reads time, is on and some episode began after iteration 0 */
+  const int envp = ep.stiffness || ep.damping || ep.coef || ep.wvel || (m.n_wc > 0 && h->episode_late);
+  const int cenvp = envp || ep.fric;
+#ifdef FB_HOST_EMU
+  /* The emulation steps one environment at a time (BLK = 1; a constrained group is one
+   * environment, so emu_per_thread gives the constrained SPLIT variant each handed-over environment
+   * that has not stepped yet) and has no occupancy or cost model: the SPLIT variants run whenever
+   * they are enabled and the model's tree splits. */
+  const int blk = 1;
+  const bool split = h->fast_split && !h->fast_slim && nw > 1;
+  const bool con_split = h->con_split && !h->fast_slim && nw > 1;
+#else
+  const int blk = h->fast_block;
+  const bool split = h->fast_split && !h->fast_slim && nw > 1 && blk == 32 && (h->P.n_envs + 31)/32 <= h->split_capacity;
+  const bool con_split = h->con_split && !h->fast_slim && nw > 1 && fb_con_split_pays(h);
+#endif
+  if (split) {
+    /* small batch: the tree of every 32 environments split over several warps */
+    p.uncon = fb_kernel_sel(h, FB_FAST_SPLIT, blk);
+  } else if (h->fast_slim && blk != 16) {
+    /* multi-warp blocks: SLIM layout only (measured 3-5 % slower on the regular one) */
+    p.uncon = fb_kernel_sel(h, FB_FAST, blk, 1, h->fast_wpb >= 2 && h->fast_wpb <= 8 ? h->fast_wpb : 1);
+  } else {
+    p.uncon = fb_kernel_sel(h, FB_FAST, blk);
+  }
+  p.uncon.lean = lean; p.uncon.envp = envp;
+  p.con_thread = h->con_thread && m.X.con_ok;
+  if (p.con_thread) {
+    p.con = fb_kernel_sel(h, FB_FASTC, blk);
+    p.con.lean = lean; p.con.envp = cenvp;
+    /* small ground-contact batch: the tree of every group split over several warps */
+    p.con_split = con_split;
+    p.csplit = fb_kernel_sel(h, FB_FASTC_SPLIT, blk);
+    p.csplit.lean = lean; p.csplit.envp = cenvp;
+  }
+  return p;
+}
+
+/* the plan of the next fb_step */
+static FbPlan fb_next_step(const FbHandle *h) { return fb_plan(h, FB_MODE_STEP, 0, h->cpg_on || h->seq_len > 0); }
+
 #ifdef FB_HOST_EMU
 /* test harness: the warps of a SPLIT block as host threads meeting at FB_BLOCK_BARRIER */
 template <class F> static void emu_split_run(int nw, F body) {
@@ -672,79 +861,76 @@ template <class F> static void emu_split_run(int nw, F body) {
   fb_emu_bar = nullptr;
   pthread_barrier_destroy(&bar);
 }
-#endif
 
-#ifdef FB_HOST_EMU
-/* test harness: the per-thread kernels run serially on the host (ENVP: the unconstrained kernels'
- * twins, CENVP: the constrained kernels') */
-template <int ENVP, int CENVP> static void emu_per_thread(FbHandle *h, FbParams &P, int n_steps, int con_thread) {
+/* test harness: the body of the per-thread kernel `k` for one environment with BLK = 1; returns the
+ * steps an unconstrained kernel completed */
+static int emu_run(FbHandle *h, const FbParams &P, const FbKernelSel &k, int env, float *fs, float *fg, float *fc) {
+  const FastSplit &sp = h->hm.split;
+  const FastRec *rec = h->hm.rec.data();
+  const CandRec *crec = h->hm.crec.data();
+  int done = 0;
+  fb_dispatch(k, [&](auto v) {
+    using V = decltype(v);
+    const FbEnvTables *T = V::envp ? &h->ep : nullptr;
+    std::vector<float> extra(V::kind == FB_FAST_SPLIT || V::kind == FB_FASTC_SPLIT ? FB_CSPLIT_EXTRA : 0, 0.f);   /* one lane */
+    if constexpr (V::kind == FB_FAST) {
+      FbFast<1, V::slim, V::lean, 0, V::envp> st(P, rec, fs, fg, env, T);
+      done = st.run(0, 0);
+    } else if constexpr (V::kind == FB_FAST_SPLIT) {
+      emu_split_run(sp.nwarps, [&](int role) {
+        FbFast<1, 0, V::lean, 1, V::envp> st(P, rec, fs, fg, env, T);
+        st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
+        const int d = st.run_split(0, 0, 1);
+        if (role == 0) done = d;
+      });
+    } else if constexpr (V::kind == FB_FASTC) {
+      FbFastCon<1, V::lean, 0, V::envp> st(P, rec, crec, fs, fg, fc, env, T);
+      st.run_con(P.steps_done[env], 0, 0);
+    } else {
+      emu_split_run(sp.nwarps, [&](int role) {
+        FbFastCon<1, V::lean, 1, V::envp> st(P, rec, crec, fs, fg, fc, env, T);
+        st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
+        st.con_split_setup(sp, extra.data() + 4);
+        st.run_con_split(0, 0);
+      });
+    }
+  });
+  return done;
+}
+
+/* test harness: the per-thread kernels of the plan run serially on the host */
+static void emu_per_thread(FbHandle *h, FbParams &P, int n_steps, const FbPlan &plan) {
   const DevModel &m = P.m;
-  const FbEnvTables *T = ENVP ? &h->ep : nullptr, *CT = CENVP ? &h->ep : nullptr;
   P.pending_count[P.parity ^ 1] = 0;
   std::vector<float> fs((size_t)m.X.n_float + 8, 0.f);
   std::vector<float> fg((size_t)(m.X.n_scratch > m.X.n_scratch_slim ? m.X.n_scratch : m.X.n_scratch_slim) + 8, 0.f);
-  const FastSplit &sp = h->hm.split;
-  const int n_extra = 4 + 2*FB_SPLIT_MAXW*FB_RED_MAX;      /* root position, flag, reduction buffers (one lane) */
+  std::vector<float> fc((size_t)m.X.n_con + 8, 0.f);
   for (int env = 0; env < P.n_envs; env++) {
-    int done;
-    const bool lean = h->fast_lean && m.X.lean && !P.ctrl_seq;
-    if (h->fast_split && !h->fast_slim && sp.nwarps > 1) {
-      /* SPLIT variant: the warps of the block are host threads */
-      std::vector<float> extra(n_extra, 0.f);
-      int done0 = 0;
-      emu_split_run(sp.nwarps, [&](int role) {
-        int d;
-        if (lean) {
-          FbFast<1, 0, 1, 1, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T);
-          st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
-          d = st.run_split(0, 0, 1);
-        } else {
-          FbFast<1, 0, 0, 1, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T);
-          st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
-          d = st.run_split(0, 0, 1);
-        }
-        if (role == 0) done0 = d;
-      });
-      done = done0;
-    } else
-    if (h->fast_slim && lean) { FbFast<1, 1, 1, 0, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T); done = st.run(0, 0); }
-    else if (h->fast_slim) { FbFast<1, 1, 0, 0, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T); done = st.run(0, 0); }
-    else if (lean) { FbFast<1, 0, 1, 0, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T); done = st.run(0, 0); }
-    else { FbFast<1, 0, 0, 0, ENVP> st(P, h->hm.rec.data(), fs.data(), fg.data(), env, T); done = st.run(0, 0); }
+    const int done = emu_run(h, P, plan.uncon, env, fs.data(), fg.data(), fc.data());
     if (done < n_steps) { P.steps_done[env] = done; P.pending[P.pending_count[P.parity]++] = env; }
   }
-  if (con_thread) {
-    std::vector<float> fc((size_t)m.X.n_con + 8, 0.f);
-    for (int i = 0; i < P.pending_count[P.parity]; i++) {
-      const int env = P.pending[i];
-      if (h->con_split && !h->fast_slim && sp.nwarps > 1 && P.steps_done[env] == 0) {
-        /* SPLIT variant of the constrained kernel (a group = this environment) */
-        std::vector<float> extra(n_extra, 0.f);
-        const bool lean = h->fast_lean && m.X.lean && !P.ctrl_seq;
-        emu_split_run(sp.nwarps, [&](int role) {
-          if (lean) {
-            FbFastCon<1, 1, 1, CENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, CT);
-            st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
-            st.con_split_setup(sp, extra.data() + 4);
-            st.run_con_split(0, 0);
-          } else {
-            FbFastCon<1, 0, 1, CENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, CT);
-            st.split_setup(sp, role, extra.data(), reinterpret_cast<int *>(extra.data() + 3));
-            st.con_split_setup(sp, extra.data() + 4);
-            st.run_con_split(0, 0);
-          }
-        });
-        continue;
-      }
-      if (h->fast_lean && m.X.lean && !P.ctrl_seq) {
-        FbFastCon<1, 1, 0, CENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, CT);
-        st.run_con(P.steps_done[env], 0, 0);
-      } else {
-        FbFastCon<1, 0, 0, CENVP> st(P, h->hm.rec.data(), h->hm.crec.data(), fs.data(), fg.data(), fc.data(), env, CT);
-        st.run_con(P.steps_done[env], 0, 0);
-      }
-    }
+  if (!plan.con_thread) return;
+  for (int i = 0; i < P.pending_count[P.parity]; i++) {
+    const int env = P.pending[i];
+    emu_run(h, P, plan.con_split && P.steps_done[env] == 0 ? plan.csplit : plan.con, env, fs.data(), fg.data(), fc.data());
   }
+}
+#else
+template <class Q> static auto &fb_staging(FbHandle *h) {
+  if constexpr (std::is_base_of_v<FbFastParams, Q>) return *h->fastQ;
+  else if constexpr (std::is_base_of_v<FbFastSplitParams, Q>) return *h->splitQ;
+  else if constexpr (std::is_base_of_v<FbFastConParams, Q>) return *h->conQ;
+  else return *h->csplitQ;
+}
+template <class Q> static void fb_launch_kernel(FbHandle *h, const FbKernelSel &k, void (*kernel)(Q)) {
+  auto &S = fb_staging<Q>(h);
+  S.P = h->P; S.T = h->ep;
+  kernel<<<k.grid, k.threads, k.bytes, h->stream>>>(static_cast<const Q &>(S));
+}
+/* launch the per-thread kernel `k` with the handle's parameters and tables */
+static void fb_launch(FbHandle *h, const FbKernelSel &k) {
+  fb_dispatch(k, [&](auto v) { fb_launch_kernel(h, k, fb_kernel_of(v)); });
+  h->launches++;
 }
 #endif
 
@@ -752,9 +938,6 @@ template <int ENVP, int CENVP> static void emu_per_thread(FbHandle *h, FbParams 
 static int launch(FbHandle *h, int mode, int n_steps, int want_derived, const uint8_t *only = nullptr) {
   FbParams &P = h->P;
   P.mode = mode; P.n_steps = n_steps; P.want_derived = want_derived; P.it0 = h->it;
-  /* The per-thread kernel advances every environment while it is unconstrained; the
-   * team kernel finishes the ones it handed over.  Reset and derived-view requests go
-   * to the team kernel alone (it is the one that produces mjData-like quantities). */
   P.ctrl_seq = nullptr; P.seq_pos = 0;
   P.seq_stride = h->hm.m.nu; P.n_spring = 0; P.spring_qadr = nullptr;
   if (mode == FB_MODE_STEP && h->cpg_on) {
@@ -777,36 +960,25 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived, const ui
     h->seq_pos += n_steps;
     if (h->seq_pos == h->seq_len) h->seq_len = h->seq_pos = 0;     /* consumed: ctrl is held again */
   }
-  const int use_fast = h->fast_enabled && P.m.X.ok && mode == FB_MODE_STEP && !want_derived;
-  /* the per-thread kernels' ENVP twins while a per-environment parameter table they read is set (the
-   * unconstrained kernels never read the candidate friction), or the episode clock is bound: only
-   * while the wave controller, the one step code that reads time, is on and some episode began
-   * after iteration 0 */
+  const FbPlan plan = fb_plan(h, mode, want_derived, P.ctrl_seq != nullptr);
   h->ep.episode_start = P.m.n_wc > 0 && h->episode_late ? h->episode_start : nullptr;
-  const bool envp = h->ep.stiffness || h->ep.damping || h->ep.coef || h->ep.wvel || h->ep.episode_start;
-  const bool cenvp = envp || h->ep.fric;
-  const int con_thread = use_fast && h->con_thread && P.m.X.con_ok;
-  P.use_pending = use_fast;
+  P.use_pending = plan.fast;
   P.parity = (int)(h->launch_parity & 1);
-  if (use_fast) h->launch_parity++;
+  if (plan.fast) h->launch_parity++;
 #ifdef FB_HOST_EMU
   const DevModel &m = P.m;
-  if (use_fast) {
-    if (envp) emu_per_thread<1, 1>(h, P, n_steps, con_thread);
-    else if (cenvp) emu_per_thread<0, 1>(h, P, n_steps, con_thread);
-    else emu_per_thread<0, 0>(h, P, n_steps, con_thread);
-  }
+  if (plan.fast) emu_per_thread(h, P, n_steps, plan);
   std::vector<float> s((size_t)m.L.n_float + 8, 0.f);
   std::vector<int> si((size_t)m.L.n_int + 8, 0);
-  const int count = use_fast ? (con_thread ? 0 : P.pending_count[P.parity]) : P.n_envs;
+  const int count = plan.fast ? (plan.con_thread ? 0 : P.pending_count[P.parity]) : P.n_envs;
   for (int i = 0; i < count; i++) {
-    int env = use_fast ? P.pending[i] : i;
+    int env = plan.fast ? P.pending[i] : i;
     if (only && !only[env]) continue;
-    fb_run_env<1>(P, h->ep, env, use_fast ? P.steps_done[env] : 0, s.data(), si.data(), 0, 0, 1u);
+    fb_run_env<1>(P, h->ep, env, plan.fast ? P.steps_done[env] : 0, s.data(), si.data(), 0, 0, 1u);
   }
   h->last_ms = 0.f;
+  h->launches++;
 #else
-  int blocks = (P.n_envs + h->envs_per_block - 1)/h->envs_per_block;
   if (h->host_calls > 0) {
     /* fb_step_host's row gathers run on the gather stream, in call order.  This launch overwrites
      * the ring rows of iterations it+1 .. it+n_steps, i.e. what iterations <= it+n_steps-ring left
@@ -822,71 +994,17 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived, const ui
     if (dep >= 0 && cudaStreamWaitEvent(h->stream, h->ev_gathered[dep & 3], 0) != cudaSuccess) return fail(dev_error());
   }
   cudaEventRecord(h->ev0, h->stream);
-  if (use_fast) {
-    int fblocks = (P.n_envs + h->fast_block - 1)/h->fast_block;
-    h->fastQ->P = P; h->fastQ->T = h->ep;
-    {
-      int wpb = h->fast_block == 32 ? h->fast_wpb : 1;
-      if (!h->fast_slim || wpb < 2 || wpb > 8) wpb = 1;      /* multi-warp blocks: SLIM layout only (measured 3-5 % slower on the regular one) */
-      const int warps = (P.n_envs + 31)/32;
-      const int wblocks = (warps + wpb - 1)/wpb;
-      size_t bytes = (h->fast_slim ? h->fast_slim_smem_bytes : h->fast_smem_bytes)*(h->fast_block == 32 ? wpb : 1);
-      /* LEAN variants: same arithmetic with the model's unused paths compiled out (smaller loops) */
-      const bool lean = h->fast_lean && P.m.X.lean && !P.ctrl_seq;
-      if (h->fast_split && h->fast_block == 32 && !h->fast_slim && h->hm.split.nwarps > 1 && warps <= h->split_capacity) {
-        /* small batch: the tree of every 32 environments split over several warps */
-        h->splitQ->P = P; h->splitQ->T = h->ep;
-        const size_t sbytes = h->fast_smem_bytes + FB_SPLIT_EXTRA_BYTES;
-        const int threads = 32*h->hm.split.nwarps;
-        if (lean) fb_launch_fast_split<1>(envp, warps, threads, sbytes, h->stream, *h->splitQ);
-        else fb_launch_fast_split<0>(envp, warps, threads, sbytes, h->stream, *h->splitQ);
-      } else if (h->fast_block == 16) {
-        if (lean) fb_launch_fast<16, 0, 0, 1>(envp, fblocks, 16, bytes, h->stream, *h->fastQ);
-        else fb_launch_fast<16, 0, 0, 0>(envp, fblocks, 16, bytes, h->stream, *h->fastQ);
-      } else if (h->fast_slim && wpb > 1) {
-        if (lean) fb_launch_fast<32, 1, 1, 1>(envp, wblocks, 32*wpb, bytes, h->stream, *h->fastQ);
-        else fb_launch_fast<32, 1, 1, 0>(envp, wblocks, 32*wpb, bytes, h->stream, *h->fastQ);
-      } else if (h->fast_slim) {
-        if (lean) fb_launch_fast<32, 1, 0, 1>(envp, warps, 32, bytes, h->stream, *h->fastQ);
-        else fb_launch_fast<32, 1, 0, 0>(envp, warps, 32, bytes, h->stream, *h->fastQ);
-      } else {
-        if (lean) fb_launch_fast<32, 0, 0, 1>(envp, warps, 32, bytes, h->stream, *h->fastQ);
-        else fb_launch_fast<32, 0, 0, 0>(envp, warps, 32, bytes, h->stream, *h->fastQ);
-      }
-    }
-    h->launches++;
-    if (con_thread) {
-      const bool clean = h->fast_lean && P.m.X.lean && !P.ctrl_seq;
-      P.con_split_done = nullptr;
-      if (h->con_split && P.use_pending && !h->fast_slim && h->hm.split.nwarps > 1 && fb_con_split_pays(h)) {
-        /* small ground-contact batch: the tree of every group split over several warps */
-        P.con_split_done = h->con_split_done;
-        h->csplitQ->P = P; h->csplitQ->T = h->ep;
-        const size_t sbytes = h->fast_smem_bytes + (size_t)FB_CSPLIT_EXTRA*h->fast_block*sizeof(float);
-        const int threads = 32*h->hm.split.nwarps;
-        if (h->fast_block == 16) {
-          if (clean) fb_launch_fastc_split<16, 1>(cenvp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
-          else fb_launch_fastc_split<16, 0>(cenvp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
-        } else {
-          if (clean) fb_launch_fastc_split<32, 1>(cenvp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
-          else fb_launch_fastc_split<32, 0>(cenvp, fblocks, threads, sbytes, h->stream, *h->csplitQ);
-        }
-        h->launches++;
-      }
-      h->conQ->P = P; h->conQ->T = h->ep;
-      if (h->fast_block == 16) {
-        if (clean) fb_launch_fastc<16, 1>(cenvp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
-        else fb_launch_fastc<16, 0>(cenvp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
-      } else {
-        if (clean) fb_launch_fastc<32, 1>(cenvp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
-        else fb_launch_fastc<32, 0>(cenvp, fblocks, h->fast_smem_bytes, h->stream, *h->conQ);
-      }
+  if (plan.fast) {
+    fb_launch(h, plan.uncon);
+    if (plan.con_thread) {
+      P.con_split_done = plan.con_split ? h->con_split_done : nullptr;
+      if (plan.con_split) fb_launch(h, plan.csplit);
+      fb_launch(h, plan.con);
     }
   }
-  if (!con_thread) switch (h->team) {
-    case 8: fb_step_kernel<8><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep, only); break;
-    case 16: fb_step_kernel<16><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep, only); break;
-    default: fb_step_kernel<32><<<blocks, h->threads, h->smem_bytes, h->stream>>>(P, h->ep, only); break;
+  if (!plan.con_thread) {
+    fb_team_kernel(h->team)<<<plan.team_grid, h->threads, h->smem_bytes, h->stream>>>(P, h->ep, only);
+    h->launches++;
   }
   cudaEventRecord(h->ev1, h->stream);
   {
@@ -894,7 +1012,6 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived, const ui
     if (le != cudaSuccess) return fail(std::string("kernel launch failed: ") + cudaGetErrorString(le));
   }
 #endif
-  h->launches++;
   if (mode == FB_MODE_STEP) h->it += n_steps;       /* fb_reset set it to 0 before, fb_reset_envs keeps it */
 #ifndef FB_HOST_EMU
   /* Half-filled warps (16 environments each) pay for candidate-rich models only through the
@@ -904,12 +1021,12 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived, const ui
    * the unconstrained kernel at every batch size (r2l: 1.14e8 against 1.08e8 env-steps/s at 8,192
    * SALAMANDERs); ground-contact batches keep 16 (7.46e6 against 7.24e6 at 4,096).  The scratch
    * layouts depend on the block size but hold nothing across launches. */
-  if (use_fast && h->block_review) {
+  if (plan.fast && h->block_review) {
     h->block_review = 0;
     int both[2] = {0, 0};
     if (d2h(both, P.pending_count, sizeof(both), h->stream) || dev_sync(h->stream)) return fail(dev_error());
     int want = 2*both[P.parity] >= P.n_envs ? 16 : 32;
-    if (want == 16 && con_thread && h->con_split && h->hm.split.nwarps > 1) {
+    if (want == 16 && plan.con_thread && h->con_split && h->hm.split.nwarps > 1) {
       /* with the constrained SPLIT variant a group is several warps: 16 per group pays only while
        * every group has an SM to itself (r2x, SALAMANDER ground: 1,024 envs 3.47e6 against 3.31e6
        * env-steps/s with 32; 4,096 envs 1.09e7 against 1.29e7); beyond that, whichever group size
@@ -924,126 +1041,6 @@ static int launch(FbHandle *h, int mode, int n_steps, int want_derived, const ui
 #endif
   return 0;
 }
-
-#ifndef FB_HOST_EMU
-/* blocks of the constrained SPLIT variant the device holds at once with `blk` environments per group
- * (0: not applicable); sets the kernels' shared-memory attributes on the way */
-static long long fb_con_split_blocks(FbHandle *h, int blk, cudaError_t *ce) {
-  const size_t sbytes = ((size_t)h->hm.m.X.n_float + FB_CSPLIT_EXTRA)*blk*sizeof(float);
-  if (!h->hm.m.X.con_ok || h->hm.split.nwarps < 2 || sbytes > (size_t)h->max_smem) return 0;
-  int per_sm = 1 << 30;
-  for (int v = 0; v < 4 && *ce == cudaSuccess; v++) {      /* LEAN x ENVP */
-    const void *k16[4] = {(const void *)fb_fastc_split_kernel<16, 0>, (const void *)fb_fastc_split_kernel<16, 1>,
-                          (const void *)fb_fastc_split_envp_kernel<16, 0>, (const void *)fb_fastc_split_envp_kernel<16, 1>};
-    const void *k32[4] = {(const void *)fb_fastc_split_kernel<32, 0>, (const void *)fb_fastc_split_kernel<32, 1>,
-                          (const void *)fb_fastc_split_envp_kernel<32, 0>, (const void *)fb_fastc_split_envp_kernel<32, 1>};
-    const void *k = blk == 16 ? k16[v] : k32[v];
-    *ce = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
-    if (*ce == cudaSuccess) *ce = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    int nb = 0;
-    if (*ce == cudaSuccess) *ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k, 32*h->hm.split.nwarps, sbytes);
-    if (nb < per_sm) per_sm = nb;
-  }
-  return *ce == cudaSuccess ? (long long)per_sm*h->sms : 0;
-}
-
-/* blocks (= warps) of the single-warp constrained kernel the device holds at once */
-static long long fb_con_single_blocks(FbHandle *h, int blk, cudaError_t *ce) {
-  const size_t sbytes = (size_t)h->hm.m.X.n_float*blk*sizeof(float);
-  if (!h->hm.m.X.con_ok || sbytes > (size_t)h->max_smem) return 0;
-  int per_sm = 1 << 30;
-  for (int v = 0; v < 4 && *ce == cudaSuccess; v++) {      /* LEAN x ENVP */
-    const void *k16[4] = {(const void *)fb_fastc_kernel<16, 0>, (const void *)fb_fastc_kernel<16, 1>,
-                          (const void *)fb_fastc_envp_kernel<16, 0>, (const void *)fb_fastc_envp_kernel<16, 1>};
-    const void *k32[4] = {(const void *)fb_fastc_kernel<32, 0>, (const void *)fb_fastc_kernel<32, 1>,
-                          (const void *)fb_fastc_envp_kernel<32, 0>, (const void *)fb_fastc_envp_kernel<32, 1>};
-    const void *k = blk == 16 ? k16[v] : k32[v];
-    *ce = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sbytes);
-    if (*ce == cudaSuccess) *ce = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    int nb = 0;
-    if (*ce == cudaSuccess) *ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k, blk, sbytes);
-    if (nb < per_sm) per_sm = nb;
-  }
-  return *ce == cudaSuccess ? (long long)per_sm*h->sms : 0;
-}
-
-/* A ground-contact launch is as long as one group's step sequence times the number of waves its
- * blocks take: the SPLIT variant shortens the sequence (x FB_CSPLIT_GAIN, measured r2y: 1.7 .. 2.0
- * faster per wave) and holds fewer groups per wave.  Cost of stepping n_envs environments in
- * groups of blk, in units of a single-warp wave x 100; 0 = not available. */
-#define FB_CSPLIT_GAIN 55
-static long long fb_con_cost(long long n_envs, int blk, long long capacity, int split) {
-  if (capacity <= 0) return 0;
-  const long long groups = (n_envs + blk - 1)/blk, waves = (groups + capacity - 1)/capacity;
-  return waves*(split ? FB_CSPLIT_GAIN : 100);
-}
-static bool fb_con_split_pays(FbHandle *h) {
-  const long long cs = fb_con_cost(h->P.n_envs, h->fast_block, h->con_split_capacity, 1);
-  const long long c1 = fb_con_cost(h->P.n_envs, h->fast_block, h->con_single_capacity, 0);
-  return cs > 0 && (c1 == 0 || cs < c1);
-}
-
-/* environments per warp of the per-thread kernels (regular layout): shared-memory attributes */
-static int fb_set_fast_block(FbHandle *h, int blk) {
-  const size_t per_thread = (size_t)h->hm.m.X.n_float*sizeof(float);
-  h->fast_block = blk;
-  h->fast_smem_bytes = per_thread*blk;
-  const int bytes = (int)h->fast_smem_bytes;
-  cudaError_t ce = cudaSuccess;
-#define FB_SET_SMEM(K_) \
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(K_, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes); \
-  if (ce == cudaSuccess) ce = cudaFuncSetAttribute(K_, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  switch (blk) {
-    case 16: FB_SET_SMEM((fb_fast_kernel<16, 0, 0>)) FB_SET_SMEM((fb_fast_kernel<16, 0, 0, 1>)) FB_SET_SMEM(fb_fastc_kernel<16>) FB_SET_SMEM((fb_fastc_kernel<16, 1>))
-             FB_SET_SMEM((fb_fast_envp_kernel<16, 0, 0>)) FB_SET_SMEM((fb_fast_envp_kernel<16, 0, 0, 1>)) FB_SET_SMEM(fb_fastc_envp_kernel<16>) FB_SET_SMEM((fb_fastc_envp_kernel<16, 1>)) break;
-    default: FB_SET_SMEM((fb_fast_kernel<32, 0, 0>)) FB_SET_SMEM((fb_fast_kernel<32, 0, 0, 1>)) FB_SET_SMEM(fb_fastc_kernel<32>) FB_SET_SMEM((fb_fastc_kernel<32, 1>))
-             FB_SET_SMEM((fb_fast_envp_kernel<32, 0, 0>)) FB_SET_SMEM((fb_fast_envp_kernel<32, 0, 0, 1>)) FB_SET_SMEM(fb_fastc_envp_kernel<32>) FB_SET_SMEM((fb_fastc_envp_kernel<32, 1>)) break;
-  }
-#undef FB_SET_SMEM
-  h->split_capacity = 0;
-  if (blk == 32 && h->hm.split.nwarps > 1 && (size_t)bytes + FB_SPLIT_EXTRA_BYTES <= (size_t)h->max_smem) {
-    int per_sm = 1 << 30;
-    for (int v = 0; v < 4 && ce == cudaSuccess; v++) {      /* LEAN x ENVP */
-      const void *split_k[4] = {(const void *)fb_fast_split_kernel<0>, (const void *)fb_fast_split_kernel<1>,
-                                (const void *)fb_fast_split_envp_kernel<0>, (const void *)fb_fast_split_envp_kernel<1>};
-      const void *k = split_k[v];
-      ce = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes + FB_SPLIT_EXTRA_BYTES);
-      if (ce == cudaSuccess) ce = cudaFuncSetAttribute(k, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-      int nb = 0;
-      if (ce == cudaSuccess) ce = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k, 32*h->hm.split.nwarps, (size_t)bytes + FB_SPLIT_EXTRA_BYTES);
-      if (nb < per_sm) per_sm = nb;
-    }
-    /* the SPLIT variant pays while ALL its blocks are resident at once (one wave) */
-    if (ce == cudaSuccess) h->split_capacity = (long long)per_sm*h->sms;
-  }
-  if (ce == cudaSuccess) h->con_split_capacity = fb_con_split_blocks(h, blk, &ce);
-  if (ce == cudaSuccess) h->con_single_capacity = fb_con_single_blocks(h, blk, &ce);
-  return ce == cudaSuccess ? 0 : fail(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ce));
-}
-
-/* shared-memory attributes of the SLIM variants (one warp per block, or 2..8 kept in step) */
-static int fb_slim_attributes(FbHandle *h, int max_smem) {
-  h->fast_slim_smem_bytes = (size_t)h->hm.m.X.n_float_slim*sizeof(float)*32;
-  const int b1 = (int)h->fast_slim_smem_bytes;
-  int fit = max_smem/b1;     /* warps of one block that fit an SM's shared memory */
-  if (fit > 8) fit = 8;
-  const void *one[4] = {(const void *)fb_fast_kernel<32, 1, 0>, (const void *)fb_fast_kernel<32, 1, 0, 1>,
-                        (const void *)fb_fast_envp_kernel<32, 1, 0>, (const void *)fb_fast_envp_kernel<32, 1, 0, 1>};
-  const void *multi[4] = {(const void *)fb_fast_kernel<32, 1, 1>, (const void *)fb_fast_kernel<32, 1, 1, 1>,
-                          (const void *)fb_fast_envp_kernel<32, 1, 1>, (const void *)fb_fast_envp_kernel<32, 1, 1, 1>};
-  cudaError_t ce = cudaSuccess;
-  for (int v = 0; v < 4; v++) {      /* LEAN x ENVP */
-    if (ce == cudaSuccess) ce = cudaFuncSetAttribute(one[v], cudaFuncAttributeMaxDynamicSharedMemorySize, b1);
-    if (ce == cudaSuccess) ce = cudaFuncSetAttribute(one[v], cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-    if (ce == cudaSuccess && fit >= 2) ce = cudaFuncSetAttribute(multi[v], cudaFuncAttributeMaxDynamicSharedMemorySize, fit*b1);
-    if (ce == cudaSuccess) ce = cudaFuncSetAttribute(multi[v], cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
-  }
-  if (ce != cudaSuccess) return fail(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ce));
-  if (h->fast_wpb > fit) h->fast_wpb = fit;
-  if (h->fast_wpb < 2) h->fast_wpb = 1;
-  return 0;
-}
-#endif
 
 #ifndef FB_HOST_EMU
 /* FP32 roof of the device as this path could use it at best: every lane of every scheduler issuing
@@ -1130,10 +1127,10 @@ int fb_create(const FbModel *model, const FbFarms *farms, int n_envs, int device
   h->reset_mask = nullptr; h->reset_list = h->reset_row = nullptr; h->reset_q = h->reset_v = nullptr;
   h->joint_sel_n = 0; h->link_sel_n = 0; h->link_items_n = 0; h->ctrl_sel_n = 0;
   h->export_stage[0] = h->export_stage[1] = nullptr; h->export_stage_floats = 0;
-  h->fast_enabled = 1; h->fast_block = 1; h->fast_smem_bytes = 0; h->launch_parity = 0;
+  h->fast_enabled = 1; h->fast_block = 1; h->launch_parity = 0;
   h->con_thread = 1; h->log_used = 0;
   if (const char *ev = getenv("FARMS_B200_CON_THREAD")) h->con_thread = atoi(ev) != 0;
-  h->fast_slim = 0; h->fast_slim_smem_bytes = 0; h->fast_wpb = 1;
+  h->fast_slim = 0; h->fast_wpb = 1;
   h->fast_lean = 1; h->fast_block_auto = false; h->block_review = 0; h->max_smem = 0; h->fast_split = 0;
   h->split_capacity = 0; h->con_split = 0; h->con_split_capacity = 0; h->con_single_capacity = 0; h->con_split_done = nullptr;
   if (const char *ev = getenv("FARMS_B200_FAST_LEAN")) h->fast_lean = atoi(ev) != 0;
@@ -1204,12 +1201,7 @@ int fb_create(const FbModel *model, const FbFarms *farms, int n_envs, int device
   h->envs_per_block = epb;
   h->threads = epb*h->team;
   h->smem_bytes = per_env*epb;
-  cudaError_t ce = cudaSuccess;
-  switch (h->team) {
-    case 8: ce = cudaFuncSetAttribute(fb_step_kernel<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes); break;
-    case 16: ce = cudaFuncSetAttribute(fb_step_kernel<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes); break;
-    default: ce = cudaFuncSetAttribute(fb_step_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes); break;
-  }
+  const cudaError_t ce = cudaFuncSetAttribute((const void *)fb_team_kernel(h->team), cudaFuncAttributeMaxDynamicSharedMemorySize, (int)h->smem_bytes);
   if (ce != cudaSuccess) { fb_destroy(h); return fail(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ce)); }
   /* environment-per-thread kernels: one warp per block, as many blocks per SM as their
    * shared-memory working sets allow; models beyond that run on the team kernel.  A warp holds 32
@@ -1247,7 +1239,7 @@ int fb_create(const FbModel *model, const FbFarms *farms, int n_envs, int device
         h->fast_wpb = (warps + sms*rounds - 1)/(sms*rounds);
         if (h->fast_wpb < 4) h->fast_wpb = 4;
       }
-      if (h->fast_slim && fb_slim_attributes(h, max_smem)) { fb_destroy(h); return -1; }
+      if (h->fast_slim && fb_slim_attributes(h)) { fb_destroy(h); return -1; }
       /* SPLIT variant: pays while the batch leaves schedulers idle (a launch is then one warp's
        * latency, which the split shortens); beyond ~2 warps per scheduler the single-warp kernel
        * does the same work with fewer instructions */
@@ -1255,7 +1247,6 @@ int fb_create(const FbModel *model, const FbFarms *farms, int n_envs, int device
       if (const char *ev = getenv("FARMS_B200_FAST_SPLIT")) h->fast_split = atoi(ev) != 0;
       h->con_split = !h->fast_slim && h->hm.split.nwarps > 1 && m.X.con_ok;
       if (const char *ev = getenv("FARMS_B200_CON_SPLIT")) h->con_split = atoi(ev) != 0;
-      if (ce != cudaSuccess) { fb_destroy(h); return fail(std::string("cudaFuncSetAttribute: ") + cudaGetErrorString(ce)); }
     }
   }
 #else
@@ -2280,19 +2271,21 @@ int fb_set_constraint_path(FbHandle *h, int per_thread) {
   h->con_thread = per_thread != 0;
   return 0;
 }
-int fb_constraint_path(FbHandle *h) { return h && h->fast_enabled && h->hm.m.X.con_ok ? h->con_thread : 0; }
+int fb_constraint_path(FbHandle *h) { return h && fb_next_step(h).con_thread ? 1 : 0; }
 /* 0: team kernel only; otherwise the environments per block of the per-thread kernel */
 int fb_fast_path(FbHandle *h) {
   if (!h) return 0;
-  return h->fast_enabled && h->hm.m.X.ok ? h->fast_block : 0;
+  const FbPlan p = fb_next_step(h);
+  return p.fast ? p.uncon.blk : 0;
 }
 int fb_fast_smem_bytes_per_env(FbHandle *h) {
   return h ? (int)((h->fast_slim ? h->hm.m.X.n_float_slim : h->hm.m.X.n_float)*sizeof(float)) : 0;
 }
 /* 0: regular layout; else the warps per block of the large-batch (SLIM) layout (1 .. 8) */
 int fb_fast_slim(FbHandle *h) {
-  if (!h || !h->fast_enabled || !h->hm.m.X.ok || !h->fast_slim) return 0;
-  return h->fast_wpb >= 2 && h->fast_wpb <= 8 ? h->fast_wpb : 1;
+  if (!h) return 0;
+  const FbPlan p = fb_next_step(h);
+  return p.fast && p.uncon.slim ? p.uncon.threads/32 : 0;
 }
 int fb_set_fast_slim(FbHandle *h, int enable) {
   if (!h) return fail("null handle");
@@ -2300,11 +2293,7 @@ int fb_set_fast_slim(FbHandle *h, int enable) {
   h->fast_wpb = enable > 1 ? enable : 1;
 #ifndef FB_HOST_EMU
   if (enable && h->fast_block != 32) return fail("fb_set_fast_slim: needs 32 environments per warp");
-  if (enable) {
-    int max_smem = 0;
-    cudaDeviceGetAttribute(&max_smem, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device);
-    if (fb_slim_attributes(h, max_smem)) return -1;
-  }
+  if (enable && fb_slim_attributes(h)) return -1;
 #endif
   h->fast_slim = enable != 0;
   return 0;
@@ -2319,11 +2308,9 @@ int fb_set_fast_split(FbHandle *h, int enable) {
  * wave of its blocks; while fb_create's 16-per-warp guess stands -- until the first launch of an
  * episode has been reviewed -- the single-warp kernels run) */
 int fb_fast_split(FbHandle *h) {
-  if (!h || !h->fast_enabled || !h->fast_split || h->fast_slim || !h->hm.m.X.ok) return 0;
-#ifndef FB_HOST_EMU
-  if (h->fast_block != 32 || (h->P.n_envs + 31)/32 > h->split_capacity) return 0;
-#endif
-  return h->hm.split.nwarps > 1 ? h->hm.split.nwarps : 0;
+  if (!h) return 0;
+  const FbPlan p = fb_next_step(h);
+  return p.fast && p.uncon.kind == FB_FAST_SPLIT ? h->hm.split.nwarps : 0;
 }
 /* drag_forces (swimming/drag.pyx:152-268) as a stand-alone device operator, see include/farms_b200.h */
 int fb_drag_forces(int device, int n, const double *links, const double *coefficients, const double *mass,
@@ -2380,24 +2367,14 @@ int fb_set_con_split(FbHandle *h, int enable) {
 }
 
 /* 1 when the next launch hands the fully handed-over groups to the SPLIT variant */
-int fb_con_split(FbHandle *h) {
-  if (!h || !h->fast_enabled || !h->con_thread || !h->con_split || h->fast_slim || !h->hm.m.X.con_ok) return 0;
-  if (h->hm.split.nwarps < 2) return 0;
-#ifdef FB_HOST_EMU
-  return 1;
-#else
-  return fb_con_split_pays(h);
-#endif
-}
+int fb_con_split(FbHandle *h) { return h && fb_next_step(h).con_split ? 1 : 0; }
 
 /* resident SPLIT blocks per SM as the runtime computes it (0: not applicable) */
 int fb_fast_split_blocks_per_sm(FbHandle *h) {
 #ifndef FB_HOST_EMU
   if (!h || !h->hm.m.X.ok || h->hm.split.nwarps < 2) return 0;
   int nb = 0;
-  const size_t sbytes = (size_t)h->hm.m.X.n_float*sizeof(float)*32 + FB_SPLIT_EXTRA_BYTES;
-  if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, fb_fast_split_kernel<1>, 32*h->hm.split.nwarps, sbytes) != cudaSuccess) return 0;
-  return nb;
+  return fb_kernel_attributes(fb_kernel_sel(h, FB_FAST_SPLIT, 32), &nb) == cudaSuccess ? nb : 0;
 #else
   (void)h; return 0;
 #endif
@@ -2417,7 +2394,11 @@ int fb_set_fast_lean(FbHandle *h, int enable) {
   return 0;
 }
 /* 1 when fb_step launches the LEAN variant for this model (a control sequence falls back) */
-int fb_fast_lean(FbHandle *h) { return h && h->fast_enabled && h->fast_lean && h->hm.m.X.ok && h->hm.m.X.lean ? 1 : 0; }
+int fb_fast_lean(FbHandle *h) {
+  if (!h) return 0;
+  const FbPlan p = fb_next_step(h);
+  return p.fast && p.uncon.lean ? 1 : 0;
+}
 /* environments the team kernel had to finish in the last fb_step (synchronises) */
 int fb_last_pending(FbHandle *h, int *count) {
   if (!h || !count) return fail("null argument");

@@ -386,7 +386,7 @@ SAMPLE = (0, 1, 31, 32, 33)
 @pytest.mark.parametrize('lean', [True, False])
 @pytest.mark.parametrize('split', [True, False])
 def test_gpu_oracle_parity_constrained(cuda_library, name, blk, lean, split, monkeypatch):
-    """Every variant of the per-thread constrained kernel's ENVP twin: BLK 16 / 32, LEAN and
+    """Every variant of the per-thread constrained kernel with ENVP = 1: BLK 16 / 32, LEAN and
     general, the SPLIT constrained kernel on and off."""
     monkeypatch.setenv('FARMS_B200_FAST_BLOCK', str(blk))
     n_envs, n_steps = 64, 8
@@ -436,7 +436,7 @@ def touch_down_case(n_envs, seed=5):
 @pytest.mark.gpu
 def test_gpu_touch_down_mid_launch(cuda_library):
     """A friction table alone: the unconstrained default kernel steps the falling environments and
-    hands each over to the constrained ENVP twin at its touch-down step, in the middle of one launch."""
+    hands each over to the constrained ENVP = 1 kernel at its touch-down step, in the middle of one launch."""
     n_envs, n_steps = 70, 16
     case = touch_down_case(n_envs)
     _, values, physics = run_batch(cuda_library, 'salamander', n_envs, n_steps, case=case)
@@ -476,10 +476,10 @@ def homogeneous_physics(library, spec, model, G, env, n_envs, n_steps):
 @pytest.mark.gpu
 @pytest.mark.parametrize('name,path', [('salamander', 'fast'), ('centipede', 'fast'), ('salamander', 'team')])
 def test_gpu_mixed_batch_equals_homogeneous_batches(cuda_library, name, path):
-    """Environment e of a batch with a friction table (the constrained ENVP twin, or the team kernel
+    """Environment e of a batch with a friction table (the constrained ENVP = 1 kernel, or the team kernel
     reading the table) against a batch of the MJCF edited to e's frictions (the default entry
     points), same inputs in every environment: bit-identical, or within 1e-5 relative where ptxas
-    contracts the twins differently."""
+    contracts the ENVP = 1 kernels differently."""
     from farms_mujoco_b200.engine import BatchedPhysics
     n_envs, n_steps = 64, 8
     spec, model, qpos0, qvel0, ctrl = make_case(name, 1)

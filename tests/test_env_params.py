@@ -315,7 +315,7 @@ def test_gpu_oracle_parity_slim(cuda_library, slim, monkeypatch):
 @pytest.mark.gpu
 def test_gpu_hand_over_mid_launch(cuda_library):
     """Swimming environments meet a joint limit after a few steps (a different step in every
-    environment, some never): the unconstrained twin hands them over to the constrained twin."""
+    environment, some never): the unconstrained ENVP = 1 kernel hands them over to the constrained one."""
     import fastpath_cases
     from farms_mujoco_b200.engine import BatchedPhysics
     n_envs, n_steps = 70, 16
@@ -364,9 +364,9 @@ def homogeneous_physics(library, spec, model, values, env, n_envs, n_steps):
     ('salamander_swim', 'team', 64, 0),
 ])
 def test_gpu_mixed_batch_equals_homogeneous_batches(cuda_library, name, path, n_envs, slim, monkeypatch):
-    """Environment e of a batch with per-environment tables (the ENVP twins) against a batch of
+    """Environment e of a batch with per-environment tables (the ENVP = 1 kernels) against a batch of
     the model edited to e's values (the default entry points), same kernel variant, same inputs in
-    every environment: the same bits, or a few ulp where ptxas contracts the twins differently."""
+    every environment: the same bits, or a few ulp where ptxas contracts the ENVP = 1 kernels differently."""
     from farms_mujoco_b200.engine import BatchedPhysics
     if slim:
         monkeypatch.setenv('FARMS_B200_FAST_BLOCK', '32')        # SLIM needs full warps

@@ -357,7 +357,7 @@ def gpu_paths():
 @pytest.mark.parametrize('label,env,setup,name,n_envs', gpu_paths(), ids=[p[0] for p in gpu_paths()])
 def test_gpu_parity(cuda_library, monkeypatch, label, env, setup, name, n_envs):
     """Restarted environments against a fresh batch and the others against a never-restarted one,
-    on each kernel path.  The restarted batch runs the ENVP twins (the episode clock is bound), the
+    on each kernel path.  The restarted batch runs the ENVP = 1 kernels (the episode clock is bound), the
     two reference batches the entry points: a separate compilation of the same arithmetic, held to
     1e-6 relative (the SLIM MULTI layout differs by a few ulp, DESIGN section 4); the team kernel
     is one compilation: the same bits."""
@@ -373,8 +373,8 @@ def test_gpu_parity(cuda_library, monkeypatch, label, env, setup, name, n_envs):
 
 def check_hand_over_mid_launch(library, n, tol):
     """Restarted swimming environments start just inside a joint limit that their position actuator
-    pulls them through after a few steps (fastpath_cases.hand_over_case): the unconstrained twin
-    hands them over to the constrained twin in the middle of the launch.  The wave controller (on
+    pulls them through after a few steps (fastpath_cases.hand_over_case): the unconstrained ENVP = 1 kernel
+    hands them over to the constrained one in the middle of the launch.  The wave controller (on
     the leg joints, so that it does not hold the driven body joints) keeps the episode clock bound."""
     import fastpath_cases
     from farms_mujoco_b200.engine import BatchedPhysics

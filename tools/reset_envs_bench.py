@@ -5,8 +5,9 @@ clock on the step kernels.
      SALAMANDERs with 1 environment, 1 %, 10 % and 100 % of them masked, next to the host time of
      one fb_reset of the whole batch (it uploads every row and synchronises).
   2. Step throughput with the episode clock bound (an environment restarted after iteration 0:
-     the ENVP twins run) against unbound (no restart: the entry points), alternated round after
-     round: 65,536 swimming SALAMANDERs (bench.py's headline configuration) and 4,096 on the ground.
+     the ENVP = 1 kernels run) against unbound (no restart: the ENVP = 0 kernels), alternated round
+     after round: 65,536 swimming SALAMANDERs (bench.py's headline configuration) and 4,096 on the
+     ground.
   3. With --parent TREE (a checkout of the parent commit, built): bench.py's headline line of this
      tree and of TREE alternated, and bench.py --dump-outputs of both compared file by file.
 
