@@ -89,7 +89,7 @@ struct EnvPtrs {
   long long ev_links, ev_joints, ev_contacts, ev_xfrc;
   /* per-environment parameters (fb_set_env_param), already offset by the environment: value c of
    * item i at ep_*[(i*k + c)*ep_pad]; NULL = the model's value */
-  const float *ep_stiffness, *ep_damping, *ep_coef, *ep_wvel;
+  const float *ep_stiffness, *ep_damping, *ep_coef, *ep_wvel, *ep_gain, *ep_bias;
   long long ep_pad;
   /* sliding friction of candidate c at fric[c*fric_stride]: this environment's column of the
    * FB_ENV_CAND_FRICTION table (stride env_pad), else the model's cand_friction (stride 1) */
@@ -652,7 +652,11 @@ FB_UNROLL
       float len = gear*qpos[MI(jnt_qposadr, j)], vel = gear*qvel[MI(jnt_dofadr, j)];
       float c = ctrl[a];
       if (MI(act_ctrllimited, a)) c = fminf(MF(act_ctrlrange, 2*a+1), fmaxf(MF(act_ctrlrange, 2*a), c));
-      float f = MF(act_gain, a)*c + MF(act_bias, 3*a) + MF(act_bias, 3*a+1)*len + MF(act_bias, 3*a+2)*vel;
+      const float gain = g.ep_gain ? g.ep_gain[a*g.ep_pad] : MF(act_gain, a);
+      float b0, b1, b2;
+      if (g.ep_bias) { b0 = g.ep_bias[3*a*g.ep_pad]; b1 = g.ep_bias[(3*a + 1)*g.ep_pad]; b2 = g.ep_bias[(3*a + 2)*g.ep_pad]; }
+      else { b0 = MF(act_bias, 3*a); b1 = MF(act_bias, 3*a+1); b2 = MF(act_bias, 3*a+2); }
+      float f = gain*c + b0 + b1*len + b2*vel;
       if (MI(act_forcelimited, a)) f = fminf(MF(act_forcerange, 2*a+1), fmaxf(MF(act_forcerange, 2*a), f));
       actf[a] = f;
     }
@@ -1785,12 +1789,15 @@ struct FbParams {
 
 /* Per-environment parameter tables (fb_set_env_param), float32 environment-minor: value c of item i
  * of environment env at [(i*k + c)*env_pad + env] -- jnt_stiffness [njnt], dof_damping [nv], drag
- * coefficients [n_swim][6], water velocity [3], candidate friction [ncand].  NULL: the model's value
- * for every environment.
+ * coefficients [n_swim][6], water velocity [3], candidate friction [ncand], actuator gain [nu] and
+ * bias [nu][3].  NULL: the model's value for every environment.
+ * lin [njnt][6] is derived on the host from `bias` while it is set (fb_env_act_derive): the records'
+ * linear actuation form Kq, Kqd, T0, KqU, KqdU, T0U of each FT_ACT_SIMPLE joint with this
+ * environment's biases, summed in double precision as the model compiler sums them.
  * A launch argument of its own (not a member of FbParams), so that the parameter blocks of the
  * kernels that do not read it keep their layout: the team kernel tests the pointers at run time,
- * the per-thread kernels read them in their ENVP twins only (the unconstrained twins never read
- * `fric`: the member is last, so the members they read keep their offsets).
+ * the per-thread kernels read them in their ENVP = 1 variants only (members are appended, so the
+ * earlier ones keep their offsets).
  * episode_start [n_envs] (fb_reset_envs): batch iteration of each environment's episode row 0; the
  * travelling-wave controller reads the episode's time (it0 + k - episode_start).  Bound only while
  * the wave controller is on and some episode began after iteration 0; NULL: it0 + k. */
@@ -1798,6 +1805,7 @@ struct FbEnvTables {
   const float *stiffness, *damping, *coef, *wvel;
   const float *fric;
   const long long *episode_start;
+  const float *gain, *bias, *lin;
 };
 
 #define FB_NEVER_DIRTY (-(1LL << 60))
@@ -1832,6 +1840,8 @@ FB_DEV EnvPtrs fb_env_ptrs(const FbParams &P, const FbEnvTables &T, int env) {
   g.ep_damping = T.damping ? T.damping + e : 0;
   g.ep_coef = T.coef ? T.coef + e : 0;
   g.ep_wvel = T.wvel ? T.wvel + e : 0;
+  g.ep_gain = T.gain ? T.gain + e : 0;
+  g.ep_bias = T.bias ? T.bias + e : 0;
   g.ep_pad = P.env_pad;
   g.fric = T.fric ? T.fric + e : m.F + m.o.cand_friction;
   g.fric_stride = T.fric ? (int)P.env_pad : 1;

@@ -483,7 +483,7 @@ static FbTeamKernel fb_team_kernel(int team) {
 #endif
 
 /* ---------------------------------------------------------------- handle */
-enum { FB_N_ENV_PARAM = FB_ENV_CAND_FRICTION + 1 };     /* fields of fb_set_env_param */
+enum { FB_N_ENV_PARAM = FB_ENV_ACT_BIAS + 1 };     /* fields of fb_set_env_param */
 
 struct FbHandle {
   FbHostModel hm;
@@ -520,7 +520,8 @@ struct FbHandle {
    * (FbParams::ep_*, float32 [item*k + c][env_pad]) and the values as set ([n_envs][width]) */
   float *ep_dev[FB_N_ENV_PARAM];
   std::vector<double> ep_host[FB_N_ENV_PARAM];
-  FbEnvTables ep;                   /* ep_dev as the kernels take it */
+  float *ep_lin;                    /* FbEnvTables::lin, derived while FB_ENV_ACT_BIAS is set (env_act_derive) */
+  FbEnvTables ep;                   /* ep_dev and ep_lin as the kernels take it */
   /* per-environment episodes (fb_reset_envs): device [n_envs] batch iteration of each episode's row 0,
    * and whether one may be non-zero (a restart after iteration 0 since fb_reset) */
   long long *episode_start;
@@ -633,6 +634,55 @@ static void deep_copy_model(FbHandle *h, const FbModel *m, const FbFarms *f) {
   }
 }
 
+/* ---- per-environment parameters: the tables as the kernels take them */
+static void env_param_bind(FbHandle *h) {
+  h->ep.stiffness = h->ep_dev[FB_ENV_JNT_STIFFNESS];
+  h->ep.damping = h->ep_dev[FB_ENV_DOF_DAMPING];
+  h->ep.coef = h->ep_dev[FB_ENV_DRAG_COEF];
+  h->ep.wvel = h->ep_dev[FB_ENV_WATER_VELOCITY];
+  h->ep.fric = h->ep_dev[FB_ENV_CAND_FRICTION];
+  h->ep.gain = h->ep_dev[FB_ENV_ACT_GAIN];
+  h->ep.bias = h->ep_dev[FB_ENV_ACT_BIAS];
+  h->ep.lin = h->ep_lin;
+}
+
+/* FbEnvTables::lin from the FB_ENV_ACT_BIAS table as set (double) and the current records: each
+ * FT_ACT_SIMPLE joint's linear actuation form with environment e's biases, summed by the model
+ * compiler's own fb_joint_actuation and rounded once, so that e steps bit for bit as a batch of the
+ * model edited to its biases.  Freed while no bias table is set.  The gains feed no such sum: the
+ * kernels read them from FB_ENV_ACT_GAIN where they use them. */
+static int env_act_derive(FbHandle *h) {
+  if (!h->ep_dev[FB_ENV_ACT_BIAS] || !h->hm.m.X.ok) {
+    if (h->ep_lin) { dev_sync(h->stream); dev_free(h->ep_lin); h->ep_lin = nullptr; }
+    env_param_bind(h);
+    return 0;
+  }
+  const FbModel &fm = h->fm_shallow;
+  const int n = h->P.n_envs, nu = fm.nu, nj = fm.njnt;
+  const long long pad = h->P.env_pad;
+  const int32_t *actwc = h->hm.I.data() + h->hm.m.o.ft_actwc;
+  std::vector<float> dev((size_t)6*nj*pad, 0.f);
+  for (size_t b = 1; b < h->hm.rec.size(); b++) {
+    const FastRec &r = h->hm.rec[b];
+    if (!(r.flags & FT_ACT_SIMPLE)) continue;
+    for (int e = 0; e < n; e++) {
+      const FbJointAct ja = fb_joint_actuation(&fm, h->has_farms ? &h->ff_shallow : nullptr, actwc, r,
+                                               h->ep_host[FB_ENV_ACT_BIAS].data() + (size_t)e*3*nu, nullptr);
+      const double t[6] = {ja.Kq, ja.Kqd, ja.T0, ja.KqU, ja.KqdU, ja.T0U};
+      for (int k = 0; k < 6; k++) dev[(size_t)(6*r.jid + k)*pad + e] = (float)t[k];
+    }
+  }
+  if (!h->ep_lin) {
+    void *p = nullptr;
+    if (dev_alloc(&p, dev.size()*sizeof(float))) return fail("per-environment actuator biases: device allocation failed");
+    h->ep_lin = static_cast<float *>(p);
+  }
+  if (h2d(h->ep_lin, dev.data(), dev.size()*sizeof(float), h->stream) || dev_sync(h->stream))
+    return fail(std::string("per-environment actuator biases: upload failed: ") + dev_error());
+  env_param_bind(h);
+  return 0;
+}
+
 /* (re)build the device model tables from the handle's host copies */
 static int upload_model(FbHandle *h) {
   FbWaveController wc;
@@ -680,7 +730,7 @@ static int upload_model(FbHandle *h) {
     h->csplitQ->split = h->hm.split;
   }
 #endif
-  return 0;
+  return env_act_derive(h);      /* the records' linear actuation forms may have changed */
 }
 
 /* capacity of the device control sequence ([n_steps][nu][env_pad] + the upload staging) */
@@ -809,7 +859,8 @@ static FbPlan fb_plan(const FbHandle *h, int mode, int want_derived, bool ctrl_s
   /* ENVP while a per-environment parameter table the kernel reads is set (the unconstrained kernels
    * never read the candidate friction), or the episode clock is bound: only while the wave
    * controller, the one step code that reads time, is on and some episode began after iteration 0 */
-  const int envp = ep.stiffness || ep.damping || ep.coef || ep.wvel || (m.n_wc > 0 && h->episode_late);
+  const int envp = ep.stiffness || ep.damping || ep.coef || ep.wvel || ep.gain || ep.bias ||
+                   (m.n_wc > 0 && h->episode_late);
   const int cenvp = envp || ep.fric;
 #ifdef FB_HOST_EMU
   /* The emulation steps one environment at a time (BLK = 1; a constrained group is one
@@ -1090,6 +1141,7 @@ void fb_destroy(FbHandle *h) {
   if (h->I_dev) dev_free(h->I_dev);
   if (h->F_dev) dev_free(h->F_dev);
   for (float *p : h->ep_dev) if (p) dev_free(p);
+  if (h->ep_lin) dev_free(h->ep_lin);
 #ifndef FB_HOST_EMU
   cudaEventDestroy(h->ev0); cudaEventDestroy(h->ev1);
   cudaStreamSynchronize(h->copy_stream);
@@ -1119,6 +1171,7 @@ int fb_create(const FbModel *model, const FbFarms *farms, int n_envs, int device
   if (!h) return fail("out of host memory");
   h->device = device; h->I_dev = nullptr; h->F_dev = nullptr; h->launches = 0; h->it = 0;
   for (float *&p : h->ep_dev) p = nullptr;
+  h->ep_lin = nullptr;
   memset(&h->ep, 0, sizeof(h->ep));
   h->last_ms = 0.f; h->has_wc = false; h->gather_links = h->gather_joints = h->gather_env = nullptr;
   h->seq_dev = h->seq_stage = nullptr; h->seq_len = h->seq_pos = h->seq_cap = h->seq_rows = 0;
@@ -1653,15 +1706,18 @@ int fb_set_water_velocity(FbHandle *h, double vx, double vy, double vz) {
 
 /* ---- per-environment parameters (fb_set_env_param) */
 static const char *const kEnvParamName[FB_N_ENV_PARAM] = {"FB_ENV_JNT_STIFFNESS", "FB_ENV_DOF_DAMPING", "FB_ENV_DRAG_COEF",
-                                                          "FB_ENV_WATER_VELOCITY", "FB_ENV_CAND_FRICTION"};
+                                                          "FB_ENV_WATER_VELOCITY", "FB_ENV_CAND_FRICTION",
+                                                          "FB_ENV_ACT_GAIN", "FB_ENV_ACT_BIAS"};
 
 /* Lowest candidate friction a table may hold (mjcf_subset.PAIR_MIN_FRICTION): the pyramid rows'
  * D = 1/(2 mu^2 R) stiffens as 1/mu^2, and the fp32 solver's error grows with it (DESIGN.md section 8) */
 #define FB_MIN_ENV_FRICTION 0.1
 
-/* values per environment of a field: njnt, nv, 6*n_swim, 3, ncand */
+/* values per environment of a field: njnt, nv, 6*n_swim, 3, ncand, nu, 3*nu */
 static int env_param_width(const FbHandle *h, int field) {
   switch (field) {
+    case FB_ENV_ACT_GAIN: return h->fm_shallow.nu;
+    case FB_ENV_ACT_BIAS: return 3*h->fm_shallow.nu;
     case FB_ENV_JNT_STIFFNESS: return h->fm_shallow.njnt;
     case FB_ENV_DOF_DAMPING: return h->fm_shallow.nv;
     case FB_ENV_DRAG_COEF: return h->has_farms ? 6*h->ff_shallow.n_swim : 0;
@@ -1677,16 +1733,10 @@ static double env_param_model(const FbHandle *h, int field, int c) {
     case FB_ENV_DOF_DAMPING: return h->fm_shallow.dof_damping[c];
     case FB_ENV_DRAG_COEF: return h->ff_shallow.swim_coefficients[c];
     case FB_ENV_CAND_FRICTION: return h->fm_shallow.cand_friction[c];
+    case FB_ENV_ACT_GAIN: return h->fm_shallow.actuator_gainprm[3*c];
+    case FB_ENV_ACT_BIAS: return h->fm_shallow.actuator_biasprm[c];
     default: return h->has_farms ? h->ff_shallow.water_velocity[c] : 0.0;
   }
-}
-
-static void env_param_bind(FbHandle *h) {
-  h->ep.stiffness = h->ep_dev[FB_ENV_JNT_STIFFNESS];
-  h->ep.damping = h->ep_dev[FB_ENV_DOF_DAMPING];
-  h->ep.coef = h->ep_dev[FB_ENV_DRAG_COEF];
-  h->ep.wvel = h->ep_dev[FB_ENV_WATER_VELOCITY];
-  h->ep.fric = h->ep_dev[FB_ENV_CAND_FRICTION];
 }
 
 int fb_set_env_param(FbHandle *h, int field, const double *values) {
@@ -1697,22 +1747,28 @@ int fb_set_env_param(FbHandle *h, int field, const double *values) {
     if (h->ep_dev[field]) { dev_sync(h->stream); dev_free(h->ep_dev[field]); h->ep_dev[field] = nullptr; }
     h->ep_host[field].clear();
     env_param_bind(h);
-    return 0;
+    return field == FB_ENV_ACT_BIAS ? env_act_derive(h) : 0;
   }
   if ((field == FB_ENV_DRAG_COEF || field == FB_ENV_WATER_VELOCITY) && (!h->has_farms || h->ff_shallow.n_swim <= 0))
     return fail(name + ": the model has no swimming links");
   if (field == FB_ENV_CAND_FRICTION && h->fm_shallow.ncand <= 0) return fail(name + ": the model has no collision candidates");
+  if ((field == FB_ENV_ACT_GAIN || field == FB_ENV_ACT_BIAS) && h->fm_shallow.nu <= 0) return fail(name + ": the model has no actuators");
   const FbModel &fm = h->fm_shallow;
   const int n = h->P.n_envs, w = env_param_width(h, field);
   const long long pad = h->P.env_pad;
   for (int e = 0; e < n; e++)
     for (int c = 0; c < w; c++) {
       const double v = values[(size_t)e*w + c];
-      const std::string at = " at environment " + std::to_string(e) +
-                             (field == FB_ENV_CAND_FRICTION ? ", candidate " : ", index ") + std::to_string(c);
-      /* drag coefficients are negative in FARMS (the force opposes the motion) and a water velocity is
-       * a vector: only stiffness and damping have a sign to check */
-      const int signed_field = field == FB_ENV_DRAG_COEF || field == FB_ENV_WATER_VELOCITY;
+      std::string at = " at environment " + std::to_string(e);
+      if (field == FB_ENV_CAND_FRICTION) at += ", candidate " + std::to_string(c);
+      else if (field == FB_ENV_ACT_GAIN) at += ", actuator " + std::to_string(c);
+      else if (field == FB_ENV_ACT_BIAS) at += ", actuator " + std::to_string(c/3) + ", column " + std::to_string(c%3);
+      else at += ", index " + std::to_string(c);
+      /* drag coefficients are negative in FARMS (the force opposes the motion), a water velocity is
+       * a vector, and MuJoCo checks no sign of a gain or bias (a <position kp> has bias -kp): only
+       * stiffness and damping have a sign to check */
+      const int signed_field = field == FB_ENV_DRAG_COEF || field == FB_ENV_WATER_VELOCITY ||
+                               field == FB_ENV_ACT_GAIN || field == FB_ENV_ACT_BIAS;
       if (!std::isfinite(v)) return fail(name + ": non-finite value" + at);
       if (!signed_field && v < 0.0) return fail(name + ": negative value" + at);
       const int free_entry = (field == FB_ENV_JNT_STIFFNESS && fm.jnt_type[c] == FB_JNT_FREE) ||
@@ -1742,7 +1798,7 @@ int fb_set_env_param(FbHandle *h, int field, const double *values) {
     return fail(name + ": upload failed: " + dev_error());
   h->ep_host[field].assign(values, values + (size_t)n*w);
   env_param_bind(h);
-  return 0;
+  return field == FB_ENV_ACT_BIAS ? env_act_derive(h) : 0;
 }
 
 int fb_get_env_param(FbHandle *h, int field, double *out) {

@@ -211,9 +211,11 @@ template <int SYNC> FB_DEV void fb_block_sync() {
  * warps, each visiting its own bodies of the tree in two phases per sweep (FastSplit, fb_model.h);
  * the per-body code is the one every other variant runs, in the same order along every chain, so
  * the results are bit-identical to the single-warp kernel. */
-/* ENVP = 1 (fb_set_env_param): joint stiffness and damping, drag coefficients and water velocity
- * come from the per-environment tables (FbEnvTables, `ept`) where one is set (a uniform null test
- * per table), else from the records / the model as with ENVP = 0.  Same arithmetic on the values. */
+/* ENVP = 1 (fb_set_env_param): joint stiffness and damping, drag coefficients, water velocity,
+ * actuator gains and biases come from the per-environment tables (FbEnvTables, `ept`) where one is
+ * set (a uniform null test per table), else from the records / the model as with ENVP = 0; the
+ * records' linear actuation form (Kq, Kqd, T0 and the unlogged KqU, KqdU, T0U) from the table the
+ * host derives from the biases (FbEnvTables::lin).  Same arithmetic on the values. */
 /* the tables' pointer is a member of the ENVP variants only: a member that the other variants never
  * read still changed how ptxas scheduled the SLIM kernels.  The ENVP variants also run the episode
  * clock (fb_reset_envs): the wave controller's time is formed from episode_it(it0 + k), with the
@@ -301,6 +303,21 @@ FB_UNROLL
   FB_MEM float *nroot() const { return cs + NB_NF*(m.nbody - 1)*BLK; }
   FB_MEM float *ncand(int fc) const { return csc + NC_NF*BLK*fc; }
 
+  /* actuator a's gain, entry i of the biases ([nu][3]) and term k of the joint's linear actuation
+   * form (FbEnvTables::lin; `model`: the record's value): this environment's where ENVP and a table */
+  FB_MEM float gain_of(int a) const {
+    if constexpr (ENVP != 0) if (this->ept->gain) return this->ept->gain[(size_t)a*P.env_pad + env];
+    return MF(act_gain, a);
+  }
+  FB_MEM float bias_of(int i) const {
+    if constexpr (ENVP != 0) if (this->ept->bias) return this->ept->bias[(size_t)i*P.env_pad + env];
+    return MF(act_bias, i);
+  }
+  FB_MEM float lin_of(const FastRec &rc, int k, float model) const {
+    if constexpr (ENVP != 0) if (this->ept->lin) return this->ept->lin[(size_t)(6*rc.jid + k)*P.env_pad + env];
+    return model;
+  }
+
   /* generic actuation (clamps, gears, partial logging): force sum and farms joint_torque */
   /* ctrl of actuator a at this step: the uploaded sequence when there is one, else the held value */
   FB_MEM float ctrl_of(int a, const float *seqk) const {
@@ -309,13 +326,13 @@ FB_UNROLL
 
   /* per-step constants of a joint's linear actuation form (load_state does this once when ctrl is held) */
   FB_MEM void seq_constants(const FastRec &rc, const float *seqk, float *tc, float *tu) const {
-    float c = rc.T0, u = rc.T0U;
+    float c = lin_of(rc, 2, rc.T0), u = lin_of(rc, 5, rc.T0U);
     int ap = -1, av = -1, at = -1;
     if (rc.fj >= 0) { ap = MI(fj_actpos, rc.fj); av = MI(fj_actvel, rc.fj); at = MI(fj_acttrq, rc.fj); }
     for (int t = MI(jnt_actstart, rc.jid); t < MI(jnt_actstart, rc.jid + 1); t++) {
       int a = MI(act_sorted, t);
       if (a == rc.wave_act || MI(ft_actoff, a)) continue;
-      float f = MF(act_gain, a)*seqk[(long long)a*P.env_pad];
+      float f = gain_of(a)*seqk[(long long)a*P.env_pad];
       c += f;
       if (!(a == ap || a == av || a == at)) u += f;
     }
@@ -342,7 +359,7 @@ FB_UNROLL
         c = ctrl_of(a, seqk);
       }
       if (MI(act_ctrllimited, a)) c = fminf(MF(act_ctrlrange, 2*a+1), fmaxf(MF(act_ctrlrange, 2*a), c));
-      float f = MF(act_gain, a)*c + MF(act_bias, 3*a) + MF(act_bias, 3*a+1)*(gear*q) + MF(act_bias, 3*a+2)*(gear*qd);
+      float f = gain_of(a)*c + bias_of(3*a) + bias_of(3*a+1)*(gear*q) + bias_of(3*a+2)*(gear*qd);
       if (MI(act_forcelimited, a)) f = fminf(MF(act_forcerange, 2*a+1), fmaxf(MF(act_forcerange, 2*a), f));
       tsum += gear*f;
       if (a == ap || a == av || a == at) lsum += f;
@@ -388,14 +405,14 @@ FB_UNROLL
         fb_st_scr(pg + FG_QD*BLK, gv[rc.da]);
         /* constant part of the joint's actuation over this launch (ctrl is held), and of
          * the actuators the farms joint_torque column leaves out */
-        float tc = rc.T0, tu = rc.T0U;
+        float tc = lin_of(rc, 2, rc.T0), tu = lin_of(rc, 5, rc.T0U);
         if (rc.flags & FT_ACT_SIMPLE) {
           int ap = -1, av = -1, at = -1;
           if (rc.fj >= 0) { ap = MI(fj_actpos, rc.fj); av = MI(fj_actvel, rc.fj); at = MI(fj_acttrq, rc.fj); }
           for (int t = MI(jnt_actstart, rc.jid); t < MI(jnt_actstart, rc.jid + 1); t++) {
             int a = MI(act_sorted, t);
             if (a == rc.wave_act || MI(ft_actoff, a)) continue;
-            float f = MF(act_gain, a)*g_ctrl[a];
+            float f = gain_of(a)*g_ctrl[a];
             tc += f;
             if (!(a == ap || a == av || a == at)) tu += f;
           }
@@ -759,15 +776,23 @@ FB_UNROLL
       for (int k = 0; k < 3; k++) { FB_PIN_F(rc.hloc[k]); FB_PIN_F(rc.axis[k]); }
 FB_UNROLL
       for (int k = 0; k < 5; k++) FB_PIN_F(rc.Ib[k]);
-      float estiff = 0.f, edamp = 0.f;       /* ENVP: this environment's values, loads issued here */
+      /* ENVP: this environment's values, loads issued here */
+      float estiff = 0.f, edamp = 0.f, eKq = 0.f, eKqd = 0.f, eKqU = 0.f, eKqdU = 0.f, ewgain = 0.f;
       if constexpr (ENVP) {
         const FbEnvTables *ept = this->ept;
         estiff = rc.stiffness; edamp = rc.damping;
+        eKq = rc.Kq; eKqd = rc.Kqd; eKqU = rc.KqU; eKqdU = rc.KqdU; ewgain = rc.wgain;
         if (rc.jtype > FB_JNT_FREE) {
           if (ept->stiffness) estiff = ept->stiffness[(size_t)rc.jid*P.env_pad + env];
           if (ept->damping) edamp = ept->damping[(size_t)rc.da*P.env_pad + env];
+          if (ept->lin) {
+            const float *l = ept->lin + (size_t)6*rc.jid*P.env_pad + env;
+            eKq = l[0]; eKqd = l[P.env_pad]; eKqU = l[3*P.env_pad]; eKqdU = l[4*P.env_pad];
+          }
+          if (ept->gain && rc.wave_act >= 0) ewgain = ept->gain[(size_t)rc.wave_act*P.env_pad + env];
         }
         FB_PIN_F(estiff); FB_PIN_F(edamp);
+        FB_PIN_F(eKq); FB_PIN_F(eKqd); FB_PIN_F(eKqU); FB_PIN_F(eKqdU); FB_PIN_F(ewgain);
       }
       if (SPLIT) { pb = block(b); pg = gblock(b); }
       else { pb -= NF*BLK; pg -= GNF*BLK; }
@@ -902,14 +927,14 @@ FB_UNROLL
         if (LEAN || (flags & FT_ACT_SIMPLE)) {
           float tc = cx[8], tu = cx[9];
           if (!LEAN && seqk) seq_constants(rc, seqk, &tc, &tu);
-          tau = tc + rc.Kq*qj + rc.Kqd*qd;
+          tau = tc + (ENVP ? eKq : rc.Kq)*qj + (ENVP ? eKqd : rc.Kqd)*qd;
           if (flags & FT_HAS_WAVE) {
             float ph = 6.283185307179586f*rc.wfreq*time - rc.wlag + env_phase;
             float cw = rc.woff + rc.wamp*sinf(ph);
-            tau += rc.wgain*cw;
+            tau += (ENVP ? ewgain : rc.wgain)*cw;
             if (store_ctrl) P.ctrl[(size_t)env*m.nu + rc.wave_act] = cw;
           }
-          trq = tau - (tu + rc.KqU*qj + rc.KqdU*qd);
+          trq = tau - (tu + (ENVP ? eKqU : rc.KqU)*qj + (ENVP ? eKqdU : rc.KqdU)*qd);
         } else {
           actuation_generic(rc, qj, qd, time, store_ctrl, seqk, &tau, &trq);
         }

@@ -298,6 +298,43 @@ inline void quat2mat(const double *q, double *m) {
 }
 }  // namespace fbdetail
 
+/* The actuation of joint record r (hinge or slide) from the biasprm rows `biasprm` ([nu][3]: the
+ * model's, or one environment's of fb_set_env_param): one linear form T0 + Kq q + Kqd qd (+ the ctrl
+ * terms the kernels add) when nothing clamps, gears are 1 and the farms joint_torque column sums
+ * exactly the joint's actuators (physics.py:510-524); the U terms are the part of it that column
+ * leaves out.  actwc[a]: the wave-controller entry driving actuator a (-1: none).  is_off (may be
+ * NULL) receives the actuators switched off by initialize_control. */
+struct FbJointAct {
+  bool simple;
+  int nwave, wave_act;            /* wave-driven actuators of the joint, the last one */
+  double Kq, Kqd, T0, KqU, KqdU, T0U;
+};
+inline FbJointAct fb_joint_actuation(const FbModel *fm, const FbFarms *ff, const int32_t *actwc, const FastRec &r,
+                                     const double *biasprm, int32_t *is_off) {
+  FbJointAct o = {true, 0, -1, 0, 0, 0, 0, 0, 0};
+  for (int a = 0; a < fm->nu; a++) {
+    if (fm->actuator_trnid[a] != r.jid) continue;
+    /* switched off by initialize_control (task.py:274-286): contributes exactly zero */
+    const bool off = fm->actuator_forcelimited[a] && fm->actuator_forcerange[2*a] == 0.0 &&
+                     fm->actuator_forcerange[2*a + 1] == 0.0;
+    if (off && actwc[a] < 0) { if (is_off) is_off[a] = 1; continue; }
+    if (fm->actuator_ctrllimited[a] || fm->actuator_forcelimited[a] || fm->actuator_gear[a] != 1.0) o.simple = false;
+    bool logged = r.fj >= 0 && (ff->joint_act_position[r.fj] == a || ff->joint_act_velocity[r.fj] == a ||
+                                ff->joint_act_torque[r.fj] == a);
+    o.T0 += biasprm[3*a]; o.Kq += biasprm[3*a + 1]; o.Kqd += biasprm[3*a + 2];
+    if (!logged) {
+      o.T0U += biasprm[3*a]; o.KqU += biasprm[3*a + 1]; o.KqdU += biasprm[3*a + 2];
+    }
+    if (actwc[a] >= 0) {
+      o.nwave++;
+      if (!logged && r.fj >= 0) o.simple = false;
+      o.wave_act = a;
+    }
+  }
+  if (o.nwave > 1) o.simple = false;
+  return o;
+}
+
 /* Flatten FbModel + FbFarms.  Returns false and sets out.error when the model
  * leaves the supported subset. */
 inline bool fb_build_model(const FbModel *fm, const FbFarms *ff, const FbWaveController *wc,
@@ -823,46 +860,23 @@ inline bool fb_build_model(const FbModel *fm, const FbFarms *ff, const FbWaveCon
       rec[b].height = (float)ff->swim_height[i];
       for (int k = 0; k < 6; k++) rec[b].coef[k] = (float)ff->swim_coefficients[6*i + k];
     }
-    /* actuation: one linear form per joint when nothing clamps, gears are 1 and the farms
-     * joint_torque column sums exactly the joint's actuators (physics.py:510-524) */
+    /* actuation: one linear form per joint where fb_joint_actuation finds one */
     std::vector<int32_t> is_off(nu > 0 ? nu : 1, 0);
     for (int b = 1; b < nb; b++) {
       FastRec &r = rec[b];
       if (r.jid < 0 || r.jtype == FB_JNT_FREE) continue;
-      bool simple = true;
-      int nwave = 0;
-      double Kq = 0, Kqd = 0, T0 = 0, KqU = 0, KqdU = 0, T0U = 0;
-      for (int a = 0; a < nu; a++) {
-        if (fm->actuator_trnid[a] != r.jid) continue;
-        /* switched off by initialize_control (task.py:274-286): contributes exactly zero */
-        const bool off = fm->actuator_forcelimited[a] && fm->actuator_forcerange[2*a] == 0.0 &&
-                         fm->actuator_forcerange[2*a + 1] == 0.0;
-        if (off && actwc[a] < 0) { is_off[a] = 1; continue; }
-        if (fm->actuator_ctrllimited[a] || fm->actuator_forcelimited[a] || fm->actuator_gear[a] != 1.0) simple = false;
-        bool logged = r.fj >= 0 && (ff->joint_act_position[r.fj] == a || ff->joint_act_velocity[r.fj] == a ||
-                                    ff->joint_act_torque[r.fj] == a);
-        T0 += fm->actuator_biasprm[3*a]; Kq += fm->actuator_biasprm[3*a + 1]; Kqd += fm->actuator_biasprm[3*a + 2];
-        if (!logged) {
-          T0U += fm->actuator_biasprm[3*a]; KqU += fm->actuator_biasprm[3*a + 1]; KqdU += fm->actuator_biasprm[3*a + 2];
-        }
-        if (actwc[a] >= 0) {
-          int w = actwc[a];
-          nwave++;
-          if (!logged && r.fj >= 0) simple = false;
-          r.wave_act = a;
-          r.wgain = (float)fm->actuator_gainprm[3*a];
-          r.wamp = (float)wc->amplitude[w]; r.woff = (float)(wc->offset ? wc->offset[w] : 0.0);
-          r.wfreq = (float)wc->frequency[w]; r.wlag = (float)wc->phase_lag[w];
-        }
+      const FbJointAct ja = fb_joint_actuation(fm, ff, actwc.data(), r, fm->actuator_biasprm, is_off.data());
+      if (ja.nwave > 0) {
+        const int a = ja.wave_act, w = actwc[a];
+        r.wgain = (float)fm->actuator_gainprm[3*a];
+        r.wamp = (float)wc->amplitude[w]; r.woff = (float)(wc->offset ? wc->offset[w] : 0.0);
+        r.wfreq = (float)wc->frequency[w]; r.wlag = (float)wc->phase_lag[w];
       }
-      if (nwave > 1) simple = false;
-      if (simple) {
+      if (ja.simple) {
         r.flags |= FT_ACT_SIMPLE;
-        if (nwave == 1) r.flags |= FT_HAS_WAVE;
-        r.Kq = (float)Kq; r.Kqd = (float)Kqd; r.T0 = (float)T0;
-        r.KqU = (float)KqU; r.KqdU = (float)KqdU; r.T0U = (float)T0U;
-      } else {
-        r.wave_act = -1;
+        if (ja.nwave == 1) { r.flags |= FT_HAS_WAVE; r.wave_act = ja.wave_act; }
+        r.Kq = (float)ja.Kq; r.Kqd = (float)ja.Kqd; r.T0 = (float)ja.T0;
+        r.KqU = (float)ja.KqU; r.KqdU = (float)ja.KqdU; r.T0U = (float)ja.T0U;
       }
     }
     /* conservative plane checks per body: no candidate of the body can be active while

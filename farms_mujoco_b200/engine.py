@@ -502,7 +502,8 @@ class BatchedPhysics:
         n_swim = len(self.tables.swim_links_index)
         return {'jnt_stiffness': (0, (self.model.njnt,)), 'dof_damping': (1, (self.model.nv,)),
                 'drag_coefficients': (2, (n_swim, 2, 3)), 'water_velocity': (3, (3,)),
-                'geom_friction': (4, (self.model.ngeom,))}
+                'geom_friction': (4, (self.model.ngeom,)),
+                'actuator_gainprm': (5, (self.model.nu,)), 'actuator_biasprm': (6, (self.model.nu, 3))}
 
     def set_env_params(self, **fields):
         """Per-environment physical parameters (fb_set_env_param): ``jnt_stiffness [n_envs, njnt]``,
@@ -510,10 +511,16 @@ class BatchedPhysics:
         ``FarmsTables.swim_coefficients``), ``water_velocity [n_envs, 3]`` and ``geom_friction [n_envs,
         ngeom]`` (the sliding friction ``model.geom_friction[:, 0]``; each collision candidate gets the
         two geoms' values mixed as the compiler mixes them, ``mjcf_subset.candidate_friction``, and
-        explicit ``<pair>`` candidates keep the pair's friction).  Environment ``e`` then steps as the
-        model edited to its values.  Only the keywords passed change; ``None`` returns a field to the
-        model's value; an array without the environment axis is broadcast to every environment.  The
-        tables survive ``reset``."""
+        explicit ``<pair>`` candidates keep the pair's friction), ``actuator_gainprm [n_envs, nu]`` (the
+        fixed gain ``model.actuator_gainprm[:, 0]``, the only column the step reads) and
+        ``actuator_biasprm [n_envs, nu, 3]`` (``model.actuator_biasprm[:, 0:3]``).  A ``<position kp>``
+        actuator is gain ``kp`` and bias ``[0, -kp, 0]``, a ``<velocity kv>`` gain ``kv`` and bias
+        ``[0, 0, -kv]``: a kp sweep sets ``gainprm[:, a] = kp`` and ``biasprm[:, a, 1] = -kp``.  Gains
+        and biases have no sign check (MuJoCo has none); a kv too large for the explicit Euler step
+        diverges and shows in ``flags``.  Environment ``e`` then steps as the model edited to its
+        values.  Only the keywords passed change; ``None`` returns a field to the model's value; an
+        array without the environment axis is broadcast to every environment.  The tables survive
+        ``reset`` and ``reset_envs``."""
         known = self._env_param_fields()
         for name in fields:
             if name not in known:

@@ -264,6 +264,11 @@ int fb_set_swimming(FbHandle *h, int drag, int buoyancy);
  *   FB_ENV_CAND_FRICTION   [n_envs][ncand]    FbModel.cand_friction: the mixed sliding friction of each
  *                                             collision candidate (the geoms' friction put through the
  *                                             compiler's mixing rule, mjcf_subset.candidate_friction)
+ *   FB_ENV_ACT_GAIN        [n_envs][nu]       model.actuator_gainprm[:, 0] (the fixed gain; the other
+ *                                             columns are not read)
+ *   FB_ENV_ACT_BIAS        [n_envs][nu][3]    model.actuator_biasprm[:, 0:3]
+ *                                             (a <position kp> is gain kp, bias [0, -kp, 0]; a
+ *                                             <velocity kv> is gain kv, bias [0, 0, -kv])
  * Environment e then steps exactly as the model edited to e's values.  values: host float64; NULL
  * returns the field to the model's value.  Refused, with the field and the first bad index named:
  * non-finite values, negative stiffness or damping (drag coefficients are negative in FARMS and a
@@ -271,12 +276,14 @@ int fb_set_swimming(FbHandle *h, int drag, int buoyancy);
  * on the free joint, drag coefficients or water velocity on a model without swimming links, a
  * candidate friction below 0.1 (the pyramid rows stiffen as 1/mu^2 and the fp32 solver's error grows
  * with them), and a friction of an explicit <pair> candidate (cand_end 20 or 21) other than the
- * model's: a pair takes its friction from the pair element.  The
- * tables survive fb_reset and are freed by fb_destroy; while FB_ENV_WATER_VELOCITY is set,
+ * model's: a pair takes its friction from the pair element.  Gains and biases have no sign check, as
+ * in MuJoCo: a velocity gain too large for the explicit Euler step diverges and shows as flags bit
+ * 0, like any divergence.  The
+ * tables survive fb_reset and fb_reset_envs and are freed by fb_destroy; while FB_ENV_WATER_VELOCITY is set,
  * fb_set_water_velocity is refused.  fb_get_env_param returns the values in the same layout (the
  * model's value broadcast for a field that is not set). */
 enum { FB_ENV_JNT_STIFFNESS = 0, FB_ENV_DOF_DAMPING = 1, FB_ENV_DRAG_COEF = 2, FB_ENV_WATER_VELOCITY = 3,
-       FB_ENV_CAND_FRICTION = 4 };
+       FB_ENV_CAND_FRICTION = 4, FB_ENV_ACT_GAIN = 5, FB_ENV_ACT_BIAS = 6 };
 int fb_set_env_param(FbHandle *h, int field, const double *values);
 int fb_get_env_param(FbHandle *h, int field, double *out);
 
